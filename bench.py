@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- scan-points x RK4-steps / second of the batched FWM sweep on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[3], the configuration the metric is quoted on): the 2-D pump x signal
 wavelength sweep, 1000 x 1000 = 1e6 scan points, 2 500 RK4 steps each (z_max = 500 m, dz = 0.2 m,
@@ -28,6 +28,9 @@ done by the sweep kernel itself (NVLink peer stores into the full-size map of ev
 IPC; `--gather nccl` or a box without peer access: an NCCL all-gather after the kernel); the weak-scaling
 figure (1e6 points per GPU, NCCL all-gather) is reported alongside under "weak".
 `--impl reference` times the CPU arm with all host cores; only rank 0 works.
+
+`--dump-outputs DIR` writes what the last timed step computed as DIR/<name>.npy.  The inputs are fixed
+(linspace axes, seeded samples), so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -96,6 +99,15 @@ def ncu_traffic_bytes(seg: bool):
         if len(vals) == 2:
             best = (sum(vals.values()), path.name)
     return best if best else (None, None)
+
+
+def dump_outputs(out_dir, arrays: dict) -> None:
+    """Write the results of the last timed step as <out_dir>/<name>.npy: a map of the whole grid as [N1, N3],
+    anything smaller (a shard, a sample of points) flat."""
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(out_dir / f"{name}.npy", a.reshape(N1, N3) if a.size == N1 * N3 else a)
 
 
 # ----------------------------------------------------------------------------- CPU arm
@@ -183,8 +195,10 @@ def run_reference(args) -> None:
         cpu_sample(cores, cores, seed=99, kind=kind)
     t_total = 0.0
     for k in range(args.steps):
-        _, wall, _, _ = cpu_sample(n_points, cores, seed=k, kind=kind)
+        _, wall, idx, gains = cpu_sample(n_points, cores, seed=k, kind=kind)
         t_total += wall
+    if args.dump_outputs:       # the sampled points of the last step: flat indices into the N1 x N3 grid
+        dump_outputs(args.dump_outputs, {"gain_lin": gains, "point_index": idx.astype(np.float64)})
     value = n_points * n_steps * args.steps / t_total
     sample = f"{n_points} random points of the 1000x1000 grid x {n_steps} RK4 steps per bench step"
     print(json.dumps({
@@ -498,6 +512,12 @@ def run_ours(args) -> None:
             peers.close(dist)
     else:
         full_dev = gain_dev
+    if args.dump_outputs and rank == 0:
+        outputs = {"gain_lin": full_dev}
+        if world == 1:      # the per-point outputs of a shard are not gathered at N > 1
+            outputs.update(dbeta=sweep.t_dbeta.cpu().numpy(), valid=sweep.t_valid.cpu().numpy().astype(np.float32),
+                           status=sweep.t_status.cpu().numpy().astype(np.float32))
+        dump_outputs(args.dump_outputs, outputs)
 
     # ---- weak scaling alongside (N > 1): 1e6 points per GPU on a (1000 N) x 1000 grid
     weak = None
@@ -890,7 +910,12 @@ def main() -> None:
                     help="profiling aid (one GPU): run only rank 0's share of an N-way split of the grid, e.g. 8 -> 125 000 points")
     ap.add_argument("--no-secondary", action="store_true",
                     help="skip the secondary configurations (profiling runs under ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed sweep computed as DIR/<name>.npy (24 MB at N = 1): gain_lin and "
+                         "dbeta in float64, valid and status in float32; at N > 1 rank 0 writes the gathered gain_lin map")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     # stdout carries ONE JSON line.  Anything else written to file descriptor 1 -- NCCL prints its
     # version banner there with NCCL_DEBUG >= VERSION, libraries may print -- is sent to stderr; the

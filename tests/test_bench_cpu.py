@@ -6,6 +6,8 @@ import subprocess
 import sys
 from pathlib import Path
 
+import numpy as np
+
 ROOT = Path(__file__).resolve().parent.parent
 sys.path.insert(0, str(ROOT))
 import bench  # noqa: E402
@@ -28,9 +30,9 @@ def test_roofline_traffic_comes_from_committed_ncu_summaries():
     assert (ROOT / "profiles" / src).exists() and (ROOT / "profiles" / src_seg).exists()
 
 
-def test_reference_arm_prints_one_json_line():
-    res = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0"],
-                         capture_output=True, text=True, timeout=600)
+def test_reference_arm_prints_one_json_line(tmp_path):
+    res = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0",
+                          "--dump-outputs", str(tmp_path / "out")], capture_output=True, text=True, timeout=600)
     assert res.returncode == 0, res.stderr[-2000:]
     lines = [ln for ln in res.stdout.splitlines() if ln.strip()]
     assert len(lines) == 1
@@ -38,3 +40,7 @@ def test_reference_arm_prints_one_json_line():
     assert d["impl"] == "reference" and d["unit"] == bench.UNIT and d["higher_is_better"] is True
     assert d["cpu_baseline"]["kind"] in ("reference", "port") and d["cpu_baseline"]["cores"] >= 1
     assert d["value"] > 0 and d["e2e"]["value"] == d["value"] and d["e2e"]["h2d_bytes_per_step"] == 0
+    gain, idx = np.load(tmp_path / "out" / "gain_lin.npy"), np.load(tmp_path / "out" / "point_index.npy")
+    n = d["config"]["points_per_step"]
+    assert gain.shape == idx.shape == (n,) and gain.dtype == idx.dtype == np.float64 and np.all(gain > 0)
+    assert np.array_equal(idx, np.random.default_rng(0).choice(bench.N1 * bench.N3, size=n, replace=False))
