@@ -253,6 +253,58 @@ int fpa_yaman4_sweep_multi_host(const fpa_sweep_desc* d, int n_devices, const in
 int64_t fpa_yaman4_sweep_scratch_bytes(int64_t n_points);
 int fpa_yaman4_sweep_dev(const fpa_sweep_desc* d, void* scratch, int64_t scratch_bytes, void* stream);
 
+/* ------------------------------------------------ phase-sensitive sweep (wavelength grid x input phase)
+ * The fused sweep above with an input-phase axis: every grid point g (b = i1*n3 + i3) runs K initial
+ * states, A0_table[k] = make_initial_amplitudes(p_in, phase_in + phase_axis[k]*weights)
+ * (simulation.py:103-123, built by the host mirror), so run k of grid point g starts from exactly the
+ * bits the plain sweep would use with that phase_in.  Run (g, k) is point g*K + k (phases fastest).
+ *   gain_lin[g*K + k] = P3 / p_in[2], NaN for failed / non-finite / <= 0 runs, with P3 chosen by `metric`:
+ *     FPA_GAIN_MAX_SAVED   max over the saved samples of |A3|^2 -- the plain sweep's metric
+ *                          (scan_mismtach.py:723-738)
+ *     FPA_GAIN_LAST_SAVED  |A3|^2 of the LAST SAVED sample, the reference's Pz[-1]
+ *                          (scan_mismtach.py:27-40): not the fiber end when save_every does not divide
+ *                          the step count
+ * and, per grid point over its K gains, numpy's nan-reductions (one small kernel on the same stream
+ * right after the sweep kernel): gain_max = nanmax, gain_min = nanmin, idx_max / idx_min =
+ * nanargmax / nanargmin (first index on ties), n_finite = number of non-NaN gains; a grid point whose K
+ * gains are all NaN (e.g. an invalid plan) gives NaN, -1, -1 and 0.
+ * Shapes: sweep.plan.dbeta / valid / omega are per GRID point [G] (G = n1*n3, or n_sub_points);
+ * sweep.gain_lin, Pmax, A_end and status are per run [G*K]; the reduction outputs are [G] and each may
+ * be NULL.  sweep.first_point / n_sub_points select GRID points (the K runs of a grid point are never
+ * split).  sweep.A0 is ignored; sweep.n_peers must be 0 (FPA_ERR_INVALID).  Units, check_nan and the
+ * FPA_PHASE_EXACT refusal (FPA_ERR_UNSUPPORTED) are those of fpa_yaman4_sweep_*.
+ */
+#define FPA_GAIN_MAX_SAVED  0
+#define FPA_GAIN_LAST_SAVED 1
+#define FPA_MAX_PHASES      65536
+
+typedef struct fpa_phase_sweep_desc {
+    fpa_sweep_desc sweep;        /* wavelength grid, physics and per-run outputs (see above)        */
+    int64_t        n_phases;     /* K, 1..FPA_MAX_PHASES                                            */
+    const double*  A0_table;     /* [K,4] complex128                                                */
+    int32_t        metric;       /* FPA_GAIN_MAX_SAVED | FPA_GAIN_LAST_SAVED                        */
+    int32_t        reserved;
+    double*        gain_max;     /* [G] or NULL                                                     */
+    double*        gain_min;     /* [G] or NULL                                                     */
+    int32_t*       idx_max;      /* [G] or NULL                                                     */
+    int32_t*       idx_min;      /* [G] or NULL                                                     */
+    int32_t*       n_finite;     /* [G] or NULL                                                     */
+} fpa_phase_sweep_desc;
+
+/* Host pointers, as fpa_yaman4_sweep_host.  sweep.gain_lin may be NULL: the [G*K] gain map then stays in
+ * the library workspace and only the reductions come back (a 1000 x 1000 x 64 sweep needs no 512 MB
+ * host array). */
+int fpa_yaman4_phase_sweep_host(const fpa_phase_sweep_desc* d, int device);
+/* The grid points split over several devices of one box from ONE process (contiguous ranges whose sizes
+ * differ by at most one); bit-identical to the single-device call for any device list. */
+int fpa_yaman4_phase_sweep_multi_host(const fpa_phase_sweep_desc* d, int n_devices, const int* devices);
+/* Device scratch for the z-segment scheduler of a phase sweep of n_points = G*K runs: one more double of
+ * state per run than fpa_yaman4_scratch_bytes (the last saved signal power travels with the segment). */
+int64_t fpa_yaman4_phase_sweep_scratch_bytes(int64_t n_points);
+/* Device pointers, asynchronous on `stream`: the sweep kernel and the reduction kernel.  sweep.gain_lin
+ * must be set.  `scratch` NULL: the whole-run kernel (same results). */
+int fpa_yaman4_phase_sweep_dev(const fpa_phase_sweep_desc* d, void* scratch, int64_t scratch_bytes, void* stream);
+
 /* ------------------------------------------------ linear test RHS  y' = lambda*y
  * Lets the reference's own integrator tests (tests.py:146-226, y' = y on a real
  * state) run on the device: complex lambda per component, complex128 state.

@@ -211,6 +211,38 @@ def sweep(desc, *, want_pmax=False, want_end=False, device: Optional[int] = None
     return out
 
 
+def phase_sweep(desc, *, want_map: bool = True, device: Optional[int] = None, devices=None) -> dict:
+    """Run `fpa_yaman4_phase_sweep_host` on a PhaseSweepDesc whose plan axes, physics, n_phases, A0_table and
+    metric are filled.  Returns gain_lin / status [n1,n3,K], dbeta / valid and the reductions gain_max,
+    gain_min, idx_max, idx_min, n_finite [n1,n3].  `want_map=False` leaves the gain map in the library's
+    workspace (no gain_lin in the result).  `devices`: split the grid over several GPUs
+    (`fpa_yaman4_phase_sweep_multi_host`)."""
+    n1, n3, K = desc.sweep.plan.n1, desc.sweep.plan.n3, int(desc.n_phases)
+    big = n1 * n3 * K >= 4096
+    out = {"dbeta": result_array((n1, n3), np.float64, big), "valid": result_array((n1, n3), np.int32, big),
+           "status": result_array((n1, n3, K), np.int32, big)}
+    if want_map:
+        out["gain_lin"] = result_array((n1, n3, K), np.float64, big)
+    for key, dtype in (("gain_max", np.float64), ("gain_min", np.float64), ("idx_max", np.int32),
+                       ("idx_min", np.int32), ("n_finite", np.int32)):
+        out[key] = result_array((n1, n3), dtype, big)
+        setattr(desc, key, ptr(out[key]))
+    w = desc.sweep
+    w.plan.dbeta, w.plan.valid, w.plan.omega = ptr(out["dbeta"]), ptr(out["valid"]), None
+    w.gain_lin, w.status, w.Pmax, w.A_end = ptr(out.get("gain_lin")), ptr(out["status"]), None, None
+    if n1 * n3 == 0:
+        return out
+    if devices is not None and len(devices) > 1:
+        ids = (C.c_int * len(devices))(*[int(v) for v in devices])
+        _lib.check(_lib.lib().fpa_yaman4_phase_sweep_multi_host(C.byref(desc), len(devices), ids))
+        return out
+    dev = _lib.get_device() if device is None else int(device)
+    if devices is not None and len(devices) == 1:
+        dev = int(devices[0])
+    _lib.check(_lib.lib().fpa_yaman4_phase_sweep_host(C.byref(desc), dev))
+    return out
+
+
 def enumerate_triplets(grid_index) -> tuple[np.ndarray, np.ndarray]:
     """(table[T] of (k,l,m,weight) int16, row_ptr[N+1] int64) on an integer frequency grid."""
     g = np.ascontiguousarray(grid_index, dtype=np.int32).reshape(-1)

@@ -76,6 +76,21 @@ class SweepDesc(C.Structure):
     ]
 
 
+GAIN_MAX_SAVED, GAIN_LAST_SAVED = 0, 1
+MAX_PHASES = 65536
+
+
+class PhaseSweepDesc(C.Structure):
+    _fields_ = [
+        ("sweep", SweepDesc),
+        ("n_phases", C.c_int64),
+        ("A0_table", C.c_void_p),
+        ("metric", C.c_int32), ("reserved", C.c_int32),
+        ("gain_max", C.c_void_p), ("gain_min", C.c_void_p),
+        ("idx_max", C.c_void_p), ("idx_min", C.c_void_p), ("n_finite", C.c_void_p),
+    ]
+
+
 class Triplet(C.Structure):
     _fields_ = [("k", C.c_int16), ("l", C.c_int16), ("m", C.c_int16), ("weight", C.c_int16)]
 
@@ -122,6 +137,10 @@ SIGNATURES = {
     "fpa_yaman4_sweep_multi_host": (C.c_int, [C.POINTER(SweepDesc), C.c_int, C.POINTER(C.c_int)]),
     "fpa_yaman4_sweep_scratch_bytes": (C.c_int64, [C.c_int64]),
     "fpa_yaman4_sweep_dev": (C.c_int, [C.POINTER(SweepDesc), C.c_void_p, C.c_int64, C.c_void_p]),
+    "fpa_yaman4_phase_sweep_host": (C.c_int, [C.POINTER(PhaseSweepDesc), C.c_int]),
+    "fpa_yaman4_phase_sweep_multi_host": (C.c_int, [C.POINTER(PhaseSweepDesc), C.c_int, C.POINTER(C.c_int)]),
+    "fpa_yaman4_phase_sweep_scratch_bytes": (C.c_int64, [C.c_int64]),
+    "fpa_yaman4_phase_sweep_dev": (C.c_int, [C.POINTER(PhaseSweepDesc), C.c_void_p, C.c_int64, C.c_void_p]),
     "fpa_linear_rk4_batch_host": (C.c_int, [C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_double,
                                             C.c_double, C.c_int64, C.c_int64, C.c_void_p, C.c_uint32,
                                             C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),

@@ -22,7 +22,11 @@ int yaman4_rhs_launch(int64_t B, const double* z, const double* A, const double*
                       const double* alpha, const double* dbeta, double* dA, cudaStream_t st);
 int plan_launch(const fpa_plan_desc* d, double* dbeta_masked, cudaStream_t st);
 int yaman4_sweep_launch(const fpa_sweep_desc* d, void* scratch, int64_t scratch_bytes, cudaStream_t st);
+int yaman4_phase_sweep_launch(const fpa_phase_sweep_desc* d, void* scratch, int64_t scratch_bytes, cudaStream_t st);
+int phase_reduce_launch(int64_t G, int K, const double* gain, double* gmax, double* gmin, int32_t* imax, int32_t* imin,
+                        int32_t* nfin, cudaStream_t st);
 int64_t yaman4_scratch_bytes(int64_t n_points);
+int64_t yaman4_phase_scratch_bytes(int64_t n_points);
 int linear_launch(int64_t B, int dim, const double* y0, const double* lam, double z0, double z_max,
                   int64_t n_steps, int64_t save_every, const double* z_grid, uint32_t flags,
                   double* y_trace, double* y_end, int32_t* bad_scratch, int32_t* status,
@@ -189,6 +193,15 @@ static int nwave_dispatch(const fpa_nwave_desc* d, cudaStream_t st) {
 // arithmetic structure is available through fpa_dbeta_table_* + fpa_yaman4_rk4_batch_*.
 static int sweep_dev(const fpa_sweep_desc* d, void* scratch, int64_t scratch_bytes, cudaStream_t st) {
     return yaman4_sweep_launch(d, scratch, scratch_bytes, st);
+}
+
+// Phase sweep: the sweep kernel, then the per-grid-point reductions over its gain map on the same stream.
+static int phase_sweep_dev(const fpa_phase_sweep_desc* d, void* scratch, int64_t scratch_bytes, cudaStream_t st) {
+    FPA_TRY(yaman4_phase_sweep_launch(d, scratch, scratch_bytes, st));
+    const fpa_sweep_desc& w = d->sweep;
+    const int64_t G = (w.first_point == 0 && w.n_sub_points == 0) ? w.plan.n1 * w.plan.n3 : w.n_sub_points;
+    return phase_reduce_launch(G, (int)d->n_phases, w.gain_lin, d->gain_max, d->gain_min, d->idx_max, d->idx_min,
+                               d->n_finite, st);
 }
 
 // Contiguous share of n items for part k of `parts`: sizes differ by at most one.
@@ -546,17 +559,26 @@ int fpa_yaman4_sweep_dev(const fpa_sweep_desc* d, void* scratch, int64_t scratch
 // sweep_host_launch queues the axes upload and the kernel; sweep_host_collect queues the result
 // copies (a copy into pageable memory blocks the host until the kernel is done, so every device's
 // kernel has to be in flight before the first collect) and the caller synchronises the stream.
+// A phase sweep (`ph` set) runs K = ph->n_phases initial states per grid point: the per-run arrays hold B*K entries,
+// the plan outputs and the reductions B.
 struct PendingSweep {
     cudaStream_t st = nullptr;
-    size_t       B = 0;
+    size_t       B = 0, P = 0;  // grid points, runs (P = B*K)
     // device staging buffers, NULL where the kernel wrote straight into the caller's pinned array
     double * gain = nullptr, *db = nullptr, *Pm = nullptr, *Ae = nullptr, *om = nullptr;
     int32_t *va = nullptr, *stt = nullptr;
-    fpa_sweep_desc user;  // the caller's (host) pointers
+    double * gmax = nullptr, *gmin = nullptr;  // phase sweep reductions
+    int32_t *imax = nullptr, *imin = nullptr, *nfin = nullptr;
+    fpa_sweep_desc       user;  // the caller's (host) pointers
+    fpa_phase_sweep_desc puser;
 };
 
-static int sweep_host_launch(const fpa_sweep_desc* d, int device, PendingSweep* ps) {
+static int sweep_host_launch(const fpa_sweep_desc* d, const fpa_phase_sweep_desc* ph, int device, PendingSweep* ps) {
     FPA_REQUIRE(d != nullptr, "sweep descriptor is NULL");
+    FPA_REQUIRE(!ph || (ph->n_phases >= 1 && ph->n_phases <= FPA_MAX_PHASES), "n_phases must be in [1, %d]",
+                FPA_MAX_PHASES);
+    FPA_REQUIRE(!ph || ph->A0_table != nullptr, "A0_table must be set");
+    FPA_REQUIRE(!ph || d->n_peers == 0, "the phase sweep has no peer-store gather: n_peers must be 0");
     const fpa_plan_desc& pl = d->plan;
     FPA_REQUIRE(pl.n1 >= 0 && pl.n3 >= 0, "grid sizes must be >= 0");
     FPA_REQUIRE(pl.lambda1 && pl.lambda2 && pl.lambda3, "wavelength axes must be set");
@@ -569,14 +591,18 @@ static int sweep_host_launch(const fpa_sweep_desc* d, int device, PendingSweep* 
     // points of this call: the whole grid, or the sub-range (outputs are indexed from its first point)
     const size_t B = (d->first_point == 0 && d->n_sub_points == 0) ? n1 * n3 : (size_t)d->n_sub_points;
     if (B == 0) return FPA_OK;
-    FPA_REQUIRE(d->gain_lin != nullptr, "gain_lin must be set");
+    // the phase sweep may leave its gain map in the workspace (only the reductions come back)
+    FPA_REQUIRE(ph || d->gain_lin != nullptr, "gain_lin must be set");
+    const size_t K = ph ? (size_t)ph->n_phases : 1, P = B * K;
     const size_t n2 = pl.lambda2_stride ? n1 : 1;
-    const size_t n_sched = (size_t)yaman4_scratch_bytes((int64_t)B);
+    const size_t n_sched = (size_t)(ph ? yaman4_phase_scratch_bytes((int64_t)P) : yaman4_scratch_bytes((int64_t)B));
+    const size_t n_red = ph ? B : 0;
     size_t need = Carver::need(n1 * 8) + Carver::need(n2 * 8) + Carver::need(n3 * 8) +
-                  Carver::need(B * 8) /*gain*/ + Carver::need(B * 8) /*dbeta*/ +
-                  Carver::need(B * 4) /*valid*/ + Carver::need(B * 4) /*status*/ +
-                  Carver::need(B * 32) /*Pmax*/ + Carver::need(B * 64) /*A_end*/ +
-                  Carver::need(B * 32) /*omega*/ + Carver::need(n_sched);
+                  Carver::need(P * 8) /*gain*/ + Carver::need(B * 8) /*dbeta*/ +
+                  Carver::need(B * 4) /*valid*/ + Carver::need(P * 4) /*status*/ +
+                  Carver::need(P * 32) /*Pmax*/ + Carver::need(P * 64) /*A_end*/ +
+                  Carver::need(B * 32) /*omega*/ + Carver::need(n_sched) +
+                  Carver::need(K * 64) /*A0 table*/ + 2 * Carver::need(n_red * 8) + 3 * Carver::need(n_red * 4);
     void* ws = nullptr;
     FPA_TRY(workspace(device, 3, need, &ws));
     cudaStream_t st;
@@ -586,23 +612,31 @@ static int sweep_host_launch(const fpa_sweep_desc* d, int device, PendingSweep* 
     double*  l1   = cv.take<double>(n1);
     double*  l2   = cv.take<double>(n2);
     double*  l3   = cv.take<double>(n3);
-    double*  gain = cv.take<double>(B);
+    double*  gain = cv.take<double>(P);
     double*  db   = cv.take<double>(B);
     int32_t* va   = cv.take<int32_t>(B);
-    int32_t* stt  = cv.take<int32_t>(B);
-    double*  Pm   = cv.take<double>(B * 4);
-    double*  Ae   = cv.take<double>(B * 8);
+    int32_t* stt  = cv.take<int32_t>(P);
+    double*  Pm   = cv.take<double>(P * 4);
+    double*  Ae   = cv.take<double>(P * 8);
     double*  om   = cv.take<double>(B * 4);
     char*    sched = cv.take<char>(n_sched);
+    double*  tab  = cv.take<double>(K * 8);
+    double*  gmax = cv.take<double>(n_red);
+    double*  gmin = cv.take<double>(n_red);
+    int32_t* imax = cv.take<int32_t>(n_red);
+    int32_t* imin = cv.take<int32_t>(n_red);
+    int32_t* nfin = cv.take<int32_t>(n_red);
 
     FPA_TRY(up(l1, pl.lambda1, n1 * 8, st));
     FPA_TRY(up(l2, pl.lambda2, n2 * 8, st));
     FPA_TRY(up(l3, pl.lambda3, n3 * 8, st));
+    if (ph) FPA_TRY(up(tab, ph->A0_table, K * 64, st));
     // Outputs in pinned host memory are written by the kernel itself (each thread stores its results
     // when it finishes, so the PCIe traffic hides behind the integration of the other points; measured
     // with 8 GPUs storing into one host at once: 44.1 ms per 8e6-point sweep against 46.0 ms with staging
-    // and copies).  Pageable outputs go through the device workspace and a copy.
-    double*  m_gain = mapped(d->gain_lin);
+    // and copies).  Pageable outputs go through the device workspace and a copy.  The phase sweep keeps its gain map
+    // in device memory: the reduction kernel reads it there.
+    double*  m_gain = ph ? nullptr : mapped(d->gain_lin);
     double*  m_db   = mapped(pl.dbeta);
     int32_t* m_va   = mapped(pl.valid);
     int32_t* m_st   = mapped(d->status);
@@ -620,11 +654,30 @@ static int sweep_host_launch(const fpa_sweep_desc* d, int device, PendingSweep* 
     dd.Pmax         = d->Pmax ? (m_Pm ? m_Pm : Pm) : nullptr;
     dd.A_end        = d->A_end ? (m_Ae ? m_Ae : Ae) : nullptr;
     dd.status       = m_st ? m_st : stt;
-    FPA_TRY(sweep_dev(&dd, sched, (int64_t)n_sched, st));
+    if (ph) {
+        fpa_phase_sweep_desc pd = *ph;
+        pd.sweep    = dd;
+        pd.A0_table = tab;
+        pd.gain_max = ph->gain_max ? gmax : nullptr;
+        pd.gain_min = ph->gain_min ? gmin : nullptr;
+        pd.idx_max  = ph->idx_max ? imax : nullptr;
+        pd.idx_min  = ph->idx_min ? imin : nullptr;
+        pd.n_finite = ph->n_finite ? nfin : nullptr;
+        FPA_TRY(phase_sweep_dev(&pd, sched, (int64_t)n_sched, st));
+        ps->puser = *ph;
+        ps->gmax  = pd.gain_max;
+        ps->gmin  = pd.gain_min;
+        ps->imax  = pd.idx_max;
+        ps->imin  = pd.idx_min;
+        ps->nfin  = pd.n_finite;
+    } else {
+        FPA_TRY(sweep_dev(&dd, sched, (int64_t)n_sched, st));
+    }
     ps->st   = st;
     ps->B    = B;
+    ps->P    = P;
     ps->user = *d;
-    ps->gain = m_gain ? nullptr : gain;
+    ps->gain = (m_gain || !d->gain_lin) ? nullptr : gain;
     ps->db   = m_db ? nullptr : db;
     ps->va   = m_va ? nullptr : va;
     ps->om   = om;
@@ -637,32 +690,40 @@ static int sweep_host_launch(const fpa_sweep_desc* d, int device, PendingSweep* 
 static int sweep_host_collect(const PendingSweep& ps, int device) {
     if (!ps.st) return FPA_OK;
     FPA_TRY(use_device(device));
-    const size_t B = ps.B;
-    if (ps.gain) FPA_TRY(down(ps.user.gain_lin, ps.gain, B * 8, ps.st));
+    const size_t B = ps.B, P = ps.P;
+    if (ps.gain) FPA_TRY(down(ps.user.gain_lin, ps.gain, P * 8, ps.st));
     if (ps.db) FPA_TRY(down(ps.user.plan.dbeta, ps.db, B * 8, ps.st));
     if (ps.va) FPA_TRY(down(ps.user.plan.valid, ps.va, B * 4, ps.st));
     FPA_TRY(down(ps.user.plan.omega, ps.om, B * 32, ps.st));
-    if (ps.stt) FPA_TRY(down(ps.user.status, ps.stt, B * 4, ps.st));
-    if (ps.Pm) FPA_TRY(down(ps.user.Pmax, ps.Pm, B * 32, ps.st));
-    if (ps.Ae) FPA_TRY(down(ps.user.A_end, ps.Ae, B * 64, ps.st));
+    if (ps.stt) FPA_TRY(down(ps.user.status, ps.stt, P * 4, ps.st));
+    if (ps.Pm) FPA_TRY(down(ps.user.Pmax, ps.Pm, P * 32, ps.st));
+    if (ps.Ae) FPA_TRY(down(ps.user.A_end, ps.Ae, P * 64, ps.st));
+    if (ps.gmax) FPA_TRY(down(ps.puser.gain_max, ps.gmax, B * 8, ps.st));
+    if (ps.gmin) FPA_TRY(down(ps.puser.gain_min, ps.gmin, B * 8, ps.st));
+    if (ps.imax) FPA_TRY(down(ps.puser.idx_max, ps.imax, B * 4, ps.st));
+    if (ps.imin) FPA_TRY(down(ps.puser.idx_min, ps.imin, B * 4, ps.st));
+    if (ps.nfin) FPA_TRY(down(ps.puser.n_finite, ps.nfin, B * 4, ps.st));
     return FPA_OK;
 }
 
 int fpa_yaman4_sweep_host(const fpa_sweep_desc* d, int device) {
     PendingSweep ps;
-    FPA_TRY(sweep_host_launch(d, device, &ps));
+    FPA_TRY(sweep_host_launch(d, nullptr, device, &ps));
     FPA_TRY(sweep_host_collect(ps, device));
     if (ps.st) FPA_CUDA(cudaStreamSynchronize(ps.st));
     return FPA_OK;
 }
 
-int fpa_yaman4_sweep_multi_host(const fpa_sweep_desc* d, int n_devices, const int* devices) {
+// The grid split over several devices (see the header); `ph` set: a phase sweep, its K runs per grid point stay
+// together.
+static int sweep_multi_host(const fpa_sweep_desc* d, const fpa_phase_sweep_desc* ph, int n_devices, const int* devices) {
     FPA_REQUIRE(d != nullptr, "sweep descriptor is NULL");
     FPA_REQUIRE(n_devices >= 1 && n_devices <= 64 && devices != nullptr, "need 1..64 device ordinals");
     const int64_t n1 = d->plan.n1, n3 = d->plan.n3;
     FPA_REQUIRE(n1 >= 0 && n3 >= 0, "grid sizes must be >= 0");
     FPA_REQUIRE(d->first_point == 0 && d->n_sub_points == 0, "the multi-device sweep splits the whole grid itself");
-    if (n_devices == 1) return fpa_yaman4_sweep_host(d, devices[0]);
+    if (n_devices == 1) return ph ? fpa_yaman4_phase_sweep_host(ph, devices[0]) : fpa_yaman4_sweep_host(d, devices[0]);
+    const int64_t K = ph ? ph->n_phases : 1;
     // contiguous ranges of the FLATTENED grid, sizes differing by at most one: a 1-D sweep (n1 = 1) or a
     // grid with fewer pump rows than devices still uses every device
     PendingSweep pend[64];
@@ -679,13 +740,49 @@ int fpa_yaman4_sweep_multi_host(const fpa_sweep_desc* d, int n_devices, const in
             if (d->plan.omega) part.plan.omega = d->plan.omega + lo * 4;
             if (d->plan.dbeta) part.plan.dbeta = d->plan.dbeta + lo;
             if (d->plan.valid) part.plan.valid = d->plan.valid + lo;
-            if (d->gain_lin) part.gain_lin = d->gain_lin + lo;
-            if (d->Pmax) part.Pmax = d->Pmax + lo * 4;
-            if (d->A_end) part.A_end = d->A_end + lo * 8;
-            if (d->status) part.status = d->status + lo;
-            return sweep_host_launch(&part, devices[k], ps);
+            if (d->gain_lin) part.gain_lin = d->gain_lin + lo * K;
+            if (d->Pmax) part.Pmax = d->Pmax + lo * K * 4;
+            if (d->A_end) part.A_end = d->A_end + lo * K * 8;
+            if (d->status) part.status = d->status + lo * K;
+            if (!ph) return sweep_host_launch(&part, nullptr, devices[k], ps);
+            fpa_phase_sweep_desc pp = *ph;
+            if (ph->gain_max) pp.gain_max = ph->gain_max + lo;
+            if (ph->gain_min) pp.gain_min = ph->gain_min + lo;
+            if (ph->idx_max) pp.idx_max = ph->idx_max + lo;
+            if (ph->idx_min) pp.idx_min = ph->idx_min + lo;
+            if (ph->n_finite) pp.n_finite = ph->n_finite + lo;
+            return sweep_host_launch(&part, &pp, devices[k], ps);
         },
         sweep_host_collect);
+}
+
+int fpa_yaman4_sweep_multi_host(const fpa_sweep_desc* d, int n_devices, const int* devices) {
+    return sweep_multi_host(d, nullptr, n_devices, devices);
+}
+
+// ------------------------------------------------------------------ phase sweep
+int64_t fpa_yaman4_phase_sweep_scratch_bytes(int64_t n_points) { return yaman4_phase_scratch_bytes(n_points); }
+
+int fpa_yaman4_phase_sweep_dev(const fpa_phase_sweep_desc* d, void* scratch, int64_t scratch_bytes, void* stream) {
+    if (fpa_device_count() <= 0) {
+        set_error("no CUDA device is visible: libfpa_b200 has no CPU path");
+        return FPA_ERR_NO_DEVICE;
+    }
+    return phase_sweep_dev(d, scratch, scratch_bytes, static_cast<cudaStream_t>(stream));
+}
+
+int fpa_yaman4_phase_sweep_host(const fpa_phase_sweep_desc* d, int device) {
+    FPA_REQUIRE(d != nullptr, "phase sweep descriptor is NULL");
+    PendingSweep ps;
+    FPA_TRY(sweep_host_launch(&d->sweep, d, device, &ps));
+    FPA_TRY(sweep_host_collect(ps, device));
+    if (ps.st) FPA_CUDA(cudaStreamSynchronize(ps.st));
+    return FPA_OK;
+}
+
+int fpa_yaman4_phase_sweep_multi_host(const fpa_phase_sweep_desc* d, int n_devices, const int* devices) {
+    FPA_REQUIRE(d != nullptr, "phase sweep descriptor is NULL");
+    return sweep_multi_host(&d->sweep, d, n_devices, devices);
 }
 
 // ------------------------------------------------------------------ linear test RHS

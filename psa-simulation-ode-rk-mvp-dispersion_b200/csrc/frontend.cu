@@ -1,7 +1,8 @@
 // frontend.cu -- stand-alone Delta-beta table kernel (fpa_dbeta_table_*): frequency plan ->
 // validity -> Delta-beta for every point of a (pump x signal) wavelength grid.  The per-point
 // arithmetic lives in plan_point.cuh (shared with the fused sweep kernel in yaman4.cu), which
-// cites the reference lines it restates.
+// cites the reference lines it restates.  Also the per-grid-point reductions of the phase sweep
+// (fpa_yaman4_phase_sweep_*), which run right after its sweep kernel.
 #include "plan_point.cuh"
 
 namespace fpa {
@@ -80,6 +81,47 @@ int plan_launch(const fpa_plan_desc* d, double* dbeta_masked, cudaStream_t st) {
     plan_dbeta_kernel<<<(unsigned)((B + threads - 1) / threads), threads, 0, st>>>(p);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return cuda_fail(e, "plan_dbeta_kernel launch");
+    return FPA_OK;
+}
+
+// Per-grid-point reductions of a phase sweep (fpa_yaman4_phase_sweep_*): one thread per grid point over the K gains
+// gain[g*K .. g*K+K-1], with numpy's semantics -- nanmax / nanmin, nanargmax / nanargmin (first index on ties),
+// the count of non-NaN gains; an all-NaN row gives NaN, -1, -1, 0.
+__global__ void phase_reduce_kernel(int64_t G, int K, const double* gain, double* gmax, double* gmin, int32_t* imax,
+                                    int32_t* imin, int32_t* nfin) {
+    const int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (g >= G) return;
+    const double* r  = gain + g * K;
+    double        hi = qnan(), lo = qnan();
+    int           ih = -1, il = -1, n = 0;
+    for (int k = 0; k < K; ++k) {
+        const double v = r[k];
+        if (v != v) continue;
+        ++n;
+        if (ih < 0 || v > hi) {
+            hi = v;
+            ih = k;
+        }
+        if (il < 0 || v < lo) {
+            lo = v;
+            il = k;
+        }
+    }
+    if (gmax) gmax[g] = hi;
+    if (gmin) gmin[g] = lo;
+    if (imax) imax[g] = ih;
+    if (imin) imin[g] = il;
+    if (nfin) nfin[g] = n;
+}
+
+int phase_reduce_launch(int64_t G, int K, const double* gain, double* gmax, double* gmin, int32_t* imax, int32_t* imin,
+                        int32_t* nfin, cudaStream_t st) {
+    if (G == 0 || !(gmax || gmin || imax || imin || nfin)) return FPA_OK;
+    const int threads = 256;
+    phase_reduce_kernel<<<(unsigned)((G + threads - 1) / threads), threads, 0, st>>>(G, K, gain, gmax, gmin, imax, imin,
+                                                                                  nfin);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return cuda_fail(e, "phase_reduce_kernel launch");
     return FPA_OK;
 }
 

@@ -34,6 +34,8 @@
 
 #include <stdlib.h>
 
+#include <type_traits>
+
 namespace fpa {
 
 constexpr int kResync = 32;  // steps between exact sincos re-synchronisations of the phase
@@ -158,8 +160,11 @@ __device__ __noinline__ void write_invalid_point(const Yaman4Params& p, int64_t 
     if (p.status) p.status[b] = p.check ? 0 : FPA_POINT_OK;
 }
 
+// LAST: *plast = |A3|^2 of this sample, so that after the run it holds the LAST saved sample's signal power (the
+// phase sweep's "end" metric, which is not the fiber end when save_every does not divide the step count).
+template <bool LAST = false>
 __device__ __forceinline__ void save_sample(const double (&y)[8], double*& tr, double (&pm)[4], bool trace,
-                                            bool pmax) {
+                                            bool pmax, double* plast = nullptr) {
     if (trace) {
         // one 64-byte row [A1..A4] per saved sample: two 256-bit stores = two full 32 B sectors
         // (A_trace rows are 64-byte aligned whenever the buffer is 32-byte aligned; else 16 B stores)
@@ -180,6 +185,7 @@ __device__ __forceinline__ void save_sample(const double (&y)[8], double*& tr, d
             pm[j] = (P != P || pm[j] != pm[j]) ? qnan() : fmax(pm[j], P);
         }
     }
+    if (LAST) *plast = fma(y[5], y[5], y[4] * y[4]);
 }
 
 __device__ __forceinline__ void write_results(const Yaman4Params& p, int64_t b, const double (&y)[8],
@@ -207,11 +213,12 @@ __device__ __forceinline__ void write_results(const Yaman4Params& p, int64_t b, 
 // (0, n_steps); the z-segment scheduler (SegParams below) calls it once per segment with the
 // state, pm and bad of the previous segment.  i0 must be a multiple of kResync: the phase factor is
 // rebuilt by the exact sincos at the first step of the range, exactly where the whole-run loop rebuilds
-// it, so a segmented run is bit-identical to a whole one.
-template <bool TRACE, bool PMAX, bool LOSS, bool SEG = false>
+// it, so a segmented run is bit-identical to a whole one.  LAST: *plast follows the last saved sample (save_sample).
+template <bool TRACE, bool PMAX, bool LOSS, bool SEG = false, bool LAST = false>
 __device__ __forceinline__ int32_t fast_integrate(const Yaman4Params& p, int64_t b, double dbeta,
                                                   const Yaman4Coef& cf, double (&y)[8], double (&pm)[4],
-                                                  int i0_in = 0, int i1_in = 0, int32_t bad_in = FPA_POINT_OK) {
+                                                  int i0_in = 0, int i1_in = 0, int32_t bad_in = FPA_POINT_OK,
+                                                  double* plast = nullptr) {
     const int i0 = SEG ? i0_in : 0;
     const int i1 = SEG ? i1_in : p.n_steps;
     double* tr = nullptr;
@@ -221,7 +228,7 @@ __device__ __forceinline__ int32_t fast_integrate(const Yaman4Params& p, int64_t
 #pragma unroll
             for (int j = 0; j < 4; ++j) pm[j] = -1.0;  // |A|^2 >= 0: first sample always replaces it
         }
-        save_sample(y, tr, pm, TRACE, PMAX);
+        save_sample<LAST>(y, tr, pm, TRACE, PMAX, plast);
     }
 
     const double h = p.h, z0 = p.z0;
@@ -282,7 +289,7 @@ __device__ __forceinline__ int32_t fast_integrate(const Yaman4Params& p, int64_t
 
         if (--save_ctr == 0) {  // (i+1) % save_every == 0, integrators.py:137-140
             save_ctr = p.save_every;
-            save_sample(y, tr, pm, TRACE, PMAX);
+            save_sample<LAST>(y, tr, pm, TRACE, PMAX, plast);
         }
     }
     return bad;
@@ -339,6 +346,7 @@ struct SegParams {
     int           n_warps, n_seg, seg_steps;
 };
 constexpr int kSegDoubles = 13;  // y[8], pm[4], dbeta
+constexpr int kSegDoublesPhase = kSegDoubles + 1;  // the phase sweep adds the last saved signal power
 
 __device__ __forceinline__ int ld_acquire(const int* p) {
     int v;
@@ -441,6 +449,54 @@ struct SweepExtra {
     int        n_peers;
 };
 
+// The phase sweep (fpa_yaman4_phase_sweep_*): every grid point g runs K initial states, point b = g*K + k of the
+// launch is phase k of grid point g (phases fastest: the K runs of a grid point share warps and take the same
+// plan / validity branches).  A0_table[k] is make_initial_amplitudes(p_in, phase_in + phase_axis[k]*weights),
+// built on the host, so each run starts from the bits the plain sweep would use with that phase_in.
+struct PhaseSweepExtra : SweepExtra {
+    const double* A0_table;    // [K,4] complex128
+    int64_t       n_phases;    // K
+    int           last_saved;  // metric: 1 = |A3|^2 of the last saved sample, 0 = max over the saved samples
+};
+// The sweep kernels take their arguments as X = SweepExtra (plain sweep) or PhaseSweepExtra (phase sweep).
+template <typename X>
+constexpr bool kPhase = std::is_same<X, PhaseSweepExtra>::value;
+
+// (grid point, phase) of launch point b
+template <typename X>
+__device__ __forceinline__ void sweep_point(const X& x, int64_t b, int64_t& gp, int64_t& k) {
+    if constexpr (kPhase<X>) {
+        gp = b / x.n_phases;
+        k  = b - gp * x.n_phases;
+    } else {
+        gp = b;
+        k  = 0;
+    }
+}
+
+template <typename X>
+__device__ __forceinline__ void sweep_initial_state(const X& x, int64_t k, double (&y)[8]) {
+    if constexpr (kPhase<X>) {
+        const double2* a0 = reinterpret_cast<const double2*>(x.A0_table) + k * 4;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            const double2 v = a0[j];
+            y[2 * j] = v.x;
+            y[2 * j + 1] = v.y;
+        }
+    } else {
+#pragma unroll
+        for (int j = 0; j < 8; ++j) y[j] = x.A0[j];
+    }
+}
+
+// The signal power the gain is taken from: max over the saved samples, or (phase sweep, "end") the last saved one.
+template <typename X>
+__device__ __forceinline__ double sweep_metric(const X& x, const double (&pm)[4], double plast) {
+    if constexpr (kPhase<X>) return x.last_saved ? plast : pm[2];
+    return pm[2];
+}
+
 // The final gather of a multi-GPU sweep, fused into the kernel: the thread that finishes a point stores its gain
 // into the full-size map of every GPU of the box (NVLink peer stores, posted, 8 B per point and peer) while the
 // other points still integrate.
@@ -453,9 +509,10 @@ __device__ __forceinline__ void store_gain(const SweepExtra& x, int64_t b, doubl
     }
 }
 
-// Prologue of one scan point: frequency plan, validity, reported and integration Delta-beta; writes the
-// plan outputs.  Returns false for points the reference's per-point try/except turns into NaN.
-__device__ __forceinline__ bool sweep_prologue(const SweepExtra& x, int64_t b, double& db_run) {
+// Prologue of grid point b (of this launch): frequency plan, validity, reported and integration Delta-beta; writes
+// the plan outputs when `lead` (one lane per grid point of a phase sweep).  Returns false for points the
+// reference's per-point try/except turns into NaN.
+__device__ __forceinline__ bool sweep_prologue(const SweepExtra& x, int64_t b, double& db_run, bool lead = true) {
     const int64_t bg = b + x.first_point;
     const int64_t i1 = bg / x.plan.n3, i3 = bg - i1 * x.plan.n3;
     double w[4];
@@ -467,9 +524,9 @@ __device__ __forceinline__ bool sweep_prologue(const SweepExtra& x, int64_t b, d
         db_run = plan_dbeta(x.plan, x.beta_run, x.provided_run, w, ok_run);
         if (!ok_run) db_run = qnan();
     }
-    if (x.plan.dbeta) x.plan.dbeta[b] = db_report;
-    if (x.plan.valid) x.plan.valid[b] = ok ? 1 : 0;
-    if (x.plan.omega) {
+    if (lead && x.plan.dbeta) x.plan.dbeta[b] = db_report;
+    if (lead && x.plan.valid) x.plan.valid[b] = ok ? 1 : 0;
+    if (lead && x.plan.omega) {
         double2* o = reinterpret_cast<double2*>(x.plan.omega + b * 4);
         o[0] = make_double2(w[0], w[1]);
         o[1] = make_double2(w[2], w[3]);
@@ -488,9 +545,9 @@ __device__ __forceinline__ void sweep_invalid(const Yaman4Params& p, const Sweep
     store_gain(x, b, qn);
 }
 
-// Epilogue of an integrated point: status, optional end state / maxima, and the sweep's gain metric.
+// Epilogue of an integrated point: status, optional end state / maxima, and the sweep's gain metric P3 / p_in[2].
 __device__ __forceinline__ void sweep_epilogue(const Yaman4Params& p, const SweepExtra& x, int64_t b,
-                                               const double (&y)[8], const double (&pm)[4], int32_t bad) {
+                                               const double (&y)[8], const double (&pm)[4], int32_t bad, double P3) {
     if (p.check && bad == FPA_POINT_OK) {
         bool nf = false;
 #pragma unroll
@@ -507,56 +564,64 @@ __device__ __forceinline__ void sweep_epilogue(const Yaman4Params& p, const Swee
         o[0] = make_double2(pm[0], pm[1]);
         o[1] = make_double2(pm[2], pm[3]);
     }
-    // gain = max_saved |A3|^2 / p_in[2]; NaN for failed, non-finite or <= 0 (scan_mismtach.py:723-734)
+    // gain = max_saved |A3|^2 / p_in[2]; NaN for failed, non-finite or <= 0 (scan_mismtach.py:723-734).  The
+    // phase sweep's "end" metric takes P3 from the last saved sample under the same rule.
     double gain = qnan();
     if (!(p.check && bad != FPA_POINT_OK) && !nonfinite(pm[2])) {
-        const double q = pm[2] / x.p_signal;
+        const double q = P3 / x.p_signal;
         if (!nonfinite(q) && q > 0.0) gain = q;
     }
     store_gain(x, b, gain);
 }
 
-template <bool LOSS, int THREADS, int MIN_BLOCKS>
-__global__ void __launch_bounds__(THREADS, MIN_BLOCKS) yaman4_sweep_kernel(const Yaman4Params p, const SweepExtra x) {
+// X = PhaseSweepExtra: the phase sweep.
+template <bool LOSS, int THREADS, int MIN_BLOCKS, typename X>
+__global__ void __launch_bounds__(THREADS, MIN_BLOCKS) yaman4_sweep_kernel(const Yaman4Params p, const X x) {
+    constexpr bool PHASE = kPhase<X>;
     const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= p.n_points) return;
+    int64_t gp, k;
+    sweep_point(x, b, gp, k);
     double db_run;
-    if (!sweep_prologue(x, b, db_run)) {
+    if (!sweep_prologue(x, gp, db_run, k == 0)) {
         sweep_invalid(p, x, b);
         return;
     }
     double y[8];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) y[j] = x.A0[j];
-    double        pm[4] = {0.0, 0.0, 0.0, 0.0};
-    const int32_t bad = fast_integrate<false, true, LOSS>(p, b, db_run, p.coef, y, pm);
-    sweep_epilogue(p, x, b, y, pm, bad);
+    sweep_initial_state(x, k, y);
+    double        pm[4] = {0.0, 0.0, 0.0, 0.0}, plast = 0.0;
+    const int32_t bad = fast_integrate<false, true, LOSS, false, PHASE>(p, b, db_run, p.coef, y, pm, 0, 0, FPA_POINT_OK,
+                                                                        &plast);
+    sweep_epilogue(p, x, b, y, pm, bad, sweep_metric(x, pm, plast));
 }
 
 // ------------------------------------------------------------------ fused sweep, z-segment scheduler
 // The sweep kernel above as a persistent kernel on the z-segment scheduler: prologue at segment 0, gain
-// epilogue at the last segment, the point's integration Delta-beta travels with its state.
-template <bool LOSS, int THREADS, int MIN_BLOCKS>
+// epilogue at the last segment, the point's integration Delta-beta travels with its state (phase sweep: and the
+// last saved signal power, record kSegDoubles of the state).
+template <bool LOSS, int THREADS, int MIN_BLOCKS, typename X>
 __global__ void __launch_bounds__(THREADS, MIN_BLOCKS)
-    yaman4_sweep_seg_kernel(const Yaman4Params p, const SweepExtra x, const SegParams g) {
+    yaman4_sweep_seg_kernel(const Yaman4Params p, const X x, const SegParams g) {
+    constexpr bool PHASE = kPhase<X>;
     const int lane = threadIdx.x & 31;
     int       seg, w;
     while (seg_next_item(g, lane, seg, w)) {
         const int64_t b = (int64_t)w * 32 + lane;
         const bool    last = seg == g.n_seg - 1;
         if (b < p.n_points) {
-            double  y[8], pm[4] = {0.0, 0.0, 0.0, 0.0}, db_run;
+            double  y[8], pm[4] = {0.0, 0.0, 0.0, 0.0}, db_run, plast = 0.0;
             int32_t bad = FPA_POINT_OK;
             bool    run;
             double* const st = g.state + b;
             if (seg == 0) {
-                run = sweep_prologue(x, b, db_run);
+                int64_t gp, k;
+                sweep_point(x, b, gp, k);
+                run = sweep_prologue(x, gp, db_run, k == 0);
                 if (!run) {
                     sweep_invalid(p, x, b);
                     db_run = qnan();
                 }
-#pragma unroll
-                for (int j = 0; j < 8; ++j) y[j] = x.A0[j];
+                sweep_initial_state(x, k, y);
             } else {
                 db_run = __ldcg(st + 12 * g.n_pad);
                 run = !nonfinite(db_run);
@@ -565,14 +630,15 @@ __global__ void __launch_bounds__(THREADS, MIN_BLOCKS)
                     for (int j = 0; j < 8; ++j) y[j] = __ldcg(st + j * g.n_pad);
 #pragma unroll
                     for (int j = 0; j < 4; ++j) pm[j] = __ldcg(st + (8 + j) * g.n_pad);
+                    if (PHASE) plast = __ldcg(st + kSegDoubles * g.n_pad);
                     bad = __ldcg(g.bad + b);
                 }
             }
             if (run) {
                 const int i0 = seg * g.seg_steps;
                 const int i1 = last ? p.n_steps : i0 + g.seg_steps;
-                bad = fast_integrate<false, true, LOSS, true>(p, b, db_run, p.coef, y, pm, i0, i1, bad);
-                if (last) sweep_epilogue(p, x, b, y, pm, bad);
+                bad = fast_integrate<false, true, LOSS, true, PHASE>(p, b, db_run, p.coef, y, pm, i0, i1, bad, &plast);
+                if (last) sweep_epilogue(p, x, b, y, pm, bad, sweep_metric(x, pm, plast));
             }
             if (!last) {
                 __stcg(st + 12 * g.n_pad, db_run);
@@ -581,6 +647,7 @@ __global__ void __launch_bounds__(THREADS, MIN_BLOCKS)
                     for (int j = 0; j < 8; ++j) __stcg(st + j * g.n_pad, y[j]);
 #pragma unroll
                     for (int j = 0; j < 4; ++j) __stcg(st + (8 + j) * g.n_pad, pm[j]);
+                    if (PHASE) __stcg(st + kSegDoubles * g.n_pad, plast);
                     __stcg(g.bad + b, bad);
                 }
             }
@@ -722,12 +789,15 @@ constexpr int kSegStepsShort = 64, kSegStepsLong = 128, kSegMaxWaves = 8;
 // ---- z-segment scheduler: scratch layout and launch geometry
 static size_t seg_align(size_t v) { return (v + 255) & ~(size_t)255; }
 
-int64_t yaman4_scratch_bytes(int64_t n_points) {
+// seg_doubles: doubles of a point's state record (kSegDoubles, or kSegDoublesPhase for the phase sweep)
+static int64_t scratch_bytes(int64_t n_points, int seg_doubles) {
     if (n_points <= 0) return 0;
     const size_t n_warps = (size_t)((n_points + 31) / 32), n_pad = n_warps * 32;
-    return (int64_t)(256 + seg_align(n_warps * sizeof(int)) + seg_align(n_pad * kSegDoubles * sizeof(double)) +
+    return (int64_t)(256 + seg_align(n_warps * sizeof(int)) + seg_align(n_pad * seg_doubles * sizeof(double)) +
                      seg_align(n_pad * sizeof(int32_t)));
 }
+int64_t yaman4_scratch_bytes(int64_t n_points) { return scratch_bytes(n_points, kSegDoubles); }
+int64_t yaman4_phase_scratch_bytes(int64_t n_points) { return scratch_bytes(n_points, kSegDoublesPhase); }
 
 static int env_int(const char* name, int dflt) {
     const char* v = getenv(name);
@@ -750,7 +820,7 @@ static int resident_ctas(Kernel kernel, int threads) {
 // FPA_SWEEP_SEG=0 forces the whole-run kernels, =2 lifts the kSegMaxWaves cap, FPA_SWEEP_SEG_STEPS overrides the
 // segment length (tools, tests).
 static int seg_plan(int64_t B, int64_t n_steps, int ctas, int threads, void* scratch, int64_t scratch_bytes,
-                    cudaStream_t st, SegParams& g, bool& use_seg) {
+                    cudaStream_t st, SegParams& g, bool& use_seg, int seg_doubles = kSegDoubles) {
     const int64_t n_warps = (B + 31) / 32, resident_warps = (int64_t)ctas * (threads / 32);
     // segment length: 64 steps below two waves of the resident warps, else 128; half that for runs of fewer than
     // 1 000 steps, which would otherwise have too few segments to even out the tail (profiles/r2_seg_tune.txt:
@@ -760,7 +830,7 @@ static int seg_plan(int64_t B, int64_t n_steps, int ctas, int threads, void* scr
     int seg_steps = env_int("FPA_SWEEP_SEG_STEPS", seg_default);
     seg_steps = (seg_steps + kResync - 1) / kResync * kResync;
     if (seg_steps < kResync) seg_steps = kResync;
-    use_seg = env_int("FPA_SWEEP_SEG", 1) != 0 && scratch != nullptr && scratch_bytes >= yaman4_scratch_bytes(B) &&
+    use_seg = env_int("FPA_SWEEP_SEG", 1) != 0 && scratch != nullptr && scratch_bytes >= ::fpa::scratch_bytes(B, seg_doubles) &&
               n_warps >= resident_warps && (n_warps < kSegMaxWaves * resident_warps || env_int("FPA_SWEEP_SEG", 1) == 2) &&
               n_steps >= 2 * (int64_t)seg_steps &&
               n_warps * ((n_steps + seg_steps - 1) / seg_steps) < 4000000000LL;
@@ -771,7 +841,7 @@ static int seg_plan(int64_t B, int64_t n_steps, int ctas, int threads, void* scr
     g.state     = reinterpret_cast<double*>(base + 256 + seg_align((size_t)n_warps * sizeof(int)));
     g.n_pad     = n_warps * 32;
     g.bad       = reinterpret_cast<int32_t*>(reinterpret_cast<char*>(g.state) +
-                                             seg_align((size_t)g.n_pad * kSegDoubles * sizeof(double)));
+                                             seg_align((size_t)g.n_pad * seg_doubles * sizeof(double)));
     g.n_warps   = (int)n_warps;
     g.seg_steps = seg_steps;
     g.n_seg     = (int)((n_steps + seg_steps - 1) / seg_steps);
@@ -874,20 +944,22 @@ int yaman4_launch(const fpa_yaman4_desc* d, cudaStream_t st) {
 // gamma/alpha/z_max/dz per length unit, exactly as fpa_sweep_desc carries them.
 int plan_fill(const fpa_plan_desc* d, PlanParams& p);
 
-int yaman4_sweep_launch(const fpa_sweep_desc* d, void* scratch, int64_t scratch_bytes, cudaStream_t st) {
+// Checks a sweep descriptor and fills the kernel arguments for its n_grid grid points (the whole grid or the
+// sub-range) x n_phases runs each; the plain sweep is n_phases = 1.
+static int sweep_setup(const fpa_sweep_desc* d, int64_t n_phases, Yaman4Params& p, SweepExtra& x, int64_t& n_grid) {
     FPA_REQUIRE(d != nullptr, "sweep descriptor is NULL");
     if (d->flags & FPA_PHASE_EXACT) {
         set_error("FPA_PHASE_EXACT is not available for the fused sweep: build the table with fpa_dbeta_table_* "
                   "and integrate with fpa_yaman4_rk4_batch_* (which honours the flag)");
         return FPA_ERR_UNSUPPORTED;
     }
-    SweepExtra x;
     int rc = plan_fill(&d->plan, x.plan);
     if (rc != FPA_OK) return rc;
     const int64_t grid = d->plan.n1 * d->plan.n3;
     FPA_REQUIRE(d->first_point >= 0 && d->n_sub_points >= 0 && d->first_point + d->n_sub_points <= grid,
                 "first_point / n_sub_points must select a range of the n1*n3 grid");
-    const int64_t B = (d->first_point == 0 && d->n_sub_points == 0) ? grid : d->n_sub_points;
+    n_grid = (d->first_point == 0 && d->n_sub_points == 0) ? grid : d->n_sub_points;
+    const int64_t B = n_grid * n_phases;
     FPA_REQUIRE(d->gain_lin != nullptr || B == 0, "gain_lin must be set");
     FPA_REQUIRE(d->length_scale == 1.0 || d->length_scale == 1000.0, "length_scale must be 1 or 1000");
     FPA_REQUIRE(d->z_max > 0.0, "z_max must be positive");
@@ -913,7 +985,6 @@ int yaman4_sweep_launch(const fpa_sweep_desc* d, void* scratch, int64_t scratch_
         FPA_REQUIRE(q >= d->n_peers || x.peer[q] != nullptr, "peer_gain[%d] is NULL", q);
     }
 
-    Yaman4Params p;
     memset(&p, 0, sizeof(p));
     p.n_points   = B;
     p.A_end      = d->A_end;
@@ -927,30 +998,67 @@ int yaman4_sweep_launch(const fpa_sweep_desc* d, void* scratch, int64_t scratch_
     p.check      = (d->flags & FPA_CHECK_NAN) ? 1 : 0;
     p.n_saved    = fpa_n_saved(n_steps, d->save_every);
     p.coef       = make_coef(d->gamma / sc, d->alpha / sc, p.h);
+    p.lossless   = d->alpha == 0.0 ? 1 : 0;
+    return FPA_OK;
+}
 
-    // ---- z-segment scheduler when the batch is a wave or more, else the whole-run kernel
-    const bool lossless = d->alpha == 0.0;
-    const int  ctas = lossless ? resident_ctas(yaman4_sweep_seg_kernel<false, kFastThreads, kSweepMinBlocks>, kFastThreads)
-                               : resident_ctas(yaman4_sweep_seg_kernel<true, kFastThreads, kSweepMinBlocks>, kFastThreads);
-    SegParams  g;
-    bool       use_seg = false;
-    rc = seg_plan(B, n_steps, ctas, kFastThreads, scratch, scratch_bytes, st, g, use_seg);
+// z-segment scheduler when the batch is a wave or more, else the whole-run kernel
+template <typename X>
+static int sweep_run(const Yaman4Params& p, const X& x, void* scratch, int64_t scratch_bytes, cudaStream_t st) {
+    constexpr bool PHASE = kPhase<X>;
+    const int64_t B = p.n_points;
+    const bool    lossless = p.lossless != 0;
+    const int ctas = lossless ? resident_ctas(yaman4_sweep_seg_kernel<false, kFastThreads, kSweepMinBlocks, X>, kFastThreads)
+                              : resident_ctas(yaman4_sweep_seg_kernel<true, kFastThreads, kSweepMinBlocks, X>, kFastThreads);
+    SegParams g;
+    bool      use_seg = false;
+    int rc = seg_plan(B, p.n_steps, ctas, kFastThreads, scratch, scratch_bytes, st, g, use_seg,
+                      PHASE ? kSegDoublesPhase : kSegDoubles);
     if (rc != FPA_OK) return rc;
     if (use_seg) {
         if (lossless)
-            yaman4_sweep_seg_kernel<false, kFastThreads, kSweepMinBlocks><<<ctas, kFastThreads, 0, st>>>(p, x, g);
+            yaman4_sweep_seg_kernel<false, kFastThreads, kSweepMinBlocks, X><<<ctas, kFastThreads, 0, st>>>(p, x, g);
         else
-            yaman4_sweep_seg_kernel<true, kFastThreads, kSweepMinBlocks><<<ctas, kFastThreads, 0, st>>>(p, x, g);
+            yaman4_sweep_seg_kernel<true, kFastThreads, kSweepMinBlocks, X><<<ctas, kFastThreads, 0, st>>>(p, x, g);
     } else {
         const long blocks = (long)((B + kFastThreads - 1) / kFastThreads);
         if (lossless)
-            yaman4_sweep_kernel<false, kFastThreads, kSweepMinBlocks><<<blocks, kFastThreads, 0, st>>>(p, x);
+            yaman4_sweep_kernel<false, kFastThreads, kSweepMinBlocks, X><<<blocks, kFastThreads, 0, st>>>(p, x);
         else
-            yaman4_sweep_kernel<true, kFastThreads, kSweepMinBlocks><<<blocks, kFastThreads, 0, st>>>(p, x);
+            yaman4_sweep_kernel<true, kFastThreads, kSweepMinBlocks, X><<<blocks, kFastThreads, 0, st>>>(p, x);
     }
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return cuda_fail(e, "yaman4_sweep_kernel launch");
     return FPA_OK;
+}
+
+int yaman4_sweep_launch(const fpa_sweep_desc* d, void* scratch, int64_t scratch_bytes, cudaStream_t st) {
+    Yaman4Params p;
+    SweepExtra   x;
+    int64_t      n_grid;
+    int rc = sweep_setup(d, 1, p, x, n_grid);
+    if (rc != FPA_OK || n_grid == 0) return rc;
+    return sweep_run(p, x, scratch, scratch_bytes, st);
+}
+
+// The sweep kernels with the phase axis: n_grid * K points, plan outputs per grid point, everything else per point.
+int yaman4_phase_sweep_launch(const fpa_phase_sweep_desc* d, void* scratch, int64_t scratch_bytes, cudaStream_t st) {
+    FPA_REQUIRE(d != nullptr, "phase sweep descriptor is NULL");
+    Yaman4Params    p;
+    PhaseSweepExtra x;
+    int64_t         n_grid;
+    const int64_t   K = d->n_phases;
+    if (d->sweep.flags & FPA_PHASE_EXACT) return sweep_setup(&d->sweep, 1, p, x, n_grid);  // FPA_ERR_UNSUPPORTED
+    FPA_REQUIRE(d->sweep.n_peers == 0, "the phase sweep has no peer-store gather: n_peers must be 0");
+    FPA_REQUIRE(K >= 1 && K <= FPA_MAX_PHASES, "n_phases must be in [1, %d]", FPA_MAX_PHASES);
+    FPA_REQUIRE(d->A0_table != nullptr, "A0_table must be set");
+    FPA_REQUIRE(d->metric == FPA_GAIN_MAX_SAVED || d->metric == FPA_GAIN_LAST_SAVED, "unknown gain metric %d", d->metric);
+    int rc = sweep_setup(&d->sweep, K, p, x, n_grid);
+    if (rc != FPA_OK || n_grid == 0) return rc;
+    x.A0_table   = d->A0_table;
+    x.n_phases   = K;
+    x.last_saved = d->metric == FPA_GAIN_LAST_SAVED ? 1 : 0;
+    return sweep_run(p, x, scratch, scratch_bytes, st);
 }
 
 int yaman4_rhs_launch(int64_t B, const double* z, const double* A, const double* gamma,

@@ -169,6 +169,112 @@ def sweep_gain_2d(*, cfg: SimulationConfig, lambda_p1_m, lambda_p2_m, lambda_sig
     return out
 
 
+def _phase_axis(phase_axis, phase_weights):
+    ax = np.asarray(phase_axis, dtype=float)
+    if ax.ndim != 1 or ax.size == 0:
+        raise ValueError("phase_axis must be a non-empty 1D sequence of phases (rad)")
+    if ax.size > _lib.MAX_PHASES:
+        raise ValueError(f"phase_axis may hold at most {_lib.MAX_PHASES} phases, got {ax.size}")
+    if not np.all(np.isfinite(ax)):
+        raise ValueError("phase_axis must contain finite values")
+    w = np.asarray(list(phase_weights), dtype=float)
+    if w.shape != (4,):
+        raise ValueError(f"phase_weights must have shape (4,), got {w.shape}")
+    if not np.all(np.isfinite(w)):
+        raise ValueError("phase_weights must contain finite values")
+    return ax, w
+
+
+def phase_sweep_inputs(p_in, phase_in, phase_axis, phase_weights=(0.0, 0.0, 1.0, 0.0)):
+    """(A0_table [K,4] complex128, phases [K,4], relative_phase [K]) of a phase sweep: phase index k starts from
+    make_initial_amplitudes(p_in, phase_in + phase_axis[k] * phase_weights); its relative phase is
+    theta_k = phi_p1 + phi_p2 - phi_s - phi_i of that input phase."""
+    p0, ph0 = _powers_and_phases(p_in, phase_in)
+    ax, w = _phase_axis(phase_axis, phase_weights)
+    base = np.zeros(4) if ph0 is None else ph0
+    phases = np.stack([base + ax[k] * w for k in range(ax.size)])
+    table = np.stack([make_initial_amplitudes(p0, phases[k]) for k in range(ax.size)])
+    theta = phases[:, 0] + phases[:, 1] - phases[:, 2] - phases[:, 3]
+    return np.ascontiguousarray(table, dtype=np.complex128), phases, theta
+
+
+def sweep_phase_gain_2d(*, cfg: SimulationConfig, lambda_p1_m, lambda_p2_m, lambda_signal_m, gamma: float,
+                        alpha: float, p_in, phase_in=None, phase_axis, phase_weights=(0.0, 0.0, 1.0, 0.0),
+                        gain_metric: GainMode = "end", dispersion: Optional[DispersionParams] = None,
+                        phase_matching_cfg: Optional[PhaseMatchingConfig] = None, length_unit: str = "m",
+                        gain_unit: str = "dB", device: Optional[int] = None, devices=None) -> dict:
+    """Phase-sensitive gain on the grid lambda_p1[n1] x lambda_signal[n3] x phase_axis[K]: the wavelength grid of
+    `sweep_gain_2d`, and for every grid point K runs, run k starting from the input phase
+    phase_in + phase_axis[k] * phase_weights (default weights sweep the signal phase).  One kernel launch per GPU
+    plus one reduction launch.
+
+    gain_metric: 'end' = |A3|^2 of the last saved sample / p_in[2] (the reference's Pz[-1]), 'max' = max over the
+    saved samples (the metric of `sweep_gain_2d`); NaN for failed, non-finite or <= 0 runs.
+
+    Returns dict(gain [n1,n3,K] in gain_unit, gain_lin [n1,n3,K], status [n1,n3,K]; per grid point [n1,n3]:
+    gain_max / gain_min (linear; numpy nanmax / nanmin over the K phases), idx_max / idx_min (nanargmax /
+    nanargmin, -1 where all K are NaN), phase_at_max / phase_at_min (phase_axis at those indices, NaN there),
+    n_finite, extinction_db = 10 log10(gain_max / gain_min), dbeta, valid; relative_phase [K] = the theta_k of
+    each phase index; n_steps).  A single plan (n1 = n3 = 1) is the G(theta) curve of one amplifier."""
+    lam3 = _signal_axis(lambda_signal_m)
+    lam1 = np.atleast_1d(np.asarray(lambda_p1_m, dtype=float))
+    lam2 = np.atleast_1d(np.asarray(lambda_p2_m, dtype=float))
+    p0, _ = _powers_and_phases(p_in, phase_in)
+    table, _, theta = phase_sweep_inputs(p_in, phase_in, phase_axis, phase_weights)
+    ax = np.asarray(phase_axis, dtype=float)
+    K = ax.size
+    unit = _norm_choice(gain_unit, ("db", "linear"), "gain_unit must be 'dB' or 'linear'")
+    if gain_metric not in ("end", "max"):
+        raise ValueError(f"Unknown gain_metric={gain_metric!r}. Use 'end' or 'max'.")
+
+    pm_cfg = phase_matching_cfg
+    if pm_cfg is None:
+        try:
+            pm_cfg = _default_phase_matching_cfg(dispersion=dispersion, beta_legacy=None)
+        except ValueError:
+            pm_cfg = None
+    n1, n3 = lam1.size, lam3.size
+    if pm_cfg is None or not _run_constants_ok(cfg, gamma, alpha, dispersion, pm_cfg, length_unit):
+        # every run would raise -> all NaN; dbeta is still reported when it can be computed
+        nan = np.full((n1, n3), np.nan)
+        out = {"gain_lin": np.full((n1, n3, K), np.nan), "gain_max": nan, "gain_min": nan.copy(),
+               "idx_max": np.full((n1, n3), -1, np.int32), "idx_min": np.full((n1, n3), -1, np.int32),
+               "n_finite": np.zeros((n1, n3), np.int32), "dbeta": nan.copy(),
+               "valid": np.zeros((n1, n3), np.int32), "status": np.full((n1, n3, K), -1, np.int32), "n_steps": 0}
+        if isinstance(pm_cfg, PhaseMatchingConfig) and (dispersion is not None or
+                                                        pm_cfg.method == PhaseMatchingMethod.PROVIDED):
+            plan, keep = _device.new_plan_desc(lam1, lam2, lam3)
+            fill_plan_desc(plan, dispersion, pm_cfg)
+            out["dbeta"] = _device.dbeta_table(plan, device=device)["dbeta"]
+    else:
+        s = _length_scale_to_m(length_unit)
+        d = _lib.PhaseSweepDesc()
+        plan, keep = _device.new_plan_desc(lam1, lam2, lam3)
+        fill_plan_desc(plan, dispersion, pm_cfg)
+        w = d.sweep
+        w.plan = plan
+        w.p_signal = float(p0[2])
+        w.gamma, w.alpha = float(gamma), float(alpha)
+        w.z_max, w.dz = float(cfg.z_max), float(cfg.dz)
+        w.length_scale = s
+        w.save_every = int(cfg.save_every)
+        w.flags = _lib.CHECK_NAN if cfg.check_nan else 0
+        d.n_phases = K
+        d.A0_table = _lib.ptr(table)
+        d.metric = _lib.GAIN_LAST_SAVED if gain_metric == "end" else _lib.GAIN_MAX_SAVED
+        out = _device.phase_sweep(d, device=device, devices=devices)
+        out["n_steps"] = int(round(float(cfg.z_max) * s / (float(cfg.dz) * s)))
+    g = out["gain_lin"]
+    with np.errstate(invalid="ignore", divide="ignore"):
+        out["gain"] = g if unit == "linear" else 10.0 * np.log10(g)
+        out["extinction_db"] = 10.0 * np.log10(out["gain_max"] / out["gain_min"])
+    for key in ("max", "min"):
+        idx = out[f"idx_{key}"]
+        out[f"phase_at_{key}"] = np.where(idx >= 0, ax[np.maximum(idx, 0)], np.nan)
+    out["relative_phase"] = theta
+    return out
+
+
 def _sweep_1d(cfg, lambda_p1_m, lambda_p2_m, lam3, gamma, alpha, p_in, phase_in, dispersion,
               phase_matching_cfg, length_unit, gain_unit):
     r = sweep_gain_2d(cfg=cfg, lambda_p1_m=[float(lambda_p1_m)], lambda_p2_m=[float(lambda_p2_m)],
