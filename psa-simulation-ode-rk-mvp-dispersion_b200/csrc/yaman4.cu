@@ -28,6 +28,13 @@
 //        step (2 rotations per step) and is re-synchronised with an exact sincos every 32 steps,
 //        instead of the reference's 8 complex exp() per step.
 //    Measured against the oracle: <= 1e-13 relative on |A|^2 after 10 000 steps at 45 dB gain.
+//    Symmetric sweeps (the plain fused sweep only): when the initial state has A1 == A2 and A3 == A4 bit for
+//    bit -- the standard dual-pump set-up, p_in = [P, P, Ps, Ps] with no input phase -- every rounded
+//    operation of stage() on wave 2 (4) is the one on wave 1 (3) with the same operands, so the state stays
+//    on that subspace for the whole fiber.  stage_sym() / fast_integrate<..., SYM> then integrate the
+//    4-double state (x1, y1, x3, y3) with the same expressions in the same operand order: 186 instead of
+//    298 FP64 instructions per lossy step and the same bits (DESIGN.md §4.1c).  The launcher decides by a
+//    memcmp of A0's bit patterns; FPA_SWEEP_SYM=0 forces the 4-wave kernels.
 //  * yaman4_exact_kernel -- FPA_PHASE_EXACT or an explicit z-grid: the reference's arithmetic
 //    structure step by step (h_i by subtraction, sincos at z, z+h/2, z+h, k_j formed, y + h/6*(..)).
 #include "plan_point.cuh"
@@ -132,6 +139,51 @@ __device__ __forceinline__ void stage(const double (&in)[8], const double (&base
     }
 }
 
+// stage() on a symmetric state, in = (x1, y1, x3, y3) standing for (x1, y1, x1, y1, x3, y3, x3, y3), base the
+// same way.  Every rounded operation is the one stage() performs with x2 -> x1, y2 -> y1, x4 -> x3, y4 -> y3:
+// P2 == P1, P4 == P3, G2 == G1, G4 == G3, and out[2], out[3], out[6], out[7] of stage() are the FMA chains of
+// out[0], out[1], out[4], out[5] on the same operands, so they are not computed.  S is stage()'s
+// (P1 + P2) + (P3 + P4) with that substitution, the same two adds and the same rounding.  Every product and
+// sum is spelled out as in stage(); nothing is left to contraction.
+template <bool LOSS = true>
+__device__ __forceinline__ void stage_sym(const double (&in)[4], const double (&base)[4], double qr, double qi,
+                                          double cg, double c2g, double cn, double (&out)[4], double& S) {
+    const double x1 = in[0], y1 = in[1], x3 = in[2], y3 = in[3];
+    const double P1 = fma(y1, y1, x1 * x1);
+    const double P3 = fma(y3, y3, x3 * x3);
+    S = (P1 + P1) + (P3 + P3);
+    const double c2 = c2g * S;
+    const double G1 = fma(-cg, P1, c2);
+    const double G3 = fma(-cg, P3, c2);
+    const double Ur = fma(-y3, y3, x3 * x3), Ui = fma(x3, y3, y3 * x3);  // A3*A4
+    const double Vr = fma(-y1, y1, x1 * x1), Vi = fma(x1, y1, y1 * x1);  // A1*A2
+    const double Wr = fma(-qi, Ui, qr * Ur), Wi = fma(qr, Ui, qi * Ur);
+    const double Zr = fma(qi, Vi, qr * Vr),  Zi = fma(qr, Vi, -(qi * Vr));
+    if (LOSS) {
+        out[0] = fma(-G1, y1, fma(y1, Wr, fma(-x1, Wi, fma(cn, x1, base[0]))));
+        out[1] = fma(G1, x1, fma(x1, Wr, fma(y1, Wi, fma(cn, y1, base[1]))));
+        out[2] = fma(-G3, y3, fma(y3, Zr, fma(-x3, Zi, fma(cn, x3, base[2]))));
+        out[3] = fma(G3, x3, fma(x3, Zr, fma(y3, Zi, fma(cn, y3, base[3]))));
+    } else {
+        out[0] = fma(-G1, y1, fma(y1, Wr, fma(-x1, Wi, base[0])));
+        out[1] = fma(G1, x1, fma(x1, Wr, fma(y1, Wi, base[1])));
+        out[2] = fma(-G3, y3, fma(y3, Zr, fma(-x3, Zi, base[2])));
+        out[3] = fma(G3, x3, fma(x3, Zr, fma(y3, Zi, base[3])));
+    }
+}
+
+// One RK4 stage on the full state or (4 doubles) on the symmetric half of one.
+template <bool LOSS>
+__device__ __forceinline__ void rk_stage(const double (&in)[8], const double (&base)[8], double qr, double qi,
+                                         double cg, double c2g, double cn, double (&out)[8], double& S) {
+    stage<LOSS>(in, base, qr, qi, cg, c2g, cn, out, S);
+}
+template <bool LOSS>
+__device__ __forceinline__ void rk_stage(const double (&in)[4], const double (&base)[4], double qr, double qi,
+                                         double cg, double c2g, double cn, double (&out)[4], double& S) {
+    stage_sym<LOSS>(in, base, qr, qi, cg, c2g, cn, out, S);
+}
+
 __device__ __forceinline__ void load_state(const Yaman4Params& p, int64_t b, double (&y)[8]) {
     const double2* a0 = reinterpret_cast<const double2*>(p.A0) + b * p.A0_stride * 4;
 #pragma unroll
@@ -188,6 +240,21 @@ __device__ __forceinline__ void save_sample(const double (&y)[8], double*& tr, d
     if (LAST) *plast = fma(y[5], y[5], y[4] * y[4]);
 }
 
+// save_sample of a symmetric state (x1, y1, x3, y3): the running maxima of waves 1 and 3 (pm[1] and pm[3] would be
+// the same computation on the same bits; the epilogue copies them).  No trace.
+template <bool LAST = false>
+__device__ __forceinline__ void save_sample(const double (&y)[4], double*&, double (&pm)[4], bool, bool pmax,
+                                            double* = nullptr) {
+    static_assert(!LAST, "the symmetric path has no last-sample metric");
+    if (pmax) {
+#pragma unroll
+        for (int j = 0; j < 4; j += 2) {
+            const double P = fma(y[j + 1], y[j + 1], y[j] * y[j]);
+            pm[j] = (P != P || pm[j] != pm[j]) ? qnan() : fmax(pm[j], P);
+        }
+    }
+}
+
 __device__ __forceinline__ void write_results(const Yaman4Params& p, int64_t b, const double (&y)[8],
                                               const double (&pm)[4], bool pmax, int32_t bad) {
     if (p.check && bad == FPA_POINT_OK) {
@@ -214,11 +281,17 @@ __device__ __forceinline__ void write_results(const Yaman4Params& p, int64_t b, 
 // state, pm and bad of the previous segment.  i0 must be a multiple of kResync: the phase factor is
 // rebuilt by the exact sincos at the first step of the range, exactly where the whole-run loop rebuilds
 // it, so a segmented run is bit-identical to a whole one.  LAST: *plast follows the last saved sample (save_sample).
-template <bool TRACE, bool PMAX, bool LOSS, bool SEG = false, bool LAST = false>
+// SYM: y is the symmetric half (x1, y1, x3, y3) of a state with A1 == A2, A3 == A4 (stage_sym); pm[0] and pm[2] are
+// kept, pm[1] and pm[3] are left to the caller.
+template <bool SYM>
+constexpr int kStateLen = SYM ? 4 : 8;
+template <bool TRACE, bool PMAX, bool LOSS, bool SEG = false, bool LAST = false, bool SYM = false>
 __device__ __forceinline__ int32_t fast_integrate(const Yaman4Params& p, int64_t b, double dbeta,
-                                                  const Yaman4Coef& cf, double (&y)[8], double (&pm)[4],
+                                                  const Yaman4Coef& cf, double (&y)[kStateLen<SYM>], double (&pm)[4],
                                                   int i0_in = 0, int i1_in = 0, int32_t bad_in = FPA_POINT_OK,
                                                   double* plast = nullptr) {
+    constexpr int NS = kStateLen<SYM>;
+    static_assert(!SYM || !TRACE, "the symmetric path writes no trace");
     const int i0 = SEG ? i0_in : 0;
     const int i1 = SEG ? i1_in : p.n_steps;
     double* tr = nullptr;
@@ -260,29 +333,29 @@ __device__ __forceinline__ int32_t fast_integrate(const Yaman4Params& p, int64_t
         const double qfr = fma(-qhi, ri, qhr * rr), qfi = fma(qhr, ri, qhi * rr);
         const double q6r = qfr * third, q6i = qfi * third;
 
-        double ys[8], yt[8], acc[8], S, Sx;
+        double ys[NS], yt[NS], acc[NS], S, Sx;
         // stage 1: ys = y + (h/2) f(z, y)
-        stage<LOSS>(y, y, qr, qi, cf.cg[0], cf.c2g[0], cf.cn[0], ys, S);
+        rk_stage<LOSS>(y, y, qr, qi, cf.cg[0], cf.c2g[0], cf.cn[0], ys, S);
         // S = sum |A|^2 of the state that step i-1 produced: a non-finite component makes S
         // non-finite, so the exact per-component test runs only then (integrators.py:132-135).
         if (nonfinite(S) && bad == FPA_POINT_OK && i > 0) {
             bool nf = false;
 #pragma unroll
-            for (int j = 0; j < 8; ++j) nf |= nonfinite(y[j]);
+            for (int j = 0; j < NS; ++j) nf |= nonfinite(y[j]);
             if (nf) bad = i - 1;
         }
 #pragma unroll
-        for (int j = 0; j < 8; ++j) acc[j] = fma(third, ys[j], y[j] * (-third));
+        for (int j = 0; j < NS; ++j) acc[j] = fma(third, ys[j], y[j] * (-third));
         // stage 2: yt = y + (h/2) f(z+h/2, ys)
-        stage<LOSS>(ys, y, qhr, qhi, cf.cg[0], cf.c2g[0], cf.cn[0], yt, Sx);
+        rk_stage<LOSS>(ys, y, qhr, qhi, cf.cg[0], cf.c2g[0], cf.cn[0], yt, Sx);
 #pragma unroll
-        for (int j = 0; j < 8; ++j) acc[j] = fma(two_thirds, yt[j], acc[j]);
+        for (int j = 0; j < NS; ++j) acc[j] = fma(two_thirds, yt[j], acc[j]);
         // stage 3: ys = y + h f(z+h/2, yt)
-        stage<LOSS>(yt, y, q2r, q2i, cf.cg[1], cf.c2g[1], cf.cn[1], ys, Sx);
+        rk_stage<LOSS>(yt, y, q2r, q2i, cf.cg[1], cf.c2g[1], cf.cn[1], ys, Sx);
 #pragma unroll
-        for (int j = 0; j < 8; ++j) acc[j] = fma(third_c, ys[j], acc[j]);
+        for (int j = 0; j < NS; ++j) acc[j] = fma(third_c, ys[j], acc[j]);
         // stage 4: y' = acc + (h/6) f(z+h, ys)
-        stage<LOSS>(ys, acc, q6r, q6i, cf.cg[2], cf.c2g[2], cf.cn[2], y, Sx);
+        rk_stage<LOSS>(ys, acc, q6r, q6i, cf.cg[2], cf.c2g[2], cf.cn[2], y, Sx);
 
         qr = qfr;
         qi = qfi;
@@ -490,6 +563,24 @@ __device__ __forceinline__ void sweep_initial_state(const X& x, int64_t k, doubl
     }
 }
 
+// Symmetric sweep (A0 waves 2 and 4 are bit copies of waves 1 and 3): the state is (x1, y1, x3, y3).
+__device__ __forceinline__ void sweep_initial_state(const SweepExtra& x, int64_t, double (&y)[4]) {
+    y[0] = x.A0[0];
+    y[1] = x.A0[1];
+    y[2] = x.A0[4];
+    y[3] = x.A0[5];
+}
+
+// The full end state and maxima of a symmetric run: waves 2 and 4 are copies of waves 1 and 3.
+__device__ __forceinline__ void sym_expand(const double (&s)[4], double (&y)[8], double (&pm)[4]) {
+    y[0] = y[2] = s[0];
+    y[1] = y[3] = s[1];
+    y[4] = y[6] = s[2];
+    y[5] = y[7] = s[3];
+    pm[1] = pm[0];
+    pm[3] = pm[2];
+}
+
 // The signal power the gain is taken from: max over the saved samples, or (phase sweep, "end") the last saved one.
 template <typename X>
 __device__ __forceinline__ double sweep_metric(const X& x, const double (&pm)[4], double plast) {
@@ -574,10 +665,11 @@ __device__ __forceinline__ void sweep_epilogue(const Yaman4Params& p, const Swee
     store_gain(x, b, gain);
 }
 
-// X = PhaseSweepExtra: the phase sweep.
-template <bool LOSS, int THREADS, int MIN_BLOCKS, typename X>
+// X = PhaseSweepExtra: the phase sweep.  SYM (plain sweep only): A0 is symmetric, the z-loop runs on (A1, A3).
+template <bool LOSS, int THREADS, int MIN_BLOCKS, typename X, bool SYM = false>
 __global__ void __launch_bounds__(THREADS, MIN_BLOCKS) yaman4_sweep_kernel(const Yaman4Params p, const X x) {
     constexpr bool PHASE = kPhase<X>;
+    static_assert(!(SYM && PHASE), "the phase sweep has no symmetric path");
     const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= p.n_points) return;
     int64_t gp, k;
@@ -587,29 +679,38 @@ __global__ void __launch_bounds__(THREADS, MIN_BLOCKS) yaman4_sweep_kernel(const
         sweep_invalid(p, x, b);
         return;
     }
-    double y[8];
+    double y[kStateLen<SYM>];
     sweep_initial_state(x, k, y);
     double        pm[4] = {0.0, 0.0, 0.0, 0.0}, plast = 0.0;
-    const int32_t bad = fast_integrate<false, true, LOSS, false, PHASE>(p, b, db_run, p.coef, y, pm, 0, 0, FPA_POINT_OK,
-                                                                        &plast);
-    sweep_epilogue(p, x, b, y, pm, bad, sweep_metric(x, pm, plast));
+    const int32_t bad = fast_integrate<false, true, LOSS, false, PHASE, SYM>(p, b, db_run, p.coef, y, pm, 0, 0,
+                                                                             FPA_POINT_OK, &plast);
+    if constexpr (SYM) {
+        double yf[8];
+        sym_expand(y, yf, pm);
+        sweep_epilogue(p, x, b, yf, pm, bad, pm[2]);
+    } else {
+        sweep_epilogue(p, x, b, y, pm, bad, sweep_metric(x, pm, plast));
+    }
 }
 
 // ------------------------------------------------------------------ fused sweep, z-segment scheduler
 // The sweep kernel above as a persistent kernel on the z-segment scheduler: prologue at segment 0, gain
 // epilogue at the last segment, the point's integration Delta-beta travels with its state (phase sweep: and the
-// last saved signal power, record kSegDoubles of the state).
-template <bool LOSS, int THREADS, int MIN_BLOCKS, typename X>
+// last saved signal power, record kSegDoubles of the state).  SYM: the record carries the symmetric state
+// (x1, y1, x3, y3) in slots 0-3 and the maxima of waves 1 and 3 in slots 8 and 10.
+template <bool LOSS, int THREADS, int MIN_BLOCKS, typename X, bool SYM = false>
 __global__ void __launch_bounds__(THREADS, MIN_BLOCKS)
     yaman4_sweep_seg_kernel(const Yaman4Params p, const X x, const SegParams g) {
     constexpr bool PHASE = kPhase<X>;
+    static_assert(!(SYM && PHASE), "the phase sweep has no symmetric path");
+    constexpr int NS = kStateLen<SYM>, PM_STEP = SYM ? 2 : 1;
     const int lane = threadIdx.x & 31;
     int       seg, w;
     while (seg_next_item(g, lane, seg, w)) {
         const int64_t b = (int64_t)w * 32 + lane;
         const bool    last = seg == g.n_seg - 1;
         if (b < p.n_points) {
-            double  y[8], pm[4] = {0.0, 0.0, 0.0, 0.0}, db_run, plast = 0.0;
+            double  y[NS], pm[4] = {0.0, 0.0, 0.0, 0.0}, db_run, plast = 0.0;
             int32_t bad = FPA_POINT_OK;
             bool    run;
             double* const st = g.state + b;
@@ -627,9 +728,9 @@ __global__ void __launch_bounds__(THREADS, MIN_BLOCKS)
                 run = !nonfinite(db_run);
                 if (run) {
 #pragma unroll
-                    for (int j = 0; j < 8; ++j) y[j] = __ldcg(st + j * g.n_pad);
+                    for (int j = 0; j < NS; ++j) y[j] = __ldcg(st + j * g.n_pad);
 #pragma unroll
-                    for (int j = 0; j < 4; ++j) pm[j] = __ldcg(st + (8 + j) * g.n_pad);
+                    for (int j = 0; j < 4; j += PM_STEP) pm[j] = __ldcg(st + (8 + j) * g.n_pad);
                     if (PHASE) plast = __ldcg(st + kSegDoubles * g.n_pad);
                     bad = __ldcg(g.bad + b);
                 }
@@ -637,16 +738,25 @@ __global__ void __launch_bounds__(THREADS, MIN_BLOCKS)
             if (run) {
                 const int i0 = seg * g.seg_steps;
                 const int i1 = last ? p.n_steps : i0 + g.seg_steps;
-                bad = fast_integrate<false, true, LOSS, true, PHASE>(p, b, db_run, p.coef, y, pm, i0, i1, bad, &plast);
-                if (last) sweep_epilogue(p, x, b, y, pm, bad, sweep_metric(x, pm, plast));
+                bad = fast_integrate<false, true, LOSS, true, PHASE, SYM>(p, b, db_run, p.coef, y, pm, i0, i1, bad,
+                                                                          &plast);
+                if (last) {
+                    if constexpr (SYM) {
+                        double yf[8];
+                        sym_expand(y, yf, pm);
+                        sweep_epilogue(p, x, b, yf, pm, bad, pm[2]);
+                    } else {
+                        sweep_epilogue(p, x, b, y, pm, bad, sweep_metric(x, pm, plast));
+                    }
+                }
             }
             if (!last) {
                 __stcg(st + 12 * g.n_pad, db_run);
                 if (run) {
 #pragma unroll
-                    for (int j = 0; j < 8; ++j) __stcg(st + j * g.n_pad, y[j]);
+                    for (int j = 0; j < NS; ++j) __stcg(st + j * g.n_pad, y[j]);
 #pragma unroll
-                    for (int j = 0; j < 4; ++j) __stcg(st + (8 + j) * g.n_pad, pm[j]);
+                    for (int j = 0; j < 4; j += PM_STEP) __stcg(st + (8 + j) * g.n_pad, pm[j]);
                     if (PHASE) __stcg(st + kSegDoubles * g.n_pad, plast);
                     __stcg(g.bad + b, bad);
                 }
@@ -777,6 +887,11 @@ __global__ void yaman4_rhs_kernel(int64_t B, const double* z, const double* A, c
 constexpr int kFastThreads = FPA_YAMAN4_THREADS, kFastMinBlocks = FPA_YAMAN4_MIN_BLOCKS;
 // the fused sweep kernel gets its best schedule (fewest 3-register FMAs, tools/sass_cost.py) at 4
 constexpr int kSweepMinBlocks = 4;
+// the symmetric sweep kernels (stage_sym): resident blocks per SM, chosen by measurement (DESIGN.md §4.1c)
+#ifndef FPA_SWEEP_SYM_MIN_BLOCKS
+#define FPA_SWEEP_SYM_MIN_BLOCKS 4
+#endif
+constexpr int kSweepSymMinBlocks = FPA_SWEEP_SYM_MIN_BLOCKS;
 // z-segment scheduler: RK4 steps per segment (multiples of kResync), chosen by measurement
 // (profiles/r2_seg_tune.txt): 64 below two waves of the resident warps, 128 above -- with those the
 // scheduler is at least as fast as the whole-run kernel at every batch of one wave or more
@@ -1002,14 +1117,16 @@ static int sweep_setup(const fpa_sweep_desc* d, int64_t n_phases, Yaman4Params& 
     return FPA_OK;
 }
 
-// z-segment scheduler when the batch is a wave or more, else the whole-run kernel
-template <typename X>
+// z-segment scheduler when the batch is a wave or more, else the whole-run kernel.  SYM: the symmetric kernels (their
+// own launch shape); resident_ctas and seg_plan see the kernel that will run.
+template <typename X, bool SYM = false>
 static int sweep_run(const Yaman4Params& p, const X& x, void* scratch, int64_t scratch_bytes, cudaStream_t st) {
     constexpr bool PHASE = kPhase<X>;
+    constexpr int  MB = SYM ? kSweepSymMinBlocks : kSweepMinBlocks;
     const int64_t B = p.n_points;
     const bool    lossless = p.lossless != 0;
-    const int ctas = lossless ? resident_ctas(yaman4_sweep_seg_kernel<false, kFastThreads, kSweepMinBlocks, X>, kFastThreads)
-                              : resident_ctas(yaman4_sweep_seg_kernel<true, kFastThreads, kSweepMinBlocks, X>, kFastThreads);
+    const int ctas = lossless ? resident_ctas(yaman4_sweep_seg_kernel<false, kFastThreads, MB, X, SYM>, kFastThreads)
+                              : resident_ctas(yaman4_sweep_seg_kernel<true, kFastThreads, MB, X, SYM>, kFastThreads);
     SegParams g;
     bool      use_seg = false;
     int rc = seg_plan(B, p.n_steps, ctas, kFastThreads, scratch, scratch_bytes, st, g, use_seg,
@@ -1017,19 +1134,26 @@ static int sweep_run(const Yaman4Params& p, const X& x, void* scratch, int64_t s
     if (rc != FPA_OK) return rc;
     if (use_seg) {
         if (lossless)
-            yaman4_sweep_seg_kernel<false, kFastThreads, kSweepMinBlocks, X><<<ctas, kFastThreads, 0, st>>>(p, x, g);
+            yaman4_sweep_seg_kernel<false, kFastThreads, MB, X, SYM><<<ctas, kFastThreads, 0, st>>>(p, x, g);
         else
-            yaman4_sweep_seg_kernel<true, kFastThreads, kSweepMinBlocks, X><<<ctas, kFastThreads, 0, st>>>(p, x, g);
+            yaman4_sweep_seg_kernel<true, kFastThreads, MB, X, SYM><<<ctas, kFastThreads, 0, st>>>(p, x, g);
     } else {
         const long blocks = (long)((B + kFastThreads - 1) / kFastThreads);
         if (lossless)
-            yaman4_sweep_kernel<false, kFastThreads, kSweepMinBlocks, X><<<blocks, kFastThreads, 0, st>>>(p, x);
+            yaman4_sweep_kernel<false, kFastThreads, MB, X, SYM><<<blocks, kFastThreads, 0, st>>>(p, x);
         else
-            yaman4_sweep_kernel<true, kFastThreads, kSweepMinBlocks, X><<<blocks, kFastThreads, 0, st>>>(p, x);
+            yaman4_sweep_kernel<true, kFastThreads, MB, X, SYM><<<blocks, kFastThreads, 0, st>>>(p, x);
     }
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return cuda_fail(e, "yaman4_sweep_kernel launch");
     return FPA_OK;
+}
+
+// A0 has A1 == A2 and A3 == A4 BIT FOR BIT (a value test would take -0.0 for 0.0, and the runs would then differ in
+// the sign of a zero); FPA_SWEEP_SYM=0 turns the symmetric kernels off (tests, A/B timing).
+static bool sweep_symmetric(const SweepExtra& x) {
+    return env_int("FPA_SWEEP_SYM", 1) != 0 && memcmp(&x.A0[0], &x.A0[2], 2 * sizeof(double)) == 0 &&
+           memcmp(&x.A0[4], &x.A0[6], 2 * sizeof(double)) == 0;
 }
 
 int yaman4_sweep_launch(const fpa_sweep_desc* d, void* scratch, int64_t scratch_bytes, cudaStream_t st) {
@@ -1038,6 +1162,7 @@ int yaman4_sweep_launch(const fpa_sweep_desc* d, void* scratch, int64_t scratch_
     int64_t      n_grid;
     int rc = sweep_setup(d, 1, p, x, n_grid);
     if (rc != FPA_OK || n_grid == 0) return rc;
+    if (sweep_symmetric(x)) return sweep_run<SweepExtra, true>(p, x, scratch, scratch_bytes, st);
     return sweep_run(p, x, scratch, scratch_bytes, st);
 }
 
