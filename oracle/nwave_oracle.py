@@ -15,6 +15,8 @@ Only tests/, __graft_entry__.smoke() and bench.py's CPU legs may import this mod
 """
 from __future__ import annotations
 
+import contextlib
+
 import numpy as np
 
 
@@ -119,25 +121,38 @@ def nwave_rhs_fast(z, A, gamma, alpha, beta, tab_arr, rows):
     return out
 
 
-def march(A0, gamma, alpha, beta, table, rows, *, z_max, n_steps, save_every=1, fast=True):
-    """Classical RK4 on linspace(0, z_max, n_steps+1) with the reference's saving rule
-    (integrators.py:111-142).  Returns (z_saved, A_saved[n_saved, N])."""
+def march(A0, gamma, alpha, beta, table, rows, *, z_max, n_steps, save_every=1, fast=True, z0=0.0, check=False):
+    """Classical RK4 on linspace(z0, z_max, n_steps+1) with the reference's saving rule
+    (integrators.py:111-142).  Returns (z_saved, A_saved[n_saved, N]).
+
+    check=True: also return the status the kernels report -- the index of the first step whose result
+    has a non-finite component, or -1 (integrators.py:132-135) -- as (z_saved, A_saved, status).  The
+    march stops after that step; the samples saved up to and including it are returned."""
     beta = np.asarray(beta, dtype=float)
     rows = np.asarray(rows)
     tab_arr = np.asarray(table, dtype=np.int64).reshape(-1, 4)
     f = (lambda z, y: nwave_rhs_fast(z, y, gamma, alpha, beta, tab_arr, rows)) if fast else \
         (lambda z, y: nwave_rhs(z, y, gamma, alpha, beta, table, rows))
-    grid = np.linspace(0.0, z_max, n_steps + 1)
+    grid = np.linspace(z0, z_max, n_steps + 1)
     y = np.asarray(A0, dtype=np.complex128).copy()
     zs, ys = [grid[0]], [y.copy()]
-    for i in range(n_steps):
-        z, h = grid[i], grid[i + 1] - grid[i]
-        k1 = f(z, y)
-        k2 = f(z + 0.5 * h, y + 0.5 * h * k1)
-        k3 = f(z + 0.5 * h, y + 0.5 * h * k2)
-        k4 = f(z + h, y + h * k3)
-        y = y + (h / 6.0) * (k1 + 2.0 * k2 + 2.0 * k3 + k4)
-        if (i + 1) % save_every == 0:
-            zs.append(grid[i + 1])
-            ys.append(y.copy())
+    status = -1
+    # a run that blows up overflows inside the stages; with check=True that is an expected outcome
+    with np.errstate(over="ignore", invalid="ignore") if check else contextlib.nullcontext():
+        for i in range(n_steps):
+            z, h = grid[i], grid[i + 1] - grid[i]
+            k1 = f(z, y)
+            k2 = f(z + 0.5 * h, y + 0.5 * h * k1)
+            k3 = f(z + 0.5 * h, y + 0.5 * h * k2)
+            k4 = f(z + h, y + h * k3)
+            y = y + (h / 6.0) * (k1 + 2.0 * k2 + 2.0 * k3 + k4)
+            if (i + 1) % save_every == 0:
+                zs.append(grid[i + 1])
+                ys.append(y.copy())
+            if check and not np.all(np.isfinite(y)):
+                status = i
+                break
+    if check:
+        return np.array(zs), np.array(ys), status
     return np.array(zs), np.array(ys)
+

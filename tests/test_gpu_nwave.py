@@ -134,12 +134,15 @@ def test_nwave_invariants(gpu):
 
 
 @pytest.mark.parametrize("lines", [[0], [0, 1], list(range(-3, 4)), list(range(-16, 17)), [0, 1, 2, 100],
-                                   list(range(-40, 41)), list(range(0, 127, 2)), list(range(-64, 64))])
+                                   list(range(-40, 41)), list(range(0, 127, 2)), list(range(-64, 64)),
+                                   list(range(0, 129, 2)), list(range(0, 24)) + list(range(168, 192)),
+                                   list(range(0, 257, 4)), list(range(0, 512, 7))])
 @pytest.mark.parametrize("batch", [2, 640])          # CTA-per-point and warp-per-point mappings
 def test_comb_equals_table_on_odd_shapes(gpu, lines, batch):
     """Grid spans that are not multiples of the kernel's tile (2, 4) or block (8) sizes, one and two
-    lines, wide gaps, spans above 64 (several rounds of tiles): the correlation form must reproduce the
-    enumerated-triplet kernel, which shares no indexing code with it."""
+    lines, wide gaps, spans above 64 (several rounds of tiles) and up to the limit of 512 (the generic
+    reduce-scatter; two rounds of tiles in the batch kernel from 257 on): the correlation form must reproduce
+    the enumerated-triplet kernel, which shares no indexing code with it."""
     nw = gpu.nwave
     plan = nw.uniform_comb_plan(1.2125e15, 6.28e11, lines)
     N = plan.n_waves
