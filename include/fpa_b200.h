@@ -421,7 +421,9 @@ int fpa_ipc_close(void* dev_ptr);
 
 /* Page-lock memory the caller already owns (e.g. a POSIX shared-memory segment several processes
  * map: every rank registers it and its kernels store their shard of the result straight into the
- * one host array).  Registered memory counts as pinned for every *_host entry point. */
+ * one host array).  Registered memory counts as pinned wherever a host entry point writes results
+ * directly: fpa_yaman4_rk4_batch_*host, fpa_yaman4_sweep_*host and fpa_yaman4_phase_sweep_*host.  The
+ * N-wave, linear, RHS and Delta-beta table entries always stage their results and copy them back. */
 int fpa_host_register(void* ptr, int64_t bytes);
 int fpa_host_unregister(void* ptr);
 

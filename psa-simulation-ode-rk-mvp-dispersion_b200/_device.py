@@ -53,6 +53,19 @@ def result_array(shape, dtype, pinned: bool = True) -> np.ndarray:
     return np.empty(shape, dtype=dtype)
 
 
+def _run_host(host, multi_host, desc, device, devices) -> None:
+    """`multi_host` over `devices` when they are several, else `host` on `device` (or the one entry of
+    `devices`, or the process default)."""
+    if devices is not None and len(devices) > 1:
+        ids = (C.c_int * len(devices))(*[int(v) for v in devices])
+        _lib.check(multi_host(C.byref(desc), len(devices), ids))
+        return
+    dev = _lib.get_device() if device is None else int(device)
+    if devices is not None and len(devices) == 1:
+        dev = int(devices[0])
+    _lib.check(host(C.byref(desc), dev))
+
+
 def yaman4_batch(dbeta, gamma, alpha, A0, *, z0=0.0, z_max, n_steps, save_every=1, z_grid=None,
                  trace=False, end=True, pmax=False, check_nan=True, phase_exact=False,
                  device: Optional[int] = None, devices=None) -> dict:
@@ -97,14 +110,8 @@ def yaman4_batch(dbeta, gamma, alpha, A0, *, z0=0.0, z_max, n_steps, save_every=
     d.A_end = ptr(out.get("A_end"))
     d.Pmax = ptr(out.get("Pmax"))
     d.status = ptr(out["status"])
-    if devices is not None and len(devices) > 1:
-        ids = (C.c_int * len(devices))(*[int(v) for v in devices])
-        _lib.check(_lib.lib().fpa_yaman4_rk4_batch_multi_host(C.byref(d), len(devices), ids))
-        return out
-    dev = _lib.get_device() if device is None else int(device)
-    if devices is not None and len(devices) == 1:
-        dev = int(devices[0])
-    _lib.check(_lib.lib().fpa_yaman4_rk4_batch_host(C.byref(d), dev))
+    L = _lib.lib()
+    _run_host(L.fpa_yaman4_rk4_batch_host, L.fpa_yaman4_rk4_batch_multi_host, d, device, devices)
     return out
 
 
@@ -200,14 +207,8 @@ def sweep(desc, *, want_pmax=False, want_end=False, device: Optional[int] = None
     desc.Pmax, desc.A_end = ptr(out.get("Pmax")), ptr(out.get("A_end"))
     if n1 * n3 == 0:
         return out
-    if devices is not None and len(devices) > 1:
-        ids = (C.c_int * len(devices))(*[int(v) for v in devices])
-        _lib.check(_lib.lib().fpa_yaman4_sweep_multi_host(C.byref(desc), len(devices), ids))
-        return out
-    dev = _lib.get_device() if device is None else int(device)
-    if devices is not None and len(devices) == 1:
-        dev = int(devices[0])
-    _lib.check(_lib.lib().fpa_yaman4_sweep_host(C.byref(desc), dev))
+    L = _lib.lib()
+    _run_host(L.fpa_yaman4_sweep_host, L.fpa_yaman4_sweep_multi_host, desc, device, devices)
     return out
 
 
@@ -232,14 +233,8 @@ def phase_sweep(desc, *, want_map: bool = True, device: Optional[int] = None, de
     w.gain_lin, w.status, w.Pmax, w.A_end = ptr(out.get("gain_lin")), ptr(out["status"]), None, None
     if n1 * n3 == 0:
         return out
-    if devices is not None and len(devices) > 1:
-        ids = (C.c_int * len(devices))(*[int(v) for v in devices])
-        _lib.check(_lib.lib().fpa_yaman4_phase_sweep_multi_host(C.byref(desc), len(devices), ids))
-        return out
-    dev = _lib.get_device() if device is None else int(device)
-    if devices is not None and len(devices) == 1:
-        dev = int(devices[0])
-    _lib.check(_lib.lib().fpa_yaman4_phase_sweep_host(C.byref(desc), dev))
+    L = _lib.lib()
+    _run_host(L.fpa_yaman4_phase_sweep_host, L.fpa_yaman4_phase_sweep_multi_host, desc, device, devices)
     return out
 
 
@@ -342,14 +337,8 @@ def nwave_batch(beta, gamma, alpha, A0, table, row_ptr, *, z0=0.0, z_max, n_step
             raise ValueError("grid_index must hold one entry per wave")
         slots = np.ascontiguousarray(g - g.min(), dtype=np.int32)
         d.grid_slot, d.grid_span = ptr(slots), int(g.max() - g.min() + 1)
-    if devices is not None and len(devices) > 1:
-        ids = (C.c_int * len(devices))(*[int(v) for v in devices])
-        _lib.check(_lib.lib().fpa_nwave_rk4_batch_multi_host(C.byref(d), len(devices), ids))
-        return out
-    dev = _lib.get_device() if device is None else int(device)
-    if devices is not None and len(devices) == 1:
-        dev = int(devices[0])
-    _lib.check(_lib.lib().fpa_nwave_rk4_batch_host(C.byref(d), dev))
+    L = _lib.lib()
+    _run_host(L.fpa_nwave_rk4_batch_host, L.fpa_nwave_rk4_batch_multi_host, d, device, devices)
     return out
 
 

@@ -581,17 +581,31 @@ static size_t nwave_smem_bytes(int N, int64_t n_table_entries) {
     return bytes + (size_t)n_table_entries * sizeof(fpa_triplet);
 }
 
-int nwave_launch(const fpa_nwave_desc* d, cudaStream_t st) {
+// The checks of an N-wave descriptor that the table kernel and the comb kernel share, for the device and the host
+// entries alike.  Each launcher adds its kernel's own limits.
+int nwave_check(const fpa_nwave_desc* d) {
     FPA_REQUIRE(d != nullptr, "descriptor is NULL");
     FPA_REQUIRE(d->n_points >= 0, "n_points must be >= 0");
     FPA_REQUIRE(d->n_waves >= 1, "n_waves must be >= 1");
+    FPA_REQUIRE(d->n_steps >= 1 && d->n_steps < 2147483647LL, "n_steps must be in [1, 2^31)");
+    FPA_REQUIRE(d->save_every >= 1, "save_every must be a positive integer");
+    FPA_REQUIRE(d->beta && d->gamma && d->alpha && d->A0, "beta/gamma/alpha/A0 must be set");
+    FPA_REQUIRE((d->gamma_stride | 1) == 1 && (d->alpha_stride | 1) == 1 && (d->A0_stride | 1) == 1 &&
+                    (d->beta_stride | 1) == 1,
+                "strides must be 0 (broadcast) or 1 (per point)");
+    FPA_REQUIRE(!(d->flags & FPA_OUT_TRACE) || d->A_trace, "FPA_OUT_TRACE needs A_trace");
+    FPA_REQUIRE(!(d->flags & FPA_OUT_PMAX) || d->Pmax, "FPA_OUT_PMAX needs Pmax");
+    FPA_REQUIRE(!(d->flags & FPA_OUT_END) || d->A_end, "FPA_OUT_END needs A_end");
+    return FPA_OK;
+}
+
+int nwave_launch(const fpa_nwave_desc* d, cudaStream_t st) {
+    int rc = nwave_check(d);
+    if (rc != FPA_OK) return rc;
     if (d->n_waves > 128) {
         set_error("n_waves = %d exceeds the kernel limit of 128", d->n_waves);
         return FPA_ERR_UNSUPPORTED;
     }
-    FPA_REQUIRE(d->n_steps >= 1 && d->n_steps < 2147483647LL, "n_steps must be in [1, 2^31)");
-    FPA_REQUIRE(d->save_every >= 1, "save_every must be a positive integer");
-    FPA_REQUIRE(d->beta && d->gamma && d->alpha && d->A0, "beta/gamma/alpha/A0 must be set");
     // the factored form of the table (fpa_nwave_factor_table) replaces the entry list when the caller supplies it
     const bool fact = d->factored != nullptr && !(d->flags & FPA_NWAVE_PLAIN) && getenv("FPA_NWAVE_PLAIN") == nullptr;
     if (fact) {
@@ -601,15 +615,9 @@ int nwave_launch(const fpa_nwave_desc* d, cudaStream_t st) {
         FPA_REQUIRE(d->row_ptr != nullptr, "row_ptr must be set");
         FPA_REQUIRE(d->n_triplets == 0 || d->triplets, "triplets must be set");
     }
-    FPA_REQUIRE((d->gamma_stride | 1) == 1 && (d->alpha_stride | 1) == 1 && (d->A0_stride | 1) == 1 &&
-                    (d->beta_stride | 1) == 1,
-                "strides must be 0 (broadcast) or 1 (per point)");
     const bool trace = (d->flags & FPA_OUT_TRACE) != 0;
     const bool pmax  = (d->flags & FPA_OUT_PMAX) != 0;
     const bool endo  = (d->flags & FPA_OUT_END) != 0;
-    FPA_REQUIRE(!trace || d->A_trace, "FPA_OUT_TRACE needs A_trace");
-    FPA_REQUIRE(!pmax || d->Pmax, "FPA_OUT_PMAX needs Pmax");
-    FPA_REQUIRE(!endo || d->A_end, "FPA_OUT_END needs A_end");
     if (d->n_points == 0) return FPA_OK;
 
     NwaveParams p;

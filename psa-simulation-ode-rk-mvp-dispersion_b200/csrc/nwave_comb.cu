@@ -980,8 +980,22 @@ static cudaError_t comb_launch_w(const CombParams& p, int sms, cudaStream_t st) 
     return cudaGetLastError();
 }
 
+int nwave_check(const fpa_nwave_desc* d);  // nwave.cu
+
+// The limits of the convolution form: n_waves <= 128, grid_span <= 512.
+bool nwave_comb_fits(const fpa_nwave_desc* d) { return d->n_waves <= 128 && d->grid_span <= 512; }
+
 // d->grid_slot: device pointer to the N grid slots; span = number of grid slots covered.
 int nwave_comb_launch(const fpa_nwave_desc* d, cudaStream_t st) {
+    int rc = nwave_check(d);
+    if (rc != FPA_OK) return rc;
+    FPA_REQUIRE(d->n_points < 2147483647LL, "bad n_points");
+    if (!nwave_comb_fits(d)) {
+        set_error("comb kernel limits: n_waves <= 128, grid_span <= 512 (got %d, %d)", d->n_waves, d->grid_span);
+        return FPA_ERR_UNSUPPORTED;
+    }
+    FPA_REQUIRE(d->grid_span >= d->n_waves, "grid_span must cover all waves");
+    if (d->n_points == 0) return FPA_OK;
     const int N = d->n_waves, M = d->grid_span;
     CombParams p;
     p.n_points     = d->n_points;

@@ -994,7 +994,9 @@ static int launch_fast(const Yaman4Params& p, bool uniform, void* scratch, int64
     return FPA_OK;
 }
 
-int yaman4_launch(const fpa_yaman4_desc* d, cudaStream_t st) {
+// The checks of a batch descriptor, for the device and the host entries alike.  FPA_UNIFORM_PHYSICS is checked by
+// yaman4_launch alone: the host entry sets or clears that flag itself.
+int yaman4_check(const fpa_yaman4_desc* d) {
     FPA_REQUIRE(d != nullptr, "descriptor is NULL");
     FPA_REQUIRE(d->n_points >= 0, "n_points must be >= 0");
     FPA_REQUIRE(d->n_steps >= 1 && d->n_steps < 2147483647LL, "n_steps must be in [1, 2^31)");
@@ -1002,12 +1004,18 @@ int yaman4_launch(const fpa_yaman4_desc* d, cudaStream_t st) {
     FPA_REQUIRE(d->dbeta && d->gamma && d->alpha && d->A0, "dbeta/gamma/alpha/A0 must be set");
     FPA_REQUIRE((d->gamma_stride | 1) == 1 && (d->alpha_stride | 1) == 1 && (d->A0_stride | 1) == 1,
                 "strides must be 0 (broadcast) or 1 (per point)");
+    FPA_REQUIRE(!(d->flags & FPA_OUT_TRACE) || d->A_trace, "FPA_OUT_TRACE needs A_trace");
+    FPA_REQUIRE(!(d->flags & FPA_OUT_PMAX) || d->Pmax, "FPA_OUT_PMAX needs Pmax");
+    FPA_REQUIRE(!(d->flags & FPA_OUT_END) || d->A_end, "FPA_OUT_END needs A_end");
+    return FPA_OK;
+}
+
+int yaman4_launch(const fpa_yaman4_desc* d, cudaStream_t st) {
+    int rc = yaman4_check(d);
+    if (rc != FPA_OK) return rc;
     const bool trace = (d->flags & FPA_OUT_TRACE) != 0;
     const bool pmax  = (d->flags & FPA_OUT_PMAX) != 0;
     const bool endo  = (d->flags & FPA_OUT_END) != 0;
-    FPA_REQUIRE(!trace || d->A_trace, "FPA_OUT_TRACE needs A_trace");
-    FPA_REQUIRE(!pmax || d->Pmax, "FPA_OUT_PMAX needs Pmax");
-    FPA_REQUIRE(!endo || d->A_end, "FPA_OUT_END needs A_end");
     const bool uniform = (d->flags & FPA_UNIFORM_PHYSICS) != 0;
     FPA_REQUIRE(!uniform || (d->gamma_stride == 0 && d->alpha_stride == 0),
                 "FPA_UNIFORM_PHYSICS needs broadcast gamma and alpha (stride 0)");
@@ -1059,6 +1067,15 @@ int yaman4_launch(const fpa_yaman4_desc* d, cudaStream_t st) {
 // gamma/alpha/z_max/dz per length unit, exactly as fpa_sweep_desc carries them.
 int plan_fill(const fpa_plan_desc* d, PlanParams& p);
 
+// The grid points a sweep runs: the whole n1*n3 grid, or the sub-range [first_point, first_point + n_sub_points).
+int sweep_grid_points(const fpa_sweep_desc* d, int64_t* n_grid) {
+    const int64_t grid = d->plan.n1 * d->plan.n3;
+    FPA_REQUIRE(d->first_point >= 0 && d->n_sub_points >= 0 && d->first_point + d->n_sub_points <= grid,
+                "first_point / n_sub_points must select a range of the n1*n3 grid");
+    *n_grid = (d->first_point == 0 && d->n_sub_points == 0) ? grid : d->n_sub_points;
+    return FPA_OK;
+}
+
 // Checks a sweep descriptor and fills the kernel arguments for its n_grid grid points (the whole grid or the
 // sub-range) x n_phases runs each; the plain sweep is n_phases = 1.
 static int sweep_setup(const fpa_sweep_desc* d, int64_t n_phases, Yaman4Params& p, SweepExtra& x, int64_t& n_grid) {
@@ -1070,10 +1087,8 @@ static int sweep_setup(const fpa_sweep_desc* d, int64_t n_phases, Yaman4Params& 
     }
     int rc = plan_fill(&d->plan, x.plan);
     if (rc != FPA_OK) return rc;
-    const int64_t grid = d->plan.n1 * d->plan.n3;
-    FPA_REQUIRE(d->first_point >= 0 && d->n_sub_points >= 0 && d->first_point + d->n_sub_points <= grid,
-                "first_point / n_sub_points must select a range of the n1*n3 grid");
-    n_grid = (d->first_point == 0 && d->n_sub_points == 0) ? grid : d->n_sub_points;
+    rc = sweep_grid_points(d, &n_grid);
+    if (rc != FPA_OK) return rc;
     const int64_t B = n_grid * n_phases;
     FPA_REQUIRE(d->gain_lin != nullptr || B == 0, "gain_lin must be set");
     FPA_REQUIRE(d->length_scale == 1.0 || d->length_scale == 1000.0, "length_scale must be 1 or 1000");
@@ -1166,19 +1181,26 @@ int yaman4_sweep_launch(const fpa_sweep_desc* d, void* scratch, int64_t scratch_
     return sweep_run(p, x, scratch, scratch_bytes, st);
 }
 
+// The arguments of the phase axis, for the device and the host entries alike.
+int phase_sweep_check(const fpa_phase_sweep_desc* d) {
+    FPA_REQUIRE(d != nullptr, "phase sweep descriptor is NULL");
+    FPA_REQUIRE(d->sweep.n_peers == 0, "the phase sweep has no peer-store gather: n_peers must be 0");
+    FPA_REQUIRE(d->n_phases >= 1 && d->n_phases <= FPA_MAX_PHASES, "n_phases must be in [1, %d]", FPA_MAX_PHASES);
+    FPA_REQUIRE(d->A0_table != nullptr, "A0_table must be set");
+    FPA_REQUIRE(d->metric == FPA_GAIN_MAX_SAVED || d->metric == FPA_GAIN_LAST_SAVED, "unknown gain metric %d", d->metric);
+    return FPA_OK;
+}
+
 // The sweep kernels with the phase axis: n_grid * K points, plan outputs per grid point, everything else per point.
 int yaman4_phase_sweep_launch(const fpa_phase_sweep_desc* d, void* scratch, int64_t scratch_bytes, cudaStream_t st) {
-    FPA_REQUIRE(d != nullptr, "phase sweep descriptor is NULL");
     Yaman4Params    p;
     PhaseSweepExtra x;
     int64_t         n_grid;
-    const int64_t   K = d->n_phases;
-    if (d->sweep.flags & FPA_PHASE_EXACT) return sweep_setup(&d->sweep, 1, p, x, n_grid);  // FPA_ERR_UNSUPPORTED
-    FPA_REQUIRE(d->sweep.n_peers == 0, "the phase sweep has no peer-store gather: n_peers must be 0");
-    FPA_REQUIRE(K >= 1 && K <= FPA_MAX_PHASES, "n_phases must be in [1, %d]", FPA_MAX_PHASES);
-    FPA_REQUIRE(d->A0_table != nullptr, "A0_table must be set");
-    FPA_REQUIRE(d->metric == FPA_GAIN_MAX_SAVED || d->metric == FPA_GAIN_LAST_SAVED, "unknown gain metric %d", d->metric);
-    int rc = sweep_setup(&d->sweep, K, p, x, n_grid);
+    if (d && (d->sweep.flags & FPA_PHASE_EXACT)) return sweep_setup(&d->sweep, 1, p, x, n_grid);  // FPA_ERR_UNSUPPORTED
+    int rc = phase_sweep_check(d);
+    if (rc != FPA_OK) return rc;
+    const int64_t K = d->n_phases;
+    rc = sweep_setup(&d->sweep, K, p, x, n_grid);
     if (rc != FPA_OK || n_grid == 0) return rc;
     x.A0_table   = d->A0_table;
     x.n_phases   = K;
