@@ -4,7 +4,7 @@
 set -u
 OUT=gpurun_out
 mkdir -p $OUT
-CASES=${@:-"seg125k comb1024 comb comb16 trace table"}
+CASES=${@:-"seg125k comb1024 comb trace table"}
 for c in $CASES; do
   case $c in trace) K=yaman4_fast;; comb*) K=nwave_comb;; table*) K=nwave_rk4;; seg125k) K=yaman4_sweep;; esac
   if [ $c = seg125k ]; then CMD="python bench.py --steps 2 --warmup 3 --shard-of 8 --no-cpu-baseline --no-secondary"; SKIP=3

@@ -607,7 +607,7 @@ int nwave_launch(const fpa_nwave_desc* d, cudaStream_t st) {
         return FPA_ERR_UNSUPPORTED;
     }
     // the factored form of the table (fpa_nwave_factor_table) replaces the entry list when the caller supplies it
-    const bool fact = d->factored != nullptr && !(d->flags & FPA_NWAVE_PLAIN) && getenv("FPA_NWAVE_PLAIN") == nullptr;
+    const bool fact = d->factored != nullptr && !(d->flags & FPA_NWAVE_PLAIN);
     if (fact) {
         FPA_REQUIRE(d->n_classes >= 0 && d->n_classes < kFactMaxCls, "n_classes must be the class count of `factored`");
     } else {

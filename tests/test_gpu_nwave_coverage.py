@@ -240,19 +240,15 @@ def _config2(gpu):
     return plan, gpu.nwave.beta_per_wave(plan, _disp(gpu))
 
 
-@pytest.mark.parametrize("lanes", [32, 16])
-def test_ragged_batch_kernel_launches(gpu, nw_oracle, sm4, lanes, monkeypatch):
+def test_ragged_batch_kernel_launches(gpu, nw_oracle, sm4):
     """Batch sizes on both sides of the 4 x SM threshold and 16 x SM + 3 (eight points per CTA: the last CTA holds
-    three); with half a warp per point (FPA_COMB_LANES=16) odd batches, where the copy of the last point runs in the
-    spare half warp and must store nothing.  First and last point against the oracle, the batch against the table."""
-    if lanes == 16:
-        monkeypatch.setenv("FPA_COMB_LANES", "16")
+    three).  First and last point against the oracle, the batch against the table."""
     plan, beta = _config2(gpu)
     N = plan.n_waves
     sms = sm4 // 4
-    sizes = (sm4 - 1, sm4, sm4 + 1, 16 * sms + 3) if lanes == 32 else (sm4 + 1, 16 * sms + 3)
+    sizes = (sm4 - 1, sm4, sm4 + 1, 16 * sms + 3)
     n_steps, save_every, z_max = 40, 7, 4.0
-    rng = np.random.default_rng(lanes)
+    rng = np.random.default_rng(32)
     A0 = _amps(rng, 16 * sms + 3, N, 1e-3, 0.1)
     gam = rng.uniform(5e-3, 3e-2, A0.shape[0])
     ref0 = _oracle_steps(nw_oracle, plan, A0[0], gam[0], 1e-4, beta, z_max=z_max, n_steps=n_steps)
@@ -261,19 +257,16 @@ def test_ragged_batch_kernel_launches(gpu, nw_oracle, sm4, lanes, monkeypatch):
         A, g = A0[:B], gam[:B]
         refB = _oracle_steps(nw_oracle, plan, A[B - 1], g[B - 1], 1e-4, beta, z_max=z_max, n_steps=n_steps)
         c = _batch(gpu, plan, "auto", beta, g, 1e-4, A, **kw)
-        _check_vs_oracle(c, 0, ref0, save_every, (lanes, B))
-        _check_vs_oracle(c, B - 1, refB, save_every, (lanes, B))
-        _check_close(c, _batch(gpu, plan, "table", beta, g, 1e-4, A, **kw), TOL_FORMS, (lanes, B, "comb vs table"))
+        _check_vs_oracle(c, 0, ref0, save_every, B)
+        _check_vs_oracle(c, B - 1, refB, save_every, B)
+        _check_close(c, _batch(gpu, plan, "table", beta, g, 1e-4, A, **kw), TOL_FORMS, (B, "comb vs table"))
 
 
-@pytest.mark.parametrize("lanes", [32, 16])
-def test_nothing_is_stored_past_the_batch(gpu, sm4, lanes, monkeypatch):
+def test_nothing_is_stored_past_the_batch(gpu, sm4):
     """Through `fpa_nwave_rk4_batch_dev` with every output buffer one point longer than the batch and filled with a
-    sentinel: the comb kernel (odd batches in both mappings, 16 x SM + 3) and the table kernel write the batch's
+    sentinel: the comb kernel (odd batches in both kernels, 16 x SM + 3) and the table kernel write the batch's
     results -- the bits the host entry gives -- and leave the extra point untouched."""
     import torch
-    if lanes == 16:
-        monkeypatch.setenv("FPA_COMB_LANES", "16")
     L, lib = gpu._lib, gpu._lib.lib()
     dev = torch.device("cuda", L.get_device())
     plan, beta = _config2(gpu)
@@ -288,7 +281,7 @@ def test_nothing_is_stored_past_the_batch(gpu, sm4, lanes, monkeypatch):
     t_beta = t(beta)
     for B in (3, sm4 + 1, 16 * (sm4 // 4) + 3):
         A0 = _amps(rng, B, N, 1e-3, 0.1)
-        for form in ("comb", "table", "entries") if lanes == 32 else ("comb",):
+        for form in ("comb", "table", "entries"):
             host = _batch(gpu, plan, form, beta, 0.02, 1e-4, A0, z_max=1.2, n_steps=n_steps, save_every=save_every)
             t_A0, t_ga = t(A0.view(np.float64)), t(np.array([0.02, 1e-4]))
             t_tr = torch.full(((B + 1) * ns * N * 2,), -7.25, dtype=torch.float64, device=dev)
@@ -313,7 +306,7 @@ def test_nothing_is_stored_past_the_batch(gpu, sm4, lanes, monkeypatch):
             L.check(lib.fpa_nwave_rk4_batch_dev(C.byref(d), torch.cuda.current_stream().cuda_stream))
             torch.cuda.synchronize()
             tr, end, pm, st = t_tr.cpu().numpy(), t_end.cpu().numpy(), t_pm.cpu().numpy(), t_st.cpu().numpy()
-            what = (lanes, B, form)
+            what = (B, form)
             assert (tr[B * ns * N * 2:] == -7.25).all() and (end[B * N * 2:] == -7.25).all(), what
             assert (pm[B * N:] == -7.25).all() and st[B] == 12345, what
             assert tr[:B * ns * N * 2].tobytes() == host["A_trace"].tobytes(), what

@@ -110,11 +110,10 @@ def test_segment_scheduler_kernels_bit_identical(gpu, golden):
             _same(a, b)
 
 
-@pytest.mark.parametrize("batch, lanes", [(640, "32"), (640, "16")])
-def test_comb_batch_kernel_bit_identical(gpu, batch, lanes, monkeypatch):
+def test_comb_batch_kernel_bit_identical(gpu):
     """`nwave_comb8_kernel` goes through the pass in flags-only mode (ptxas' order kept, yield hints cleared,
-    operand-reuse flags set): both lane mappings must agree bit for bit with the ptxas-schedule build."""
-    monkeypatch.setenv("FPA_COMB_LANES", lanes)     # read once per library instance, i.e. once per build here
+    operand-reuse flags set): it must agree bit for bit with the ptxas-schedule build."""
+    batch = 640
     nw = gpu.nwave
     w0 = 2 * np.pi * 299792458.0 / 1550e-9
     for lines in (range(-32, 32), range(-10, 11), [0, 1, 2, 3, 5, 8, 13, 21, 34, 55, 89]):

@@ -9,7 +9,6 @@ a failed assert aborts the kernel and the call returns a CUDA error.
 usage (GPU box):  python tools/bounds_check.py
 """
 import ctypes as C
-import os
 import subprocess
 import sys
 from pathlib import Path
@@ -40,7 +39,7 @@ with fpa._lib.use_library(out):
     # spans that are not multiples of the tile / block sizes, gapped grids, spans 129 .. 512 (the generic
     # reduce-scatter, two rounds of tiles from 257 on), N = 128 with span 512; one CTA per point and the batch
     # mapping on both sides of its threshold (4 x SM), with a partly filled last CTA (16 x SM + 3: eight points per
-    # CTA for small plans) and half a warp per point (FPA_COMB_LANES=16) at odd batch sizes; beta per point
+    # CTA for small plans); beta per point
     wide = (range(0, 129, 2), list(range(0, 24)) + list(range(168, 192)), range(0, 256, 2), range(0, 257, 4),
             range(0, 512, 7), list(range(0, 508, 4)) + [511])
     for lines in ([0], [0, 1], range(-1, 2), range(-3, 4), [-6, -3, -1, 0, 1, 2, 5, 9], range(-10, 11),
@@ -49,17 +48,14 @@ with fpa._lib.use_library(out):
         N = plan.n_waves
         beta = nw.beta_per_wave(plan, disp)
         sizes = (1, 3, 700, sm4 - 1, sm4 + 1) + (() if N > 100 else (16 * n_sm.value + 3,))
-        for lanes in (32, 16):
-            os.environ["FPA_COMB_LANES"] = str(lanes)
-            for B in sizes if lanes == 32 else [b for b in sizes if b >= sm4 and b % 2]:
-                A0 = np.sqrt(rng.uniform(1e-6, 1e-2, (B, N))) * np.exp(1j * rng.uniform(0, 6.28, (B, N)))
-                bet = beta * rng.uniform(0.9, 1.1, (B, N)) if B % 2 else beta
-                cfg = fpa.config.custom_simulation_config(z_max=0.7, dz=0.1, save_every=3)
-                r = nw.run_nwave_simulation(cfg, plan, gamma=0.02, alpha=1e-4, A0=A0, beta=bet, form="comb",
-                                            outputs=("trace", "end", "pmax"))
-                assert np.isfinite(r["A_end"]).all()
-                n_cases += 1
-        del os.environ["FPA_COMB_LANES"]
+        for B in sizes:
+            A0 = np.sqrt(rng.uniform(1e-6, 1e-2, (B, N))) * np.exp(1j * rng.uniform(0, 6.28, (B, N)))
+            bet = beta * rng.uniform(0.9, 1.1, (B, N)) if B % 2 else beta
+            cfg = fpa.config.custom_simulation_config(z_max=0.7, dz=0.1, save_every=3)
+            r = nw.run_nwave_simulation(cfg, plan, gamma=0.02, alpha=1e-4, A0=A0, beta=bet, form="comb",
+                                        outputs=("trace", "end", "pmax"))
+            assert np.isfinite(r["A_end"]).all()
+            n_cases += 1
     print(f"bounds-checked comb kernel: {n_cases} launches without a failed assert")
     # the factored-table kernel: every offset it takes from its blob, over plan sizes 1 .. 128, single runs (512 / 256
     # / 64 threads per point) and batches (64 / 128 threads), grid plans, an off-grid plan and tables no plan gives

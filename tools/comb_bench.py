@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """tools/comb_bench.py [B ...] -- N = 64 comb plan of BASELINE config 5 through fpa_nwave_rk4_batch_dev for
 several batch sizes (device-resident, CUDA events): point.steps/s, credited TFLOP/s and the fraction of the
-measured FP64 peak.  FPA_COMB_TILE4=1 selects the round-1 tiles-of-4 mapping for comparison."""
+measured FP64 peak."""
 import ctypes as C
 import os
 import sys
@@ -29,8 +29,7 @@ plan = nw.uniform_comb_plan(w0, 2 * np.pi * 100e9, range(-32, 32))
 beta = nw.beta_per_wave(plan, ds.DispersionParams(omega_ref=w0, beta2=-2.57e-29, beta3=3.30e-41, beta4=-1.63e-55))
 phases = np.random.default_rng(0).uniform(0, 2 * np.pi, 64)
 flops = plan.flops_per_step("comb")
-print(f"{torch.cuda.get_device_name(0)}; FP64 peak {peak_tf:.2f} TF; N = 64, {steps} steps, {flops:.0f} credited flops per point.step; "
-      f"mapping: {'tiles of 4 (round 1)' if os.environ.get('FPA_COMB_TILE4') else 'tiles of 8, rolling window'}")
+print(f"{torch.cuda.get_device_name(0)}; FP64 peak {peak_tf:.2f} TF; N = 64, {steps} steps, {flops:.0f} credited flops per point.step")
 for Bn in sizes:
     A0 = np.empty((Bn, 64), dtype=complex)
     for b, pw in enumerate(np.linspace(0.1, 1.0, Bn)):

@@ -1,10 +1,9 @@
 #!/usr/bin/env python
 """tools/profile_cases.py <case> -- one small launch sequence per secondary kernel, for ncu captures.
   trace : yaman4_fast_kernel<TRACE>, 2e5 points x 2500 steps, save_every = 1 (32 GB written)
-  comb  : nwave_comb8_kernel<32,2,1> (warp per point), N = 64, B = 4736, 200 steps
+  comb  : nwave_comb8_kernel<2> (warp per point), N = 64, B = 4736, 200 steps
   comb1024 : the same kernel at the batch of BASELINE config 5, B = 1024, 400 steps
-  comb16 : nwave_comb8_kernel<16,1,1> (half a warp per point), N = 64, B = 9472, 100 steps
-  comb1 : nwave_comb_kernel<4,2,4> (CTA per point), N = 64, B = 1, 2000 steps
+  comb1 : nwave_comb_kernel (CTA per point), N = 64, B = 1, 2000 steps
   table : nwave_rk4_kernel<factored> (512 threads per point), N = 64, B = 148, 100 steps
   table4736 : the same kernel (64 threads per point) at B = 4736, 100 steps
 """
@@ -48,7 +47,7 @@ else:
     plan = nw.uniform_comb_plan(w0, 2 * np.pi * 100e9, range(-32, 32))
     disp = ds.DispersionParams(omega_ref=w0, beta2=-2.57e-29, beta3=3.30e-41, beta4=-1.63e-55)
     beta = nw.beta_per_wave(plan, disp)
-    Bn, steps = {"comb": (4736, 200), "comb1024": (1024, 400), "comb16": (9472, 100), "comb1": (1, 2000),
+    Bn, steps = {"comb": (4736, 200), "comb1024": (1024, 400), "comb1": (1, 2000),
                  "table": (148, 100), "table4736": (4736, 100)}[case]
     rng = np.random.default_rng(0)
     A0 = np.sqrt(np.full((Bn, 64), 1e-6)) * np.exp(1j * rng.uniform(0, 6.28, (Bn, 64)))
