@@ -21,6 +21,17 @@
  *   they are asynchronous on that stream.  "host" entry points take HOST
  *   pointers, stage through a library-owned device workspace and return after
  *   the results are back in host memory.
+ *
+ * Alignment
+ *   dev entries: the kernels move complex128 values and rows of maxima with 16-byte
+ *   vector accesses, so these device pointers must be 16-byte aligned (else
+ *   FPA_ERR_INVALID, error text "... must be 16-byte aligned"): yaman4 A0, A_trace,
+ *   A_end, Pmax; sweep plan.omega, A_end, Pmax; phase sweep A0_table; Delta-beta
+ *   table omega; N-wave A0, A_trace, A_end and `factored`.  (torch and cudaMalloc
+ *   allocations are; a complex128 view at an odd element offset is not.)
+ *   host entries: any naturally aligned array (numpy's rule: 8 bytes for float64 and
+ *   complex128).  A page-locked result array the kernel cannot store to directly
+ *   is staged like pageable memory.
  */
 #ifndef FPA_B200_H
 #define FPA_B200_H
@@ -422,7 +433,8 @@ int fpa_ipc_close(void* dev_ptr);
 /* Page-lock memory the caller already owns (e.g. a POSIX shared-memory segment several processes
  * map: every rank registers it and its kernels store their shard of the result straight into the
  * one host array).  Registered memory counts as pinned wherever a host entry point writes results
- * directly: fpa_yaman4_rk4_batch_*host, fpa_yaman4_sweep_*host and fpa_yaman4_phase_sweep_*host.  The
+ * directly: fpa_yaman4_rk4_batch_*host, fpa_yaman4_sweep_*host and fpa_yaman4_phase_sweep_*host; their
+ * complex128 outputs and Pmax rows only when 16-byte aligned (else staged, see "Alignment" above).  The
  * N-wave, linear, RHS and Delta-beta table entries always stage their results and copy them back. */
 int fpa_host_register(void* ptr, int64_t bytes);
 int fpa_host_unregister(void* ptr);

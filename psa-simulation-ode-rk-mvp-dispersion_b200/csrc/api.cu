@@ -180,6 +180,10 @@ static int run_on_device(int (*launch)(const Desc*, int, Pending*), const Desc* 
     return finish(p, device);
 }
 
+// Alignment the kernels need of the arrays they access with 16-byte vector loads and stores (complex128 data, rows of
+// four maxima).
+constexpr size_t kVecAlign = 16;
+
 // The device buffers of one host-pointer call, carved in 256-byte aligned pieces from one workspace slot.
 // stage() runs the entry's declaring code twice: a sizing pass that only adds up the pieces, then, with the
 // workspace at that size, the placing pass that hands out addresses, queues the uploads and records the copies
@@ -206,11 +210,13 @@ struct Staging {
         if (base && rc == FPA_OK) rc = up(p, host, n * sizeof(T), pend->st);
         return p;
     }
-    // where the kernel writes the n elements meant for `host`: the device address of `host` when may_map is set
-    // and `host` is page-locked, else a buffer that is copied to `host` after the kernel (a NULL `host` gets none)
+    // where the kernel writes the n elements meant for `host`: the device address of `host` when may_map is set,
+    // `host` is page-locked and `host` is aligned to `align` bytes, the width of the kernel's stores into it (16
+    // for complex128 data and rows of maxima, which numpy only aligns to 8); else a buffer that is copied to `host`
+    // after the kernel (a NULL `host` gets none)
     template <class T>
-    T* out(T* host, size_t n, bool may_map) {
-        if (!base) maps.push_back(may_map ? mapped(host) : nullptr);
+    T* out(T* host, size_t n, bool may_map, size_t align = alignof(T)) {
+        if (!base) maps.push_back(may_map && reinterpret_cast<uintptr_t>(host) % align == 0 ? mapped(host) : nullptr);
         if (T* m = static_cast<T*>(maps[n_out++])) return m;
         T* p = tmp<T>(n);
         if (base && host) pend->copies.push_back({host, p, n * sizeof(T)});
@@ -293,9 +299,9 @@ static int batch_host_launch(const fpa_yaman4_desc* d, int device, Pending* p) {
         dd.alpha   = s.in(d->alpha, d->alpha_stride ? B : 1);
         dd.A0      = s.in(d->A0, (d->A0_stride ? B : 1) * 8);
         dd.z_grid  = d->z_grid ? s.in(d->z_grid, (size_t)d->n_steps + 1) : nullptr;
-        dd.A_trace = (d->flags & FPA_OUT_TRACE) ? s.out(d->A_trace, B * ns * 8, true) : nullptr;
-        dd.A_end   = (d->flags & FPA_OUT_END) ? s.out(d->A_end, B * 8, true) : nullptr;
-        dd.Pmax    = (d->flags & FPA_OUT_PMAX) ? s.out(d->Pmax, B * 4, true) : nullptr;
+        dd.A_trace = (d->flags & FPA_OUT_TRACE) ? s.out(d->A_trace, B * ns * 8, true, kVecAlign) : nullptr;
+        dd.A_end   = (d->flags & FPA_OUT_END) ? s.out(d->A_end, B * 8, true, kVecAlign) : nullptr;
+        dd.Pmax    = (d->flags & FPA_OUT_PMAX) ? s.out(d->Pmax, B * 4, true, kVecAlign) : nullptr;
         dd.status  = s.out(d->status, B, true);  // the kernel always gets one
         dd.scratch = s.tmp<char>(n_sched);
     }));
@@ -347,8 +353,8 @@ static void stage_sweep(Staging& s, const fpa_sweep_desc* d, fpa_sweep_desc& dd,
     dd.plan.dbeta   = s.out(pl.dbeta, B, true);
     dd.plan.valid   = s.out(pl.valid, B, true);
     dd.gain_lin     = s.out(d->gain_lin, P, map_gain);
-    dd.Pmax         = d->Pmax ? s.out(d->Pmax, P * 4, true) : nullptr;
-    dd.A_end        = d->A_end ? s.out(d->A_end, P * 8, true) : nullptr;
+    dd.Pmax         = d->Pmax ? s.out(d->Pmax, P * 4, true, kVecAlign) : nullptr;
+    dd.A_end        = d->A_end ? s.out(d->A_end, P * 8, true, kVecAlign) : nullptr;
     dd.status       = s.out(d->status, P, true);
 }
 

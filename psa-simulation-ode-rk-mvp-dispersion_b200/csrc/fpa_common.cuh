@@ -28,6 +28,13 @@ int  cuda_fail(cudaError_t e, const char* what);
         }                                         \
     } while (0)
 
+// FPA_ERR_INVALID unless `ptr` (NULL passes) is 16-byte aligned.  The kernels move complex128 values and rows of
+// maxima with 16-byte vector accesses, which fault on an address that is only 8-byte aligned.  For the device
+// pointers of the _dev entries, checked by the launchers; the host entries stage such arrays instead.
+#define FPA_REQUIRE_ALIGNED16(ptr, name)                                                           \
+    FPA_REQUIRE((reinterpret_cast<uintptr_t>(ptr) & 15) == 0, "%s must be 16-byte aligned (got %p)", \
+                name, (const void*)(ptr))
+
 // Selects `device` (must exist) -- there is no CPU fallback anywhere in this library.
 int use_device(int device);
 

@@ -73,6 +73,7 @@ int plan_launch(const fpa_plan_desc* d, double* dbeta_masked, cudaStream_t st) {
     int rc = plan_fill(d, p);
     if (rc != FPA_OK) return rc;
     FPA_REQUIRE(d->dbeta || dbeta_masked, "a dbeta output must be set");
+    FPA_REQUIRE_ALIGNED16(d->omega, "omega");  // stored with 16-byte vector stores
     p.dbeta_masked = dbeta_masked;
     const int64_t B = d->n1 * d->n3;
     if (B == 0) return FPA_OK;

@@ -599,8 +599,19 @@ int nwave_check(const fpa_nwave_desc* d) {
     return FPA_OK;
 }
 
+// The pointers of an N-wave descriptor that a kernel accesses 16 bytes at a time: the comb kernels move A0, A_trace
+// and A_end as complex128 pairs.  Both launchers apply the rule, so a _dev call does not depend on the kernel the
+// library picks; not part of nwave_check, which the host entries run on their own (staged) arrays.
+int nwave_check_aligned(const fpa_nwave_desc* d) {
+    FPA_REQUIRE_ALIGNED16(d->A0, "A0");
+    if (d->flags & FPA_OUT_TRACE) FPA_REQUIRE_ALIGNED16(d->A_trace, "A_trace");
+    if (d->flags & FPA_OUT_END) FPA_REQUIRE_ALIGNED16(d->A_end, "A_end");
+    return FPA_OK;
+}
+
 int nwave_launch(const fpa_nwave_desc* d, cudaStream_t st) {
     int rc = nwave_check(d);
+    if (rc == FPA_OK) rc = nwave_check_aligned(d);
     if (rc != FPA_OK) return rc;
     if (d->n_waves > 128) {
         set_error("n_waves = %d exceeds the kernel limit of 128", d->n_waves);
@@ -610,6 +621,7 @@ int nwave_launch(const fpa_nwave_desc* d, cudaStream_t st) {
     const bool fact = d->factored != nullptr && !(d->flags & FPA_NWAVE_PLAIN);
     if (fact) {
         FPA_REQUIRE(d->n_classes >= 0 && d->n_classes < kFactMaxCls, "n_classes must be the class count of `factored`");
+        FPA_REQUIRE_ALIGNED16(d->factored, "factored");  // its cell map is read with 16-byte loads
     } else {
         FPA_REQUIRE(d->n_triplets >= 0 && d->n_triplets < 2147483647LL, "bad n_triplets");
         FPA_REQUIRE(d->row_ptr != nullptr, "row_ptr must be set");

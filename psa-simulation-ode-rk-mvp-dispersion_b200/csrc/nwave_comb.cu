@@ -875,7 +875,8 @@ static cudaError_t comb_launch(const CombParams& p, cudaStream_t st) {
     return cudaGetLastError();
 }
 
-int nwave_check(const fpa_nwave_desc* d);  // nwave.cu
+int nwave_check(const fpa_nwave_desc* d);          // nwave.cu
+int nwave_check_aligned(const fpa_nwave_desc* d);  // nwave.cu
 
 // The limits of the convolution form: n_waves <= 128, grid_span <= 512.
 bool nwave_comb_fits(const fpa_nwave_desc* d) { return d->n_waves <= 128 && d->grid_span <= 512; }
@@ -883,6 +884,7 @@ bool nwave_comb_fits(const fpa_nwave_desc* d) { return d->n_waves <= 128 && d->g
 // d->grid_slot: device pointer to the N grid slots; span = number of grid slots covered.
 int nwave_comb_launch(const fpa_nwave_desc* d, cudaStream_t st) {
     int rc = nwave_check(d);
+    if (rc == FPA_OK) rc = nwave_check_aligned(d);
     if (rc != FPA_OK) return rc;
     FPA_REQUIRE(d->n_points < 2147483647LL, "bad n_points");
     if (!nwave_comb_fits(d)) {

@@ -1019,6 +1019,11 @@ int yaman4_launch(const fpa_yaman4_desc* d, cudaStream_t st) {
     const bool uniform = (d->flags & FPA_UNIFORM_PHYSICS) != 0;
     FPA_REQUIRE(!uniform || (d->gamma_stride == 0 && d->alpha_stride == 0),
                 "FPA_UNIFORM_PHYSICS needs broadcast gamma and alpha (stride 0)");
+    // load_state, save_sample and write_results access these with 16-byte (trace: also 32-byte) vector accesses
+    FPA_REQUIRE_ALIGNED16(d->A0, "A0");
+    if (trace) FPA_REQUIRE_ALIGNED16(d->A_trace, "A_trace");
+    if (endo) FPA_REQUIRE_ALIGNED16(d->A_end, "A_end");
+    if (pmax) FPA_REQUIRE_ALIGNED16(d->Pmax, "Pmax");
     if (d->n_points == 0) return FPA_OK;
 
     Yaman4Params p;
@@ -1096,6 +1101,10 @@ static int sweep_setup(const fpa_sweep_desc* d, int64_t n_phases, Yaman4Params& 
     FPA_REQUIRE(d->dz > 0.0, "dz must be positive");
     FPA_REQUIRE(d->save_every >= 1, "save_every must be a positive integer");
     FPA_REQUIRE(d->p_signal > 0.0, "p_in[2] (signal seed power) must be > 0 to define gain");
+    // sweep_prologue and sweep_epilogue store these with 16-byte vector stores
+    FPA_REQUIRE_ALIGNED16(d->plan.omega, "plan.omega");
+    FPA_REQUIRE_ALIGNED16(d->A_end, "A_end");
+    FPA_REQUIRE_ALIGNED16(d->Pmax, "Pmax");
     if (B == 0) return FPA_OK;
     const double sc = d->length_scale;
     const int64_t n_steps = fpa_interval_steps(d->z_max * sc, d->dz * sc);
@@ -1199,6 +1208,7 @@ int yaman4_phase_sweep_launch(const fpa_phase_sweep_desc* d, void* scratch, int6
     if (d && (d->sweep.flags & FPA_PHASE_EXACT)) return sweep_setup(&d->sweep, 1, p, x, n_grid);  // FPA_ERR_UNSUPPORTED
     int rc = phase_sweep_check(d);
     if (rc != FPA_OK) return rc;
+    FPA_REQUIRE_ALIGNED16(d->A0_table, "A0_table");  // read with 16-byte loads (sweep_initial_state)
     const int64_t K = d->n_phases;
     rc = sweep_setup(&d->sweep, K, p, x, n_grid);
     if (rc != FPA_OK || n_grid == 0) return rc;

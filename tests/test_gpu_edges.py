@@ -48,18 +48,22 @@ def test_degenerate_step_counts(gpu, oracle):
 
 
 def test_per_point_physics_equals_broadcast_bit_for_bit(gpu, oracle):
-    """gamma / alpha / A0 given per point (registers) or broadcast (constant bank): same bits; a ragged
-    batch (not a multiple of the block size) with distinct physics per point matches the oracle."""
+    """gamma / alpha / A0 given per point (registers) or broadcast (constant bank): same bits, also for runs
+    that start at z0 != 0 (dbeta*z0 up to ~50 rad), lossless and on the exact kernel; a ragged batch (not a
+    multiple of the block size) with distinct physics per point matches the oracle."""
     D = gpu._device
     rng = np.random.default_rng(5)
     B = 301
     db = rng.normal(size=B) * 0.02
     A0 = _A0(oracle, ph=[0.2, -0.1, 0.5, 1.0])
     kw = dict(z_max=30.0, n_steps=150, save_every=7, pmax=True)
-    a = D.yaman4_batch(db, 0.015, 2e-4, A0, **kw)
-    b = D.yaman4_batch(db, np.full(B, 0.015), np.full(B, 2e-4), np.tile(A0, (B, 1)), **kw)
-    for k in ("A_end", "Pmax", "status"):
-        assert np.array_equal(a[k], b[k])
+    for z0, alpha, exact in ((0.0, 2e-4, False), (5.0, 2e-4, False), (2000.0, 2e-4, False), (2000.0, 0.0, False),
+                             (2000.0, 2e-4, True)):
+        run = dict(kw, z0=z0, z_max=z0 + 30.0, trace=z0 != 0.0, phase_exact=exact)
+        a = D.yaman4_batch(db, 0.015, alpha, A0, **run)
+        b = D.yaman4_batch(db, np.full(B, 0.015), np.full(B, alpha), np.tile(A0, (B, 1)), **run)
+        for k in a:
+            assert np.array_equal(a[k], b[k]), (k, z0, alpha, exact)
     g = rng.uniform(0.005, 0.03, B)
     al = rng.uniform(0, 5e-4, B) * (rng.random(B) < 0.7)
     A0s = np.sqrt(rng.uniform(1e-6, 0.5, (B, 4))) * np.exp(1j * rng.uniform(-3, 3, (B, 4)))

@@ -1,17 +1,21 @@
 """GPU: the staging of the host-pointer entry points.  Which result buffers the kernels write directly (page-locked
 memory) and which go through the device workspace and a copy must not change what a caller gets: every output is
 byte-equal whether it lives in pageable, pinned (`_lib.pinned_empty`), registered (`fpa_host_register`) or mixed
-memory, and whether the optional outputs are requested or NULL.  The batch, sweep, phase-sweep and N-wave entries
-also equal their `_dev` entry on torch tensors given the descriptor the host entry builds, the *_multi_host entries
-with devices=[0, 0, 0] equal the single-device call, and a large call after a small one (the grow-only workspace)
-repeats its bytes."""
+memory, and whether the optional outputs are requested or NULL.  Registered memory also comes 16 bytes past a
+32-byte boundary (what glibc's malloc hands numpy) and 8 bytes past a 16-byte boundary (a complex128 array numpy
+still calls aligned, which the kernels' 16-byte stores cannot take: the library stages it).  The batch, sweep,
+phase-sweep and N-wave entries also equal their `_dev` entry on torch tensors given the descriptor the host entry
+builds (the batch also with A_trace and A_end 16 bytes past a 32-byte boundary), the *_multi_host entries with
+devices=[0, 0, 0] equal the single-device call in every memory kind, and a large call after a small one (the
+grow-only workspace) repeats its bytes."""
 import ctypes as C
 
 import numpy as np
 import pytest
 
 pytestmark = pytest.mark.gpu
-KINDS = ("pageable", "pinned", "registered", "mixed", "null")
+KINDS = ("pageable", "pinned", "registered", "registered+16", "registered+8", "mixed", "null")
+REGISTERED = {"registered": 0, "registered+16": 16, "registered+8": 8}   # kind -> byte offset past a page boundary
 P_IN, PHASE_IN = [0.1, 0.1, 1e-4, 2e-5], [0.1, -0.2, 0.3, 0.05]
 PAGE = 4096
 
@@ -29,14 +33,16 @@ class Mem:
         nbytes = int(np.prod(shape)) * np.dtype(dtype).itemsize
         if self.kind == "pinned" or (self.kind == "mixed" and self.n % 2):
             a = self.L.pinned_empty(shape, dtype)
-        elif self.kind == "registered":
-            # whole pages of its own: two registrations never share a page
-            span = -(-nbytes // PAGE) * PAGE
+        elif self.kind in REGISTERED:
+            # whole pages of its own: two registrations never share a page; the array starts `shift` bytes in
+            shift = REGISTERED[self.kind]
+            span = -(-(shift + nbytes) // PAGE) * PAGE
             buf = np.empty(span + PAGE, np.uint8)
             off = -buf.ctypes.data % PAGE
             self.L.register_host(buf[off:off + span])
             self.registered.append(buf[off:off + span])
-            a = buf[off:off + nbytes].view(dtype).reshape(shape)
+            a = buf[off + shift:off + shift + nbytes].view(dtype).reshape(shape)
+            assert a.ctypes.data % 32 == shift
         else:
             a = np.empty(shape, dtype)
         a.view(np.uint8)[...] = 0xA5
@@ -51,13 +57,13 @@ def _ptr(L, a):
     return None if a is None else L.ptr(a)
 
 
-def _run_kinds(gpu, build, size):
-    """{kind: {output: bytes}} of build(mem, size) run once per memory kind; all agree with 'pageable'."""
+def _run_kinds(gpu, build, size, devices=None):
+    """{kind: {output: bytes}} of build(mem, size, devices) run once per memory kind; all agree with 'pageable'."""
     L, got = gpu._lib, {}
     for kind in KINDS:
         mem = Mem(L, kind)
         try:
-            outs = build(mem, size)
+            outs = build(mem, size, devices)
             got[kind] = {k: v.tobytes() for k, v in outs.items() if v is not None}
         finally:
             mem.release()
@@ -77,10 +83,13 @@ def _dev_tensors(arrays):
             for k, v in arrays.items()}
 
 
-def _dev_out(template):
-    """Device buffers shaped like the host outputs (by bytes)."""
+def _dev_out(template, shift=None):
+    """Device buffers shaped like the host outputs (by bytes); the one named k in `shift` starts shift[k] bytes past
+    its (256-byte aligned) allocation."""
     import torch
-    return {k: torch.empty(len(v), dtype=torch.uint8, device="cuda:0") for k, v in template.items()}
+    shift = shift or {}
+    return {k: torch.empty(len(v) + shift.get(k, 0), dtype=torch.uint8, device="cuda:0")[shift.get(k, 0):]
+            for k, v in template.items()}
 
 
 def _stream():
@@ -94,23 +103,22 @@ def _sync_bytes(t):
     return {k: v.cpu().numpy().tobytes() for k, v in t.items()}
 
 
-def _check_sizes(gpu, build, sizes, dev=None, multi_size=None):
-    """Large, small, large: each size agrees across memory kinds (and with `dev`); the repeated size repeats."""
+def _check_sizes(gpu, build, sizes, devs=(), multi_size=None):
+    """Large, small, large: each size agrees across memory kinds (and with every run of `devs`); the repeated size
+    repeats; the multi-device entry agrees with the single-device one in every memory kind."""
     seen = {}
     for s in sizes:
         ref = _run_kinds(gpu, build, s)
         if s in seen:
             assert ref == seen[s]
         seen[s] = ref
-        if dev is not None:
+        for dev in devs:
             want = dev(s, ref)
             for k, v in want.items():
                 assert v == ref[k], (s, k)
     if multi_size is not None:
         one = _run_kinds(gpu, build, multi_size)
-        mem = Mem(gpu._lib, "pageable")
-        many = {k: v.tobytes() for k, v in build(mem, multi_size, devices=[0, 0, 0]).items()}
-        assert many == one
+        assert _run_kinds(gpu, build, multi_size, devices=[0, 0, 0]) == one
 
 
 # ----------------------------------------------------------------- 4-wave batch
@@ -151,21 +159,25 @@ def test_batch(gpu):
         gpu._device._run_host(lib.fpa_yaman4_rk4_batch_host, lib.fpa_yaman4_rk4_batch_multi_host, d, 0, devices)
         return out
 
-    def dev(B, ref):
-        inp = _batch_inputs(B)
-        t, o = _dev_tensors(inp), _dev_out(ref)
-        d = _batch_desc(L, B, {k: v.data_ptr() for k, v in t.items()}, o)
-        for k, v in o.items():
-            setattr(d, k, v.data_ptr())
-        d.flags |= L.UNIFORM_PHYSICS
-        d.gamma_uniform, d.alpha_uniform = float(inp["gamma"][0]), float(inp["alpha"][0])
-        nb = int(lib.fpa_yaman4_scratch_bytes(B))
-        scr = _dev_out({"s": bytes(nb)})["s"]
-        d.scratch, d.scratch_bytes = scr.data_ptr(), nb
-        L.check(lib.fpa_yaman4_rk4_batch_dev(C.byref(d), _stream()))
-        return _sync_bytes(o)
+    def dev(shift):
+        def run(B, ref):
+            inp = _batch_inputs(B)
+            t, o = _dev_tensors(inp), _dev_out(ref, shift)
+            d = _batch_desc(L, B, {k: v.data_ptr() for k, v in t.items()}, o)
+            for k, v in o.items():
+                setattr(d, k, v.data_ptr())
+            d.flags |= L.UNIFORM_PHYSICS
+            d.gamma_uniform, d.alpha_uniform = float(inp["gamma"][0]), float(inp["alpha"][0])
+            nb = int(lib.fpa_yaman4_scratch_bytes(B))
+            scr = _dev_out({"s": bytes(nb)})["s"]
+            d.scratch, d.scratch_bytes = scr.data_ptr(), nb
+            L.check(lib.fpa_yaman4_rk4_batch_dev(C.byref(d), _stream()))
+            return _sync_bytes(o)
+        return run
 
-    _check_sizes(gpu, build, [40_000, 1_000, 40_000], dev, multi_size=3 * 3_001 + 1)
+    # A_trace 16 bytes past a 32-byte boundary: the trace rows take the 16-byte store branch of save_sample
+    _check_sizes(gpu, build, [40_000, 1_000, 40_000], [dev({}), dev({"A_trace": 16, "A_end": 16})],
+                 multi_size=3 * 3_001 + 1)
 
 
 # ----------------------------------------------------------------- sweeps
@@ -232,7 +244,7 @@ def test_sweep(gpu, golden):
         L.check(lib.fpa_yaman4_sweep_dev(C.byref(d), scr.data_ptr(), nb, _stream()))
         return _sync_bytes(o)
 
-    _check_sizes(gpu, build, [4 * 20_000, 4 * 500, 4 * 20_000], dev, multi_size=4 * 2_501)
+    _check_sizes(gpu, build, [4 * 20_000, 4 * 500, 4 * 20_000], [dev], multi_size=4 * 2_501)
 
 
 def test_phase_sweep(gpu, golden):
@@ -273,7 +285,7 @@ def test_phase_sweep(gpu, golden):
         L.check(lib.fpa_yaman4_phase_sweep_dev(C.byref(d), scr.data_ptr(), nb, _stream()))
         return _sync_bytes(o)
 
-    _check_sizes(gpu, build, [2 * 10_000, 2 * 300, 2 * 10_000], dev, multi_size=2 * 1_501)
+    _check_sizes(gpu, build, [2 * 10_000, 2 * 300, 2 * 10_000], [dev], multi_size=2 * 1_501)
 
 
 # ----------------------------------------------------------------- N-wave
@@ -336,7 +348,7 @@ def test_nwave(gpu, form):
 
     # the comb kernel's thread mapping depends on the batch size (one warp per point from 4 * SM count points on):
     # the whole batch and its three shards stay below that threshold, so they run the same mapping
-    _check_sizes(gpu, build, [3_000, 50, 3_000], dev, multi_size=3 * 100 + 2)
+    _check_sizes(gpu, build, [3_000, 50, 3_000], [dev], multi_size=3 * 100 + 2)
 
 
 # ----------------------------------------------------------------- linear, RHS, Delta-beta table
@@ -372,7 +384,7 @@ def test_rhs(gpu):
         return out
 
     for B in (20_000, 3, 20_000):
-        for kind in KINDS[:4]:
+        for kind in KINDS[:-1]:
             mem = Mem(L, kind)
             try:
                 got = build(mem, B)["dA"].tobytes()

@@ -13,6 +13,10 @@ from conftest import rel_err
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-10
+# beta_6 .. beta_12 [s^n/m] about 1552 nm, orders 5, 9 and 11 zero: each order adds ~1e-2 1/m to Delta-beta
+# (beta_n * dw^n / n! with dw = 4e13 rad/s), far from underflow (beta_12 * dw^12 > 1e-30 for dw >= 1e11)
+TAYLOR_HIGH = {6: 1.8e-81, 7: -3.1e-94, 8: 6.2e-107, 10: -3.5e-132, 12: 2.9e-157}
+EVEN_12 = (2, 4, 6, 8, 10, 12)
 
 
 def _disp(fpa, b2, b3, b4, wref):
@@ -276,22 +280,28 @@ def test_dbeta_table_vs_oracle_all_methods(gpu, oracle):
     """The device front-end against the per-point oracle on a 2-D grid incl. invalid points.
     (a) beta0 = beta1 = 0: agreement 1e-12 on the scale of the Taylor terms and >= 90 % of the
     entries bit-equal; (b) beta0 ~ 6e6, beta1 ~ 5e-9 (general Taylor cancels 10 digits): within
-    8 ulp of the largest beta(omega)."""
+    8 ulp of the largest beta(omega).  Up to the supported Taylor order 12: every order from 6 on
+    adds ~1e-2 1/m at the 90th percentile of the grid (1e16 at the far outliers), orders 5, 9 and 11
+    are zero."""
     rng = np.random.default_rng(31)
     lam1 = rng.uniform(1540e-9, 1560e-9, 7)
     lam2 = rng.uniform(1540e-9, 1560e-9, 7)
     lam3 = np.concatenate((rng.uniform(1500e-9, 1600e-9, 40), [700e-9, 780e-9, 3e-6]))
     wref = oracle.omega_from_lambda(1552e-9)
     PM = gpu.phase_matching.PhaseMatchingConfig
-    cases = ((PM(method="general_taylor", max_order=6), oracle.GENERAL_TAYLOR, dict(max_order=6)),
-             (PM(method="general_taylor", max_order=3), oracle.GENERAL_TAYLOR, dict(max_order=3)),
-             (PM(method="symmetric_even", even_orders=(2, 4, 6)), oracle.SYMMETRIC_EVEN, dict(even_orders=(2, 4, 6))),
-             (PM(method="provided", provided_delta_beta=0.125), oracle.PROVIDED, dict(provided=0.125)))
+    low, high = {6: 2e-85}, TAYLOR_HIGH
+    cases = ((PM(method="general_taylor", max_order=6), oracle.GENERAL_TAYLOR, dict(max_order=6), low),
+             (PM(method="general_taylor", max_order=3), oracle.GENERAL_TAYLOR, dict(max_order=3), low),
+             (PM(method="symmetric_even", even_orders=(2, 4, 6)), oracle.SYMMETRIC_EVEN, dict(even_orders=(2, 4, 6)),
+              low),
+             (PM(method="provided", provided_delta_beta=0.125), oracle.PROVIDED, dict(provided=0.125), low),
+             (PM(method="general_taylor", max_order=12), oracle.GENERAL_TAYLOR, dict(max_order=12), high),
+             (PM(method="symmetric_even", even_orders=EVEN_12), oracle.SYMMETRIC_EVEN, dict(even_orders=EVEN_12), high))
     for b0, b1, abs_tol in ((0.0, 0.0, None), (5.8e6, 4.9e-9, 8 * np.spacing(5.9e6))):
-        disp = gpu.dispersion.DispersionParams(omega_ref=wref, beta0=b0, beta1=b1, beta2=-2.6e-29, beta3=3.3e-41,
-                                               beta4=-1.6e-55, extra={6: 2e-85})
-        odisp = oracle.Taylor(wref, b0, b1, -2.6e-29, 3.3e-41, -1.6e-55, extra={6: 2e-85})
-        for cfg, ometh, okw in cases:
+        for cfg, ometh, okw, extra in cases:
+            disp = gpu.dispersion.DispersionParams(omega_ref=wref, beta0=b0, beta1=b1, beta2=-2.6e-29, beta3=3.3e-41,
+                                                   beta4=-1.6e-55, extra=extra)
+            odisp = oracle.Taylor(wref, b0, b1, -2.6e-29, 3.3e-41, -1.6e-55, extra=extra)
             plan, keep = gpu._device.new_plan_desc(lam1, lam2, lam3)
             gpu.phase_matching.fill_plan_desc(plan, disp, cfg)
             out = gpu._device.dbeta_table(plan, want_omega=True)
@@ -312,11 +322,42 @@ def test_dbeta_table_vs_oracle_all_methods(gpu, oracle):
                     n_equal += int(got == ref)
                     if abs_tol is None or ometh != oracle.GENERAL_TAYLOR:
                         assert abs(got - ref) <= 1e-12 * max(abs(ref), 1e-3)
-                    else:
+                    elif extra is low:
                         assert abs(got - ref) <= abs_tol
+                    else:   # the high orders make beta(omega) of the far outliers ~1e16: 8 ulp of that point's largest
+                        big = max(abs(oracle.beta_taylor(w, odisp, okw["max_order"])) for w in om)
+                        assert abs(got - ref) <= max(abs_tol, 8 * np.spacing(big))
             assert n_bad >= 7
             if abs_tol is None:
                 assert n_equal >= 0.9 * n_ok, f"only {n_equal}/{n_ok} dbeta entries bit-equal"
+
+
+@pytest.mark.parametrize("unit", ["m", "km"])
+def test_sweep_at_taylor_order_12_vs_oracle(gpu, oracle, unit):
+    """The fused sweep with general Taylor to order 12 (the same coefficients as above): the reported dbeta uses
+    beta_n as given, the integration beta_n / 1000 in km -- every coefficient of the table is rescaled.  Order 12
+    moves the gain of the outer signal wavelengths by up to 1 %."""
+    s = 1.0 if unit == "m" else 1e3
+    wref = oracle.omega_from_lambda(1552e-9)
+    lam1, lam3 = np.array([1549e-9, 1551e-9]), np.linspace(1500e-9, 1600e-9, 7)
+    extra = {n: v * s for n, v in TAYLOR_HIGH.items()}
+    disp = gpu.dispersion.DispersionParams(omega_ref=wref, beta2=-2.6e-29 * s, beta3=3.3e-41 * s, beta4=-1.6e-55 * s,
+                                           extra=extra)
+    odisp = oracle.Taylor(wref, 0.0, 0.0, -2.6e-29 * s, 3.3e-41 * s, -1.6e-55 * s, extra=extra)
+    p_in = [0.3, 0.3, 1e-4, 0.0]
+    cfg = gpu.config.custom_simulation_config(z_max=300.0 / s, dz=1.0 / s, save_every=10)
+    r = gpu.scan_mismtach.sweep_gain_2d(
+        cfg=cfg, lambda_p1_m=lam1, lambda_p2_m=1558e-9, lambda_signal_m=lam3, gamma=11.5e-3 * s, alpha=2e-4 * s,
+        p_in=p_in, dispersion=disp, length_unit=unit, gain_unit="linear",
+        phase_matching_cfg=gpu.phase_matching.PhaseMatchingConfig(method="general_taylor", max_order=12))
+    for i in range(lam1.size):
+        g_ref, d_ref = oracle.sweep_lambda3_gain(
+            lam1=lam1[i], lam2=1558e-9, lam3_arr=lam3, z_max=300.0 / s, dz=1.0 / s, save_every=10, check_nan=True,
+            gamma=11.5e-3 * s, alpha=2e-4 * s, p_in=p_in, disp=odisp, method=oracle.GENERAL_TAYLOR, max_order=12,
+            length_unit=unit, gain_unit="linear")
+        assert np.isfinite(g_ref).all()
+        assert rel_err(r["gain"][i], g_ref) < TOL
+        assert np.max(np.abs(r["dbeta"][i] - d_ref)) <= 1e-12 * np.max(np.abs(d_ref))
 
 
 # ------------------------------------------------------------------ properties at full size
