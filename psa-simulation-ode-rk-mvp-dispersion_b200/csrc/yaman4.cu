@@ -35,6 +35,12 @@
 //    4-double state (x1, y1, x3, y3) with the same expressions in the same operand order: 186 instead of
 //    298 FP64 instructions per lossy step and the same bits (DESIGN.md §4.1c).  The launcher decides by a
 //    memcmp of A0's bit patterns; FPA_SWEEP_SYM=0 forces the 4-wave kernels.
+//    Each family -- the batch (yaman4_fast_kernel) and the fused sweep (yaman4_sweep_kernel) -- has one per-point
+//    body, fast_point / sweep_run_point.  Its whole-run kernel runs it once, for the single segment [0, n_steps); its
+//    z-segment scheduler kernel (yaman4_fast_seg_kernel / yaman4_sweep_seg_kernel) runs it once per work item through
+//    seg_items, with the point carried between segments in a SegRecord.  Both families write a point's outputs with
+//    write_results / write_nan_outputs, and launch_fast_family makes the lossy / lossless and segmented / whole-run
+//    choice for both.
 //  * yaman4_exact_kernel -- FPA_PHASE_EXACT or an explicit z-grid: the reference's arithmetic
 //    structure step by step (h_i by subtraction, sincos at z, z+h/2, z+h, k_j formed, y + h/6*(..)).
 #include "plan_point.cuh"
@@ -184,32 +190,44 @@ __device__ __forceinline__ void rk_stage(const double (&in)[4], const double (&b
     stage_sym<LOSS>(in, base, qr, qi, cg, c2g, cn, out, S);
 }
 
-__device__ __forceinline__ void load_state(const Yaman4Params& p, int64_t b, double (&y)[8]) {
-    const double2* a0 = reinterpret_cast<const double2*>(p.A0) + b * p.A0_stride * 4;
+// One state (4 x complex128, 16-byte aligned): A0 of a batch point, a row of the phase sweep's A0_table.
+__device__ __forceinline__ void load_c128x4(const double* a, double (&y)[8]) {
+    const double2* a2 = reinterpret_cast<const double2*>(a);
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
-        const double2 v = a0[j];
+        const double2 v = a2[j];
         y[2 * j] = v.x;
         y[2 * j + 1] = v.y;
     }
+}
+
+__device__ __forceinline__ void load_state(const Yaman4Params& p, int64_t b, double (&y)[8]) {
+    load_c128x4(p.A0 + b * p.A0_stride * 8, y);
+}
+
+// A_end and Pmax all NaN and status 0 (failed at step 0) under the check: the outputs of a point that is not
+// integrated.
+__device__ __forceinline__ void write_nan_outputs(const Yaman4Params& p, int64_t b) {
+    const double qn = qnan();
+    if (p.A_end)
+        for (int j = 0; j < 4; ++j) store_c128(p.A_end + b * 8 + 2 * j, qn, qn);
+    if (p.Pmax)
+        for (int j = 0; j < 4; ++j) p.Pmax[b * 4 + j] = qn;
+    if (p.status) p.status[b] = p.check ? 0 : FPA_POINT_OK;
 }
 
 // A point whose dbeta is not finite: exp(i*dbeta*z) is NaN from the first stage on, every later
 // sample is NaN and step 0 is the bad one (integrators.py:132-135).  Invalid scan points of a sweep
 // arrive here with dbeta = NaN and cost nothing.
 __device__ __noinline__ void write_invalid_point(const Yaman4Params& p, int64_t b, const double (&y)[8]) {
-    const double qn = qnan();
     if (p.A_trace) {
-        double* t = p.A_trace + b * p.n_saved * 8;
+        const double qn = qnan();
+        double*      t  = p.A_trace + b * p.n_saved * 8;
         for (int j = 0; j < 4; ++j) store_c128(t + 2 * j, y[2 * j], y[2 * j + 1]);
         for (int64_t s = 1; s < p.n_saved; ++s)
             for (int j = 0; j < 4; ++j) store_c128(t + s * 8 + 2 * j, qn, qn);
     }
-    if (p.A_end)
-        for (int j = 0; j < 4; ++j) store_c128(p.A_end + b * 8 + 2 * j, qn, qn);
-    if (p.Pmax)
-        for (int j = 0; j < 4; ++j) p.Pmax[b * 4 + j] = qn;
-    if (p.status) p.status[b] = p.check ? 0 : FPA_POINT_OK;
+    write_nan_outputs(p, b);
 }
 
 // LAST: *plast = |A3|^2 of this sample, so that after the run it holds the LAST saved sample's signal power (the
@@ -255,8 +273,10 @@ __device__ __forceinline__ void save_sample(const double (&y)[4], double*&, doub
     }
 }
 
-__device__ __forceinline__ void write_results(const Yaman4Params& p, int64_t b, const double (&y)[8],
-                                              const double (&pm)[4], bool pmax, int32_t bad) {
+// Outputs of an integrated point: status (the end state's finite check decides a run that was finite until its
+// last step), A_end and, when pmax, Pmax.  Returns the point's first bad step (FPA_POINT_OK: none).
+__device__ __forceinline__ int32_t write_results(const Yaman4Params& p, int64_t b, const double (&y)[8],
+                                                 const double (&pm)[4], bool pmax, int32_t bad) {
     if (p.check && bad == FPA_POINT_OK) {
         bool nf = false;
 #pragma unroll
@@ -273,6 +293,7 @@ __device__ __forceinline__ void write_results(const Yaman4Params& p, int64_t b, 
         o[0] = make_double2(pm[0], pm[1]);
         o[1] = make_double2(pm[2], pm[3]);
     }
+    return bad;
 }
 
 // The z-loop of the fast path: advances y over the steps [i0, i1) of the run, keeps the running maxima
@@ -368,33 +389,6 @@ __device__ __forceinline__ int32_t fast_integrate(const Yaman4Params& p, int64_t
     return bad;
 }
 
-// UNIFORM: 0 = gamma/alpha per thread; 1 = uniform physics, coefficients from the constant bank;
-// 2 = uniform and lossless (alpha == 0): the 32 loss FMAs per step are not issued.
-template <bool TRACE, bool PMAX, int UNIFORM, int THREADS, int MIN_BLOCKS>
-__global__ void __launch_bounds__(THREADS, MIN_BLOCKS) yaman4_fast_kernel(const Yaman4Params p) {
-    const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (b >= p.n_points) return;
-
-    double y[8];
-    load_state(p, b, y);
-    const double dbeta = p.dbeta[b];
-    if (nonfinite(dbeta)) {
-        write_invalid_point(p, b, y);
-        return;
-    }
-    // stage-weighted coefficients: from the constant bank when the physics is uniform over the
-    // batch (sweeps), else per thread
-    Yaman4Coef cf;
-    if (UNIFORM != 0) {
-        cf = p.coef;
-    } else {
-        cf = make_coef(p.gamma[b * p.gamma_stride], p.alpha[b * p.alpha_stride], p.h);
-    }
-    double        pm[4] = {0.0, 0.0, 0.0, 0.0};
-    const int32_t bad = fast_integrate<TRACE, PMAX, UNIFORM != 2>(p, b, dbeta, cf, y, pm);
-    write_results(p, b, y, pm, PMAX, bad);
-}
-
 // ------------------------------------------------------------------ z-segment scheduler
 // The integrators as PERSISTENT kernels for batches of one wave or more.  Every point costs the same, so a
 // batch of 1.65 waves (125 000 points per GPU when the 1e6-point grid is split over 8 GPUs) runs as one
@@ -402,9 +396,10 @@ __global__ void __launch_bounds__(THREADS, MIN_BLOCKS) yaman4_fast_kernel(const 
 // most warps sets the time.  Here the fiber is cut into segments of seg_steps RK4 steps and the work
 // items (warp of 32 points, segment) are handed out in segment-major order from one atomic counter to
 // the resident warps: the chip stays full until the last seg_steps of the last item, so the tail costs
-// at most one segment instead of one wave.  Between segments a point's state (y, running maxima, first
-// bad step, its Delta-beta: 14 doubles + 1 int, SoA) goes through global memory -- 116 B per point per
-// segment, L2-resident -- and done[w] counts the finished segments of warp-item w (release / acquire).
+// at most one segment instead of one wave.  Between segments a point's record (y, running maxima, first
+// bad step and, for the sweeps, its Delta-beta: at most 14 doubles + 1 int, SoA) goes through global memory --
+// up to 116 B per point per segment, L2-resident -- and done[w] counts the finished segments of warp-item w
+// (release / acquire).
 // When item t is handed out at most R-1 older items (R = resident warps) can still be running, and the
 // launcher only segments batches of n_warps >= R items per segment, so the item t depends on, t - n_warps,
 // is normally finished: the acquire loop is a correctness guard, not a wait.  Segment boundaries are
@@ -413,13 +408,54 @@ __global__ void __launch_bounds__(THREADS, MIN_BLOCKS) yaman4_fast_kernel(const 
 struct SegParams {
     unsigned int* counter;    // [1] next work item (zeroed by the launcher)
     int*          done;       // [n_warps] finished segments per warp-item (zeroed by the launcher)
-    double*       state;      // [kSegDoubles][n_pad]
+    double*       state;      // [kSegDoubles or kSegDoublesPhase][n_pad]: the records below
     int32_t*      bad;        // [n_pad]
     int64_t       n_pad;      // n_warps * 32
     int           n_warps, n_seg, seg_steps;
 };
-constexpr int kSegDoubles = 13;  // y[8], pm[4], dbeta
-constexpr int kSegDoublesPhase = kSegDoubles + 1;  // the phase sweep adds the last saved signal power
+// The record of point b: slot s at state[s * n_pad + b], the first bad step at bad[b].  Slots: the state y from
+// kSegY (8 doubles; symmetric path: the 4 of (x1, y1, x3, y3)), the running maxima from kSegPmax (symmetric path:
+// those of waves 1 and 3 only), the sweep's integration Delta-beta at kSegDbeta (the batch path re-reads dbeta[b]
+// and leaves it unused) and the phase sweep's last saved signal power at kSegPlast.
+constexpr int kSegY = 0, kSegPmax = 8, kSegDbeta = 12, kSegPlast = 13;
+constexpr int kSegDoubles      = kSegDbeta + 1;  // batch, plain sweep
+constexpr int kSegDoublesPhase = kSegPlast + 1;  // phase sweep
+
+// Point b's view of its record.
+struct SegRecord {
+    const SegParams& g;
+    int64_t          b;
+    double*          st;  // slot 0 of point b
+    __device__ __forceinline__ SegRecord(const SegParams& g, int64_t b) : g(g), b(b), st(g.state + b) {}
+    __device__ __forceinline__ double* slot(int s) const { return st + s * g.n_pad; }
+
+    // Saves (store) or restores (load) the state y of NS doubles, the maxima when PMAX (NS = 4: those of waves 1
+    // and 3), the last saved signal power when LAST, and the first bad step.
+    template <bool PMAX, bool LAST, int NS>
+    __device__ __forceinline__ void store(const double (&y)[NS], const double (&pm)[4], double plast, int32_t bad) const {
+        constexpr int PM_STEP = NS == 8 ? 1 : 2;
+#pragma unroll
+        for (int j = 0; j < NS; ++j) __stcg(slot(kSegY + j), y[j]);
+        if (PMAX) {
+#pragma unroll
+            for (int j = 0; j < 4; j += PM_STEP) __stcg(slot(kSegPmax + j), pm[j]);
+        }
+        if (LAST) __stcg(slot(kSegPlast), plast);
+        __stcg(g.bad + b, bad);
+    }
+    template <bool PMAX, bool LAST, int NS>
+    __device__ __forceinline__ void load(double (&y)[NS], double (&pm)[4], double& plast, int32_t& bad) const {
+        constexpr int PM_STEP = NS == 8 ? 1 : 2;
+#pragma unroll
+        for (int j = 0; j < NS; ++j) y[j] = __ldcg(slot(kSegY + j));
+        if (PMAX) {
+#pragma unroll
+            for (int j = 0; j < 4; j += PM_STEP) pm[j] = __ldcg(slot(kSegPmax + j));
+        }
+        if (LAST) plast = __ldcg(slot(kSegPlast));
+        bad = __ldcg(g.bad + b);
+    }
+};
 
 __device__ __forceinline__ int ld_acquire(const int* p) {
     int v;
@@ -451,55 +487,73 @@ __device__ __forceinline__ void seg_publish(const SegParams& g, int lane, int se
     if (lane == 0) st_release(g.done + w, seg + 1);
 }
 
-// The batch integrator through the z-segment scheduler:
-// same arithmetic as yaman4_fast_kernel, bit-identical results.  Uniform physics only (UNIFORM = 1 | 2).
-template <bool TRACE, bool PMAX, int UNIFORM, int THREADS, int MIN_BLOCKS>
-__global__ void __launch_bounds__(THREADS, MIN_BLOCKS) yaman4_fast_seg_kernel(const Yaman4Params p, const SegParams g) {
+// The persistent kernels' loop: point(b, seg, last) for point b = 32 w + lane of every work item (w, seg) this warp
+// takes, b past the batch included; last: seg is the fiber's last segment.
+template <typename Point>
+__device__ __forceinline__ void seg_items(const SegParams& g, Point point) {
     const int lane = threadIdx.x & 31;
     int       seg, w;
     while (seg_next_item(g, lane, seg, w)) {
-        const int64_t b = (int64_t)w * 32 + lane;
-        const bool    last = seg == g.n_seg - 1;
-        if (b < p.n_points) {
-            const double dbeta = p.dbeta[b];
-            double       y[8], pm[4] = {0.0, 0.0, 0.0, 0.0};
-            int32_t      bad = FPA_POINT_OK;
-            double* const st = g.state + b;
-            if (nonfinite(dbeta)) {
-                if (seg == 0) {
-                    load_state(p, b, y);
-                    write_invalid_point(p, b, y);
-                }
-            } else {
-                if (seg == 0) {
-                    load_state(p, b, y);
-                } else {
-#pragma unroll
-                    for (int j = 0; j < 8; ++j) y[j] = __ldcg(st + j * g.n_pad);
-                    if (PMAX) {
-#pragma unroll
-                        for (int j = 0; j < 4; ++j) pm[j] = __ldcg(st + (8 + j) * g.n_pad);
-                    }
-                    bad = __ldcg(g.bad + b);
-                }
-                const int i0 = seg * g.seg_steps;
-                const int i1 = last ? p.n_steps : i0 + g.seg_steps;
-                bad = fast_integrate<TRACE, PMAX, UNIFORM != 2, true>(p, b, dbeta, p.coef, y, pm, i0, i1, bad);
-                if (last) {
-                    write_results(p, b, y, pm, PMAX, bad);
-                } else {
-#pragma unroll
-                    for (int j = 0; j < 8; ++j) __stcg(st + j * g.n_pad, y[j]);
-                    if (PMAX) {
-#pragma unroll
-                        for (int j = 0; j < 4; ++j) __stcg(st + (8 + j) * g.n_pad, pm[j]);
-                    }
-                    __stcg(g.bad + b, bad);
-                }
-            }
-        }
+        const bool last = seg == g.n_seg - 1;
+        point((int64_t)w * 32 + lane, seg, last);
         if (!last) seg_publish(g, lane, seg, w);
     }
+}
+
+// ------------------------------------------------------------------ batch integrator
+// Point b of a batch (nothing when b >= n_points): the whole run (SEG = false, seg = 0, last), or segment `seg` of
+// it on the z-segment scheduler.  y is the kernel's array, and A0 is read ahead of dbeta[b] on the whole run only:
+// write_invalid_point takes y's address, and with y a local of this function, or one read order for both kernels,
+// the compiler emits different machine code for the two kernels (same results).
+// UNIFORM: 0 = gamma/alpha per thread (whole run only); 1 = uniform physics, coefficients from the constant bank;
+// 2 = uniform and lossless (alpha == 0): the 32 loss FMAs per step are not issued.
+template <bool TRACE, bool PMAX, int UNIFORM, bool SEG>
+__device__ __forceinline__ void fast_point(const Yaman4Params& p, const SegParams& g, int64_t b, int seg, bool last,
+                                           double (&y)[8]) {
+    if (b >= p.n_points) return;
+    if (!SEG) load_state(p, b, y);
+    const double    dbeta = p.dbeta[b];
+    double          pm[4] = {0.0, 0.0, 0.0, 0.0}, plast;
+    int32_t         bad = FPA_POINT_OK;
+    const SegRecord rec(g, b);
+    if (nonfinite(dbeta)) {
+        if (seg == 0) {
+            if (SEG) load_state(p, b, y);
+            write_invalid_point(p, b, y);
+        }
+        return;
+    }
+    if (seg == 0) {
+        if (SEG) load_state(p, b, y);
+    } else {
+        rec.load<PMAX, false>(y, pm, plast, bad);
+    }
+    const int i0 = seg * g.seg_steps;
+    const int i1 = last ? p.n_steps : i0 + g.seg_steps;
+    if constexpr (UNIFORM != 0) {
+        bad = fast_integrate<TRACE, PMAX, UNIFORM != 2, SEG>(p, b, dbeta, p.coef, y, pm, i0, i1, bad);
+    } else {
+        const Yaman4Coef cf = make_coef(p.gamma[b * p.gamma_stride], p.alpha[b * p.alpha_stride], p.h);
+        bad = fast_integrate<TRACE, PMAX, UNIFORM != 2, SEG>(p, b, dbeta, cf, y, pm, i0, i1, bad);
+    }
+    if (last) {
+        write_results(p, b, y, pm, PMAX, bad);
+    } else {
+        rec.store<PMAX, false>(y, pm, plast, bad);
+    }
+}
+
+template <bool TRACE, bool PMAX, int UNIFORM, int THREADS, int MIN_BLOCKS>
+__global__ void __launch_bounds__(THREADS, MIN_BLOCKS) yaman4_fast_kernel(const Yaman4Params p) {
+    double y[8];
+    fast_point<TRACE, PMAX, UNIFORM, false>(p, SegParams{}, (int64_t)blockIdx.x * blockDim.x + threadIdx.x, 0, true, y);
+}
+
+// The batch integrator on the z-segment scheduler: uniform physics only (UNIFORM = 1 | 2).
+template <bool TRACE, bool PMAX, int UNIFORM, int THREADS, int MIN_BLOCKS>
+__global__ void __launch_bounds__(THREADS, MIN_BLOCKS) yaman4_fast_seg_kernel(const Yaman4Params p, const SegParams g) {
+    double y[8];
+    seg_items(g, [&](int64_t b, int seg, bool last) { fast_point<TRACE, PMAX, UNIFORM, true>(p, g, b, seg, last, y); });
 }
 
 // ------------------------------------------------------------------ fused sweep
@@ -550,13 +604,7 @@ __device__ __forceinline__ void sweep_point(const X& x, int64_t b, int64_t& gp, 
 template <typename X>
 __device__ __forceinline__ void sweep_initial_state(const X& x, int64_t k, double (&y)[8]) {
     if constexpr (kPhase<X>) {
-        const double2* a0 = reinterpret_cast<const double2*>(x.A0_table) + k * 4;
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-            const double2 v = a0[j];
-            y[2 * j] = v.x;
-            y[2 * j + 1] = v.y;
-        }
+        load_c128x4(x.A0_table + k * 8, y);
     } else {
 #pragma unroll
         for (int j = 0; j < 8; ++j) y[j] = x.A0[j];
@@ -627,34 +675,14 @@ __device__ __forceinline__ bool sweep_prologue(const SweepExtra& x, int64_t b, d
 
 // the reference's per-point try/except leaves NaN (scan_mismtach.py:736-738)
 __device__ __forceinline__ void sweep_invalid(const Yaman4Params& p, const SweepExtra& x, int64_t b) {
-    const double qn = qnan();
-    if (p.A_end)
-        for (int j = 0; j < 4; ++j) store_c128(p.A_end + b * 8 + 2 * j, qn, qn);
-    if (p.Pmax)
-        for (int j = 0; j < 4; ++j) p.Pmax[b * 4 + j] = qn;
-    if (p.status) p.status[b] = p.check ? 0 : FPA_POINT_OK;
-    store_gain(x, b, qn);
+    write_nan_outputs(p, b);
+    store_gain(x, b, qnan());
 }
 
 // Epilogue of an integrated point: status, optional end state / maxima, and the sweep's gain metric P3 / p_in[2].
 __device__ __forceinline__ void sweep_epilogue(const Yaman4Params& p, const SweepExtra& x, int64_t b,
                                                const double (&y)[8], const double (&pm)[4], int32_t bad, double P3) {
-    if (p.check && bad == FPA_POINT_OK) {
-        bool nf = false;
-#pragma unroll
-        for (int j = 0; j < 8; ++j) nf |= nonfinite(y[j]);
-        if (nf) bad = p.n_steps - 1;
-    }
-    if (p.status) p.status[b] = p.check ? bad : FPA_POINT_OK;
-    if (p.A_end) {
-#pragma unroll
-        for (int j = 0; j < 4; ++j) store_c128(p.A_end + b * 8 + 2 * j, y[2 * j], y[2 * j + 1]);
-    }
-    if (p.Pmax) {
-        double2* o = reinterpret_cast<double2*>(p.Pmax + b * 4);
-        o[0] = make_double2(pm[0], pm[1]);
-        o[1] = make_double2(pm[2], pm[3]);
-    }
+    bad = write_results(p, b, y, pm, p.Pmax != nullptr, bad);
     // gain = max_saved |A3|^2 / p_in[2]; NaN for failed, non-finite or <= 0 (scan_mismtach.py:723-734).  The
     // phase sweep's "end" metric takes P3 from the last saved sample under the same rule.
     double gain = qnan();
@@ -665,105 +693,65 @@ __device__ __forceinline__ void sweep_epilogue(const Yaman4Params& p, const Swee
     store_gain(x, b, gain);
 }
 
+// Point b of a sweep launch (nothing when b >= n_points): the whole run (SEG = false, seg = 0, last), or segment
+// `seg` of it on the z-segment scheduler.  The prologue runs at segment 0, the gain epilogue at the last; between
+// segments the record carries the integration Delta-beta, NaN for an invalid point, which then runs no segment.
 // X = PhaseSweepExtra: the phase sweep.  SYM (plain sweep only): A0 is symmetric, the z-loop runs on (A1, A3).
-template <bool LOSS, int THREADS, int MIN_BLOCKS, typename X, bool SYM = false>
-__global__ void __launch_bounds__(THREADS, MIN_BLOCKS) yaman4_sweep_kernel(const Yaman4Params p, const X x) {
+template <bool LOSS, typename X, bool SYM, bool SEG>
+__device__ __forceinline__ void sweep_run_point(const Yaman4Params& p, const X& x, const SegParams& g, int64_t b,
+                                                int seg, bool last) {
     constexpr bool PHASE = kPhase<X>;
     static_assert(!(SYM && PHASE), "the phase sweep has no symmetric path");
-    const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= p.n_points) return;
-    int64_t gp, k;
-    sweep_point(x, b, gp, k);
-    double db_run;
-    if (!sweep_prologue(x, gp, db_run, k == 0)) {
-        sweep_invalid(p, x, b);
-        return;
-    }
-    double y[kStateLen<SYM>];
-    sweep_initial_state(x, k, y);
-    double        pm[4] = {0.0, 0.0, 0.0, 0.0}, plast = 0.0;
-    const int32_t bad = fast_integrate<false, true, LOSS, false, PHASE, SYM>(p, b, db_run, p.coef, y, pm, 0, 0,
-                                                                             FPA_POINT_OK, &plast);
-    if constexpr (SYM) {
-        double yf[8];
-        sym_expand(y, yf, pm);
-        sweep_epilogue(p, x, b, yf, pm, bad, pm[2]);
+    double          y[kStateLen<SYM>], pm[4] = {0.0, 0.0, 0.0, 0.0}, db_run, plast = 0.0;
+    int32_t         bad = FPA_POINT_OK;
+    bool            run;
+    const SegRecord rec(g, b);
+    if (seg == 0) {
+        int64_t gp, k;
+        sweep_point(x, b, gp, k);
+        run = sweep_prologue(x, gp, db_run, k == 0);
+        if (!run) {
+            sweep_invalid(p, x, b);
+            if (!SEG) return;
+            db_run = qnan();
+        }
+        sweep_initial_state(x, k, y);
     } else {
-        sweep_epilogue(p, x, b, y, pm, bad, sweep_metric(x, pm, plast));
+        db_run = __ldcg(rec.slot(kSegDbeta));
+        run = !nonfinite(db_run);
+        if (run) rec.load<true, PHASE>(y, pm, plast, bad);
+    }
+    if (run) {
+        const int i0 = seg * g.seg_steps;
+        const int i1 = last ? p.n_steps : i0 + g.seg_steps;
+        bad = fast_integrate<false, true, LOSS, SEG, PHASE, SYM>(p, b, db_run, p.coef, y, pm, i0, i1, bad, &plast);
+        if (last) {
+            if constexpr (SYM) {
+                double yf[8];
+                sym_expand(y, yf, pm);
+                sweep_epilogue(p, x, b, yf, pm, bad, pm[2]);
+            } else {
+                sweep_epilogue(p, x, b, y, pm, bad, sweep_metric(x, pm, plast));
+            }
+        }
+    }
+    if (!last) {
+        __stcg(rec.slot(kSegDbeta), db_run);
+        if (run) rec.store<true, PHASE>(y, pm, plast, bad);
     }
 }
 
-// ------------------------------------------------------------------ fused sweep, z-segment scheduler
-// The sweep kernel above as a persistent kernel on the z-segment scheduler: prologue at segment 0, gain
-// epilogue at the last segment, the point's integration Delta-beta travels with its state (phase sweep: and the
-// last saved signal power, record kSegDoubles of the state).  SYM: the record carries the symmetric state
-// (x1, y1, x3, y3) in slots 0-3 and the maxima of waves 1 and 3 in slots 8 and 10.
+template <bool LOSS, int THREADS, int MIN_BLOCKS, typename X, bool SYM = false>
+__global__ void __launch_bounds__(THREADS, MIN_BLOCKS) yaman4_sweep_kernel(const Yaman4Params p, const X x) {
+    sweep_run_point<LOSS, X, SYM, false>(p, x, SegParams{}, (int64_t)blockIdx.x * blockDim.x + threadIdx.x, 0, true);
+}
+
+// The sweep kernel on the z-segment scheduler.
 template <bool LOSS, int THREADS, int MIN_BLOCKS, typename X, bool SYM = false>
 __global__ void __launch_bounds__(THREADS, MIN_BLOCKS)
     yaman4_sweep_seg_kernel(const Yaman4Params p, const X x, const SegParams g) {
-    constexpr bool PHASE = kPhase<X>;
-    static_assert(!(SYM && PHASE), "the phase sweep has no symmetric path");
-    constexpr int NS = kStateLen<SYM>, PM_STEP = SYM ? 2 : 1;
-    const int lane = threadIdx.x & 31;
-    int       seg, w;
-    while (seg_next_item(g, lane, seg, w)) {
-        const int64_t b = (int64_t)w * 32 + lane;
-        const bool    last = seg == g.n_seg - 1;
-        if (b < p.n_points) {
-            double  y[NS], pm[4] = {0.0, 0.0, 0.0, 0.0}, db_run, plast = 0.0;
-            int32_t bad = FPA_POINT_OK;
-            bool    run;
-            double* const st = g.state + b;
-            if (seg == 0) {
-                int64_t gp, k;
-                sweep_point(x, b, gp, k);
-                run = sweep_prologue(x, gp, db_run, k == 0);
-                if (!run) {
-                    sweep_invalid(p, x, b);
-                    db_run = qnan();
-                }
-                sweep_initial_state(x, k, y);
-            } else {
-                db_run = __ldcg(st + 12 * g.n_pad);
-                run = !nonfinite(db_run);
-                if (run) {
-#pragma unroll
-                    for (int j = 0; j < NS; ++j) y[j] = __ldcg(st + j * g.n_pad);
-#pragma unroll
-                    for (int j = 0; j < 4; j += PM_STEP) pm[j] = __ldcg(st + (8 + j) * g.n_pad);
-                    if (PHASE) plast = __ldcg(st + kSegDoubles * g.n_pad);
-                    bad = __ldcg(g.bad + b);
-                }
-            }
-            if (run) {
-                const int i0 = seg * g.seg_steps;
-                const int i1 = last ? p.n_steps : i0 + g.seg_steps;
-                bad = fast_integrate<false, true, LOSS, true, PHASE, SYM>(p, b, db_run, p.coef, y, pm, i0, i1, bad,
-                                                                          &plast);
-                if (last) {
-                    if constexpr (SYM) {
-                        double yf[8];
-                        sym_expand(y, yf, pm);
-                        sweep_epilogue(p, x, b, yf, pm, bad, pm[2]);
-                    } else {
-                        sweep_epilogue(p, x, b, y, pm, bad, sweep_metric(x, pm, plast));
-                    }
-                }
-            }
-            if (!last) {
-                __stcg(st + 12 * g.n_pad, db_run);
-                if (run) {
-#pragma unroll
-                    for (int j = 0; j < NS; ++j) __stcg(st + j * g.n_pad, y[j]);
-#pragma unroll
-                    for (int j = 0; j < 4; j += PM_STEP) __stcg(st + (8 + j) * g.n_pad, pm[j]);
-                    if (PHASE) __stcg(st + kSegDoubles * g.n_pad, plast);
-                    __stcg(g.bad + b, bad);
-                }
-            }
-        }
-        if (!last) seg_publish(g, lane, seg, w);
-    }
+    seg_items(g, [&](int64_t b, int seg, bool last) { sweep_run_point<LOSS, X, SYM, true>(p, x, g, b, seg, last); });
 }
 
 // ------------------------------------------------------------------ exact path
@@ -935,7 +923,7 @@ static int resident_ctas(Kernel kernel, int threads) {
 // FPA_SWEEP_SEG=0 forces the whole-run kernels, =2 lifts the kSegMaxWaves cap, FPA_SWEEP_SEG_STEPS overrides the
 // segment length (tools, tests).
 static int seg_plan(int64_t B, int64_t n_steps, int ctas, int threads, void* scratch, int64_t scratch_bytes,
-                    cudaStream_t st, SegParams& g, bool& use_seg, int seg_doubles = kSegDoubles) {
+                    cudaStream_t st, SegParams& g, bool& use_seg, int seg_doubles) {
     const int64_t n_warps = (B + 31) / 32, resident_warps = (int64_t)ctas * (threads / 32);
     // segment length: 64 steps below two waves of the resident warps, else 128; half that for runs of fewer than
     // 1 000 steps, which would otherwise have too few segments to even out the tail (profiles/r2_seg_tune.txt:
@@ -964,32 +952,42 @@ static int seg_plan(int64_t B, int64_t n_steps, int ctas, int threads, void* scr
     return FPA_OK;
 }
 
+// Runs p.n_points points of a fast-path kernel family: its z-segment scheduler kernel (seg*, arguments (p, x..., g))
+// when seg_plan takes the batch, else its whole-run kernel (run*, arguments (p, x...)); the *_lossless kernels when
+// p.lossless.  resident_ctas and seg_plan see the scheduler kernel that would run; seg_doubles is its record size.
+template <typename SegK, typename RunK, typename... X>
+static int launch_fast_family(SegK seg, SegK seg_lossless, RunK run, RunK run_lossless, int seg_doubles,
+                              const char* what, const Yaman4Params& p, void* scratch, int64_t scratch_bytes,
+                              cudaStream_t st, const X&... x) {
+    const bool lossless = p.lossless != 0;
+    const SegK seg_kernel = lossless ? seg_lossless : seg;
+    const int  ctas = resident_ctas(seg_kernel, kFastThreads);
+    SegParams  g;
+    bool       use_seg = false;
+    int rc = seg_plan(p.n_points, p.n_steps, ctas, kFastThreads, scratch, scratch_bytes, st, g, use_seg, seg_doubles);
+    if (rc != FPA_OK) return rc;
+    if (use_seg) {
+        seg_kernel<<<ctas, kFastThreads, 0, st>>>(p, x..., g);
+    } else {
+        const long blocks = (long)((p.n_points + kFastThreads - 1) / kFastThreads);
+        (lossless ? run_lossless : run)<<<blocks, kFastThreads, 0, st>>>(p, x...);
+    }
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return cuda_fail(e, what);
+    return FPA_OK;
+}
+
+// Uniform physics: the family of UNIFORM = 1 (lossless: 2); per-point physics: the whole-run kernel of UNIFORM = 0.
 template <bool TRACE, bool PMAX>
 static int launch_fast(const Yaman4Params& p, bool uniform, void* scratch, int64_t scratch_bytes, cudaStream_t st) {
-    const int  threads = kFastThreads;
-    const long blocks  = (long)((p.n_points + threads - 1) / threads);
-    if (uniform) {  // the z-segment scheduler carries the uniform-physics instantiations
-        SegParams g;
-        bool      use_seg = false;
-        const int ctas = p.lossless ? resident_ctas(yaman4_fast_seg_kernel<TRACE, PMAX, 2, kFastThreads, kFastMinBlocks>, threads)
-                                    : resident_ctas(yaman4_fast_seg_kernel<TRACE, PMAX, 1, kFastThreads, kFastMinBlocks>, threads);
-        int       rc = seg_plan(p.n_points, p.n_steps, ctas, threads, scratch, scratch_bytes, st, g, use_seg);
-        if (rc != FPA_OK) return rc;
-        if (use_seg) {
-            if (p.lossless)
-                yaman4_fast_seg_kernel<TRACE, PMAX, 2, kFastThreads, kFastMinBlocks><<<ctas, threads, 0, st>>>(p, g);
-            else
-                yaman4_fast_seg_kernel<TRACE, PMAX, 1, kFastThreads, kFastMinBlocks><<<ctas, threads, 0, st>>>(p, g);
-            FPA_CUDA(cudaGetLastError());
-            return FPA_OK;
-        }
-    }
-    if (uniform && p.lossless)
-        yaman4_fast_kernel<TRACE, PMAX, 2, kFastThreads, kFastMinBlocks><<<blocks, threads, 0, st>>>(p);
-    else if (uniform)
-        yaman4_fast_kernel<TRACE, PMAX, 1, kFastThreads, kFastMinBlocks><<<blocks, threads, 0, st>>>(p);
-    else
-        yaman4_fast_kernel<TRACE, PMAX, 0, kFastThreads, kFastMinBlocks><<<blocks, threads, 0, st>>>(p);
+    if (uniform)
+        return launch_fast_family(yaman4_fast_seg_kernel<TRACE, PMAX, 1, kFastThreads, kFastMinBlocks>,
+                                  yaman4_fast_seg_kernel<TRACE, PMAX, 2, kFastThreads, kFastMinBlocks>,
+                                  yaman4_fast_kernel<TRACE, PMAX, 1, kFastThreads, kFastMinBlocks>,
+                                  yaman4_fast_kernel<TRACE, PMAX, 2, kFastThreads, kFastMinBlocks>, kSegDoubles,
+                                  "cudaGetLastError()", p, scratch, scratch_bytes, st);
+    const long blocks = (long)((p.n_points + kFastThreads - 1) / kFastThreads);
+    yaman4_fast_kernel<TRACE, PMAX, 0, kFastThreads, kFastMinBlocks><<<blocks, kFastThreads, 0, st>>>(p);
     FPA_CUDA(cudaGetLastError());
     return FPA_OK;
 }
@@ -1141,36 +1139,16 @@ static int sweep_setup(const fpa_sweep_desc* d, int64_t n_phases, Yaman4Params& 
     return FPA_OK;
 }
 
-// z-segment scheduler when the batch is a wave or more, else the whole-run kernel.  SYM: the symmetric kernels (their
-// own launch shape); resident_ctas and seg_plan see the kernel that will run.
+// SYM: the symmetric kernels, with their own launch shape.
 template <typename X, bool SYM = false>
 static int sweep_run(const Yaman4Params& p, const X& x, void* scratch, int64_t scratch_bytes, cudaStream_t st) {
-    constexpr bool PHASE = kPhase<X>;
-    constexpr int  MB = SYM ? kSweepSymMinBlocks : kSweepMinBlocks;
-    const int64_t B = p.n_points;
-    const bool    lossless = p.lossless != 0;
-    const int ctas = lossless ? resident_ctas(yaman4_sweep_seg_kernel<false, kFastThreads, MB, X, SYM>, kFastThreads)
-                              : resident_ctas(yaman4_sweep_seg_kernel<true, kFastThreads, MB, X, SYM>, kFastThreads);
-    SegParams g;
-    bool      use_seg = false;
-    int rc = seg_plan(B, p.n_steps, ctas, kFastThreads, scratch, scratch_bytes, st, g, use_seg,
-                      PHASE ? kSegDoublesPhase : kSegDoubles);
-    if (rc != FPA_OK) return rc;
-    if (use_seg) {
-        if (lossless)
-            yaman4_sweep_seg_kernel<false, kFastThreads, MB, X, SYM><<<ctas, kFastThreads, 0, st>>>(p, x, g);
-        else
-            yaman4_sweep_seg_kernel<true, kFastThreads, MB, X, SYM><<<ctas, kFastThreads, 0, st>>>(p, x, g);
-    } else {
-        const long blocks = (long)((B + kFastThreads - 1) / kFastThreads);
-        if (lossless)
-            yaman4_sweep_kernel<false, kFastThreads, MB, X, SYM><<<blocks, kFastThreads, 0, st>>>(p, x);
-        else
-            yaman4_sweep_kernel<true, kFastThreads, MB, X, SYM><<<blocks, kFastThreads, 0, st>>>(p, x);
-    }
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return cuda_fail(e, "yaman4_sweep_kernel launch");
-    return FPA_OK;
+    constexpr int MB = SYM ? kSweepSymMinBlocks : kSweepMinBlocks;
+    return launch_fast_family(yaman4_sweep_seg_kernel<true, kFastThreads, MB, X, SYM>,
+                              yaman4_sweep_seg_kernel<false, kFastThreads, MB, X, SYM>,
+                              yaman4_sweep_kernel<true, kFastThreads, MB, X, SYM>,
+                              yaman4_sweep_kernel<false, kFastThreads, MB, X, SYM>,
+                              kPhase<X> ? kSegDoublesPhase : kSegDoubles, "yaman4_sweep_kernel launch", p, scratch,
+                              scratch_bytes, st, x);
 }
 
 // A0 has A1 == A2 and A3 == A4 BIT FOR BIT (a value test would take -0.0 for 0.0, and the runs would then differ in
