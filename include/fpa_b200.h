@@ -28,7 +28,9 @@
  *   FPA_ERR_INVALID, error text "... must be 16-byte aligned"): yaman4 A0, A_trace,
  *   A_end, Pmax; sweep plan.omega, A_end, Pmax; phase sweep A0_table; Delta-beta
  *   table omega; N-wave A0, A_trace, A_end and `factored`.  (torch and cudaMalloc
- *   allocations are; a complex128 view at an odd element offset is not.)
+ *   allocations are; a complex128 view at an odd element offset is not.)  The transfer
+ *   kernels store jac one double at a time: its device pointer must be 8-byte aligned
+ *   ("jac must be 8-byte aligned"); their other arrays follow the rules above.
  *   host entries: any naturally aligned array (numpy's rule: 8 bytes for float64 and
  *   complex128).  A page-locked result array the kernel cannot store to directly
  *   is staged like pageable memory.
@@ -315,6 +317,38 @@ int64_t fpa_yaman4_phase_sweep_scratch_bytes(int64_t n_points);
 /* Device pointers, asynchronous on `stream`: the sweep kernel and the reduction kernel.  sweep.gain_lin
  * must be set.  `scratch` NULL: the whole-run kernel (same results). */
 int fpa_yaman4_phase_sweep_dev(const fpa_phase_sweep_desc* d, void* scratch, int64_t scratch_bytes, void* stream);
+
+/* ------------------------------------------------ small-signal transfer matrices (not in the reference)
+ * J = dA(L)/dA(z0): the exact derivative of the discrete RK4 map the fast integrator computes (not an
+ * approximation of the ODE's derivative; central finite differences of fpa_yaman4_rk4_batch_* converge to it).
+ * Each RK4 stage out = base + c*f(in) (yaman_model.py:10-52 weighted by c) is differentiated along a tangent t:
+ *   P_j' = 2(x_j x_j' + y_j y_j'),  S' = sum P_j',  G_j' = c*gamma*(2 S' - P_j')
+ *   U' = A3'A4 + A3A4',  V' = A1'A2 + A1A2',  W' = qU',  Z' = conj(q)V'
+ *   out_j' = base_j' + cn A_j' + i(G_j'A_j + G_jA_j') + i(conj(A_m)'{W|Z} + conj(A_m){W'|Z'})
+ * with the base run's phase factors q and the same RK4 combination.  The base state runs with the unchanged
+ * arithmetic: A_end, Pmax, status and gain_lin equal those of fpa_yaman4_rk4_batch_* / fpa_yaman4_sweep_* bit for
+ * bit.  One GPU thread per (point, column); uniform-grid whole-run kernels only.
+ *
+ * Batch: the descriptor of fpa_yaman4_rk4_batch_* with all its outputs but the trace; FPA_OUT_TRACE, z_grid and
+ * FPA_PHASE_EXACT give FPA_ERR_UNSUPPORTED; `scratch` is ignored.
+ * Sweep: the descriptor and units of fpa_yaman4_sweep_*; n_peers must be 0; FPA_PHASE_EXACT gives
+ * FPA_ERR_UNSUPPORTED.  gain_lin may be NULL, and only then may p_signal be 0: a zero seed gives the undepleted-pump
+ * linearisation.  The multi-device entry splits the flattened grid like fpa_yaman4_sweep_multi_host.
+ * A point that is not integrated (invalid plan point, non-finite dbeta) and, under FPA_CHECK_NAN, a point whose
+ * status is not FPA_POINT_OK get an all-NaN J.  J is dimensionless, the same in m and km units.
+ */
+typedef struct fpa_transfer_out {
+    uint32_t columns;   /* bit c (0..7) set: column d A(L) / d in_c, in_c = Re A_{c/2}(z0) (c even) or Im (c odd); != 0 */
+    uint32_t reserved;
+    double*  jac;       /* [B, 8, popcount(columns)]: row r = Re/Im of A_{r/2}(L), columns in ascending bit order */
+} fpa_transfer_out;
+
+int fpa_yaman4_transfer_batch_dev (const fpa_yaman4_desc* d, const fpa_transfer_out* t, void* stream);
+int fpa_yaman4_transfer_batch_host(const fpa_yaman4_desc* d, const fpa_transfer_out* t, int device);
+int fpa_yaman4_transfer_sweep_dev (const fpa_sweep_desc* d, const fpa_transfer_out* t, void* stream);
+int fpa_yaman4_transfer_sweep_host(const fpa_sweep_desc* d, const fpa_transfer_out* t, int device);
+int fpa_yaman4_transfer_sweep_multi_host(const fpa_sweep_desc* d, const fpa_transfer_out* t,
+                                         int n_devices, const int* devices);
 
 /* ------------------------------------------------ linear test RHS  y' = lambda*y
  * Lets the reference's own integrator tests (tests.py:146-226, y' = y on a real

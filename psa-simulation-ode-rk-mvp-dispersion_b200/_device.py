@@ -115,6 +115,100 @@ def yaman4_batch(dbeta, gamma, alpha, A0, *, z0=0.0, z_max, n_steps, save_every=
     return out
 
 
+def transfer_out(columns: int, n_points: int, pinned: bool = False):
+    """(TransferOut, jac [n_points, 8, nc]) for a column mask (bit c: d A(L) / d component c of A(z0))."""
+    columns = int(columns)
+    if columns <= 0 or columns >> 8:
+        raise ValueError(f"columns must be a non-zero mask of bits 0..7, got {columns:#x}")
+    nc = bin(columns).count("1")
+    jac = result_array((n_points, 8, nc), np.float64, pinned)
+    t = _lib.TransferOut()
+    t.columns, t.jac = columns, ptr(jac)
+    return t, jac
+
+
+def yaman4_transfer(dbeta, gamma, alpha, A0, columns, *, z0=0.0, z_max, n_steps, pmax=False, check_nan=True,
+                    device: Optional[int] = None, devices=None) -> dict:
+    """Transfer matrices of B points through `fpa_yaman4_transfer_batch_host`: jac [B,8,nc], A_end [B,4],
+    status [B] (and Pmax [B,4]).  `devices=[...]`: contiguous shares of the points, one host thread per device
+    (ctypes releases the GIL during each call, so the devices run at once); results identical to one device."""
+    dbeta = f64(dbeta).reshape(-1)
+    B = dbeta.size
+    gam, gs = _per_point(gamma, B, 1, "gamma")
+    alp, as_ = _per_point(alpha, B, 1, "alpha")
+    a0, a0s = _per_point(A0, B, 4, "A0", c128)
+    n_steps = int(n_steps)
+    if n_steps < 1:
+        raise ValueError("n_steps must be >= 1")
+    t, jac = transfer_out(columns, B)
+    out = {"jac": jac, "A_end": np.empty((B, 4), np.complex128), "status": np.empty(B, np.int32)}
+    if pmax:
+        out["Pmax"] = np.empty((B, 4))
+    devs = [(_lib.get_device() if device is None else int(device))] if not devices else [int(v) for v in devices]
+    nc = jac.shape[2]
+    L = _lib.lib()
+
+    def part(k):
+        lo, hi = (B * k) // len(devs), (B * (k + 1)) // len(devs)
+        if hi <= lo:
+            return _lib.OK, ""
+        d = _lib.Yaman4Desc()
+        d.n_points = hi - lo
+        d.dbeta = ptr(dbeta) + 8 * lo
+        d.gamma, d.gamma_stride = ptr(gam) + 8 * lo * gs, gs
+        d.alpha, d.alpha_stride = ptr(alp) + 8 * lo * as_, as_
+        d.A0, d.A0_stride = ptr(a0) + 16 * 4 * lo * a0s, a0s
+        d.z0, d.z_max, d.n_steps, d.save_every = float(z0), float(z_max), n_steps, 1
+        d.flags = _flags(False, True, pmax, check_nan, False)
+        d.A_end = ptr(out["A_end"]) + 64 * lo
+        d.Pmax = ptr(out["Pmax"]) + 32 * lo if pmax else None
+        d.status = ptr(out["status"]) + 4 * lo
+        tp = _lib.TransferOut()
+        tp.columns, tp.jac = t.columns, ptr(jac) + 8 * 8 * nc * lo
+        rc = L.fpa_yaman4_transfer_batch_host(C.byref(d), C.byref(tp), devs[k])
+        return rc, (_lib.last_error() if rc != _lib.OK else "")
+
+    if len(devs) == 1:
+        _lib.check(part(0)[0])
+    else:
+        from concurrent.futures import ThreadPoolExecutor
+        with ThreadPoolExecutor(len(devs)) as ex:
+            res = list(ex.map(part, range(len(devs))))
+        for rc, msg in res:
+            if rc != _lib.OK:
+                raise {_lib.ERR_INVALID: ValueError, _lib.ERR_UNSUPPORTED: NotImplementedError}.get(rc, _lib.FpaError)(msg)
+    return out
+
+
+def transfer_sweep(desc, columns, *, device: Optional[int] = None, devices=None) -> dict:
+    """Run `fpa_yaman4_transfer_sweep_host` on a SweepDesc whose plan axes / physics are filled; gain_lin comes
+    back only when desc.p_signal > 0.  Returns jac [n1,n3,8,nc], A_end, dbeta, valid, status (and gain_lin)."""
+    n1, n3 = desc.plan.n1, desc.plan.n3
+    G = n1 * n3
+    big = G >= 4096
+    t, jac = transfer_out(columns, G, big)
+    out = {"jac": jac.reshape(n1, n3, 8, -1), "A_end": result_array((n1, n3, 4), np.complex128, big),
+           "dbeta": result_array((n1, n3), np.float64, big), "valid": result_array((n1, n3), np.int32, big),
+           "status": result_array((n1, n3), np.int32, big)}
+    if desc.p_signal > 0.0:
+        out["gain_lin"] = result_array((n1, n3), np.float64, big)
+    desc.plan.dbeta, desc.plan.valid, desc.plan.omega = ptr(out["dbeta"]), ptr(out["valid"]), None
+    desc.gain_lin, desc.status = ptr(out.get("gain_lin")), ptr(out["status"])
+    desc.Pmax, desc.A_end = None, ptr(out["A_end"])
+    if G == 0:
+        return out
+    L = _lib.lib()
+    if devices is not None and len(devices) > 1:
+        ids = (C.c_int * len(devices))(*[int(v) for v in devices])
+        _lib.check(L.fpa_yaman4_transfer_sweep_multi_host(C.byref(desc), C.byref(t), len(devices), ids))
+    else:
+        dev = _lib.get_device() if device is None else int(device)
+        if devices is not None and len(devices) == 1:
+            dev = int(devices[0])
+        _lib.check(L.fpa_yaman4_transfer_sweep_host(C.byref(desc), C.byref(t), dev))
+    return out
+
+
 def yaman4_rhs(z, A, gamma, alpha, dbeta, *, device: Optional[int] = None) -> np.ndarray:
     """dA[b,:] for B (z, A) pairs through `fpa_yaman4_rhs_host`."""
     A = c128(A).reshape(-1, 4)

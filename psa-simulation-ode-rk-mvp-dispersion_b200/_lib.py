@@ -91,6 +91,10 @@ class PhaseSweepDesc(C.Structure):
     ]
 
 
+class TransferOut(C.Structure):
+    _fields_ = [("columns", C.c_uint32), ("reserved", C.c_uint32), ("jac", C.c_void_p)]
+
+
 class Triplet(C.Structure):
     _fields_ = [("k", C.c_int16), ("l", C.c_int16), ("m", C.c_int16), ("weight", C.c_int16)]
 
@@ -141,6 +145,12 @@ SIGNATURES = {
     "fpa_yaman4_phase_sweep_multi_host": (C.c_int, [C.POINTER(PhaseSweepDesc), C.c_int, C.POINTER(C.c_int)]),
     "fpa_yaman4_phase_sweep_scratch_bytes": (C.c_int64, [C.c_int64]),
     "fpa_yaman4_phase_sweep_dev": (C.c_int, [C.POINTER(PhaseSweepDesc), C.c_void_p, C.c_int64, C.c_void_p]),
+    "fpa_yaman4_transfer_batch_dev": (C.c_int, [C.POINTER(Yaman4Desc), C.POINTER(TransferOut), C.c_void_p]),
+    "fpa_yaman4_transfer_batch_host": (C.c_int, [C.POINTER(Yaman4Desc), C.POINTER(TransferOut), C.c_int]),
+    "fpa_yaman4_transfer_sweep_dev": (C.c_int, [C.POINTER(SweepDesc), C.POINTER(TransferOut), C.c_void_p]),
+    "fpa_yaman4_transfer_sweep_host": (C.c_int, [C.POINTER(SweepDesc), C.POINTER(TransferOut), C.c_int]),
+    "fpa_yaman4_transfer_sweep_multi_host": (C.c_int, [C.POINTER(SweepDesc), C.POINTER(TransferOut), C.c_int,
+                                                       C.POINTER(C.c_int)]),
     "fpa_linear_rk4_batch_host": (C.c_int, [C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_double,
                                             C.c_double, C.c_int64, C.c_int64, C.c_void_p, C.c_uint32,
                                             C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),

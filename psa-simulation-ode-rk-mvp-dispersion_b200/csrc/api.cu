@@ -19,6 +19,9 @@ namespace fpa {
 // launchers and descriptor checks implemented next to their kernels
 int yaman4_check(const fpa_yaman4_desc* d);
 int yaman4_launch(const fpa_yaman4_desc* d, cudaStream_t st);
+int yaman4_transfer_check(const fpa_yaman4_desc* d, const fpa_transfer_out* t);
+int yaman4_transfer_launch(const fpa_yaman4_desc* d, const fpa_transfer_out* t, cudaStream_t st);
+int yaman4_transfer_sweep_launch(const fpa_sweep_desc* d, const fpa_transfer_out* t, cudaStream_t st);
 int yaman4_rhs_launch(int64_t B, const double* z, const double* A, const double* gamma,
                       const double* alpha, const double* dbeta, double* dA, cudaStream_t st);
 int plan_launch(const fpa_plan_desc* d, double* dbeta_masked, cudaStream_t st);
@@ -283,14 +286,17 @@ static int check_devices(int n_devices, const int* devices) {
 }
 
 // ----------------------------------------------------------------- 4-wave batch
-static int batch_host_launch(const fpa_yaman4_desc* d, int device, Pending* p) {
-    FPA_TRY(yaman4_check(d));
+// t != NULL: the transfer batch (jac staged like the other outputs, no scheduler scratch).
+static int batch_host_launch(const fpa_yaman4_desc* d, int device, Pending* p, const fpa_transfer_out* t) {
+    FPA_TRY(t ? yaman4_transfer_check(d, t) : yaman4_check(d));
     FPA_TRY(use_device(device));
     const size_t B = (size_t)d->n_points;
     if (B == 0) return FPA_OK;
-    const size_t    ns      = (size_t)fpa_n_saved(d->n_steps, d->save_every);
-    const size_t    n_sched = (size_t)yaman4_scratch_bytes((int64_t)B);
-    fpa_yaman4_desc dd;
+    const size_t     ns      = (size_t)fpa_n_saved(d->n_steps, d->save_every);
+    const size_t     n_sched = t ? 0 : (size_t)yaman4_scratch_bytes((int64_t)B);
+    const size_t     nc      = t ? (size_t)__builtin_popcount(t->columns) : 0;
+    fpa_yaman4_desc  dd;
+    fpa_transfer_out tt = {};
     // outputs in pinned host memory are written by the kernel itself (no staging, no copy)
     FPA_TRY(stage(device, 0, p, [&](Staging& s) {
         dd         = *d;
@@ -304,6 +310,10 @@ static int batch_host_launch(const fpa_yaman4_desc* d, int device, Pending* p) {
         dd.Pmax    = (d->flags & FPA_OUT_PMAX) ? s.out(d->Pmax, B * 4, true, kVecAlign) : nullptr;
         dd.status  = s.out(d->status, B, true);  // the kernel always gets one
         dd.scratch = s.tmp<char>(n_sched);
+        if (t) {
+            tt     = *t;
+            tt.jac = s.out(t->jac, B * 8 * nc, true);
+        }
     }));
     dd.scratch_bytes = (int64_t)n_sched;
     if (d->gamma_stride == 0 && d->alpha_stride == 0) {  // host pointers: the broadcast values are known here
@@ -313,7 +323,11 @@ static int batch_host_launch(const fpa_yaman4_desc* d, int device, Pending* p) {
     } else {
         dd.flags &= ~FPA_UNIFORM_PHYSICS;
     }
-    return yaman4_launch(&dd, p->st);
+    return t ? yaman4_transfer_launch(&dd, &tt, p->st) : yaman4_launch(&dd, p->st);
+}
+
+static int batch_host_launch(const fpa_yaman4_desc* d, int device, Pending* p) {
+    return batch_host_launch(d, device, p, nullptr);
 }
 
 // ----------------------------------------------------------------- sweeps
@@ -358,20 +372,35 @@ static void stage_sweep(Staging& s, const fpa_sweep_desc* d, fpa_sweep_desc& dd,
     dd.status       = s.out(d->status, P, true);
 }
 
-static int sweep_host_launch(const fpa_sweep_desc* d, int device, Pending* p) {
+// t != NULL: the transfer sweep (gain_lin may be NULL, jac staged like the other outputs, no scheduler scratch).
+static int sweep_host_launch(const fpa_sweep_desc* d, int device, Pending* p, const fpa_transfer_out* t) {
     FPA_REQUIRE(d != nullptr, "sweep descriptor is NULL");
+    FPA_REQUIRE(t == nullptr || t->columns != 0, "columns must be a non-zero mask of bits 0..7 (got 0)");
     int64_t G;
     FPA_TRY(sweep_host_points(d, device, &G));
     if (G == 0) return FPA_OK;
-    FPA_REQUIRE(d->gain_lin != nullptr, "gain_lin must be set");
-    const size_t   n_sched = (size_t)yaman4_scratch_bytes(G);
-    fpa_sweep_desc dd;
-    char*          sched;
+    FPA_REQUIRE(d->gain_lin != nullptr || t, "gain_lin must be set");
+    const size_t     n_sched = t ? 0 : (size_t)yaman4_scratch_bytes(G);
+    const size_t     nc      = t ? (size_t)__builtin_popcount(t->columns) : 0;
+    fpa_sweep_desc   dd;
+    fpa_transfer_out tt = {};
+    char*            sched;
     FPA_TRY(stage(device, 3, p, [&](Staging& s) {
         stage_sweep(s, d, dd, (size_t)G, (size_t)G, true);
         sched = s.tmp<char>(n_sched);
+        if (t) {
+            tt     = *t;
+            tt.jac = s.out(t->jac, (size_t)G * 8 * nc, true);
+        }
     }));
-    return yaman4_sweep_launch(&dd, sched, (int64_t)n_sched, p->st);
+    if (!t) return yaman4_sweep_launch(&dd, sched, (int64_t)n_sched, p->st);
+    if (d->gain_lin == nullptr) dd.gain_lin = nullptr;  // no gain map: the seed power may be 0
+    dd.n_peers = d->n_peers;                            // refused by the launcher when set
+    return yaman4_transfer_sweep_launch(&dd, &tt, p->st);
+}
+
+static int sweep_host_launch(const fpa_sweep_desc* d, int device, Pending* p) {
+    return sweep_host_launch(d, device, p, nullptr);
 }
 
 // K = n_phases runs per grid point: the per-run arrays hold G*K entries, the plan outputs and the reductions G.
@@ -668,6 +697,47 @@ int fpa_yaman4_sweep_multi_host(const fpa_sweep_desc* d, int n_devices, const in
         int64_t              lo;
         const fpa_sweep_desc part = sweep_part(d, n_devices, k, 1, &lo);
         return part.n_sub_points > 0 ? sweep_host_launch(&part, devices[k], p) : (int)FPA_OK;
+    });
+}
+
+// ------------------------------------------------------------------ small-signal transfer matrices
+int fpa_yaman4_transfer_batch_dev(const fpa_yaman4_desc* d, const fpa_transfer_out* t, void* stream) {
+    FPA_TRY(need_device());
+    return yaman4_transfer_launch(d, t, static_cast<cudaStream_t>(stream));
+}
+
+int fpa_yaman4_transfer_batch_host(const fpa_yaman4_desc* d, const fpa_transfer_out* t, int device) {
+    FPA_REQUIRE(t != nullptr, "transfer output is NULL");
+    Pending p;
+    FPA_TRY(batch_host_launch(d, device, &p, t));
+    return finish(p, device);
+}
+
+int fpa_yaman4_transfer_sweep_dev(const fpa_sweep_desc* d, const fpa_transfer_out* t, void* stream) {
+    FPA_TRY(need_device());
+    return yaman4_transfer_sweep_launch(d, t, static_cast<cudaStream_t>(stream));
+}
+
+int fpa_yaman4_transfer_sweep_host(const fpa_sweep_desc* d, const fpa_transfer_out* t, int device) {
+    FPA_REQUIRE(t != nullptr, "transfer output is NULL");
+    Pending p;
+    FPA_TRY(sweep_host_launch(d, device, &p, t));
+    return finish(p, device);
+}
+
+int fpa_yaman4_transfer_sweep_multi_host(const fpa_sweep_desc* d, const fpa_transfer_out* t, int n_devices,
+                                         const int* devices) {
+    FPA_REQUIRE(d != nullptr, "sweep descriptor is NULL");
+    FPA_REQUIRE(t != nullptr, "transfer output is NULL");
+    FPA_TRY(sweep_multi_check(d, n_devices, devices));
+    if (n_devices == 1) return fpa_yaman4_transfer_sweep_host(d, t, devices[0]);
+    const int64_t nc = __builtin_popcount(t->columns);
+    return run_on_devices(n_devices, devices, [&](int k, Pending* p) {
+        int64_t              lo;
+        const fpa_sweep_desc part = sweep_part(d, n_devices, k, 1, &lo);
+        fpa_transfer_out     tp   = *t;
+        if (tp.jac) tp.jac += lo * 8 * nc;
+        return part.n_sub_points > 0 ? sweep_host_launch(&part, devices[k], p, &tp) : (int)FPA_OK;
     });
 }
 

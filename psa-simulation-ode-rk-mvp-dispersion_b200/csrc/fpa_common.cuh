@@ -35,6 +35,11 @@ int  cuda_fail(cudaError_t e, const char* what);
     FPA_REQUIRE((reinterpret_cast<uintptr_t>(ptr) & 15) == 0, "%s must be 16-byte aligned (got %p)", \
                 name, (const void*)(ptr))
 
+// The same for the arrays the kernels store one double at a time (the transfer kernels' jac).
+#define FPA_REQUIRE_ALIGNED8(ptr, name)                                                          \
+    FPA_REQUIRE((reinterpret_cast<uintptr_t>(ptr) & 7) == 0, "%s must be 8-byte aligned (got %p)", \
+                name, (const void*)(ptr))
+
 // Selects `device` (must exist) -- there is no CPU fallback anywhere in this library.
 int use_device(int device);
 

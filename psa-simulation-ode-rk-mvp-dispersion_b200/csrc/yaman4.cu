@@ -178,6 +178,97 @@ __device__ __forceinline__ void stage_sym(const double (&in)[4], const double (&
     }
 }
 
+// Tangent of stage() along t (DESIGN.md §4.1d): tout = tbase + c*Df(in)*t, where in, (qr, qi) and the coefficients
+// are those of the base run's stage.  Term by term, with A_j = x_j + i y_j and A_j' = t_{2j} + i t_{2j+1}:
+//   P_j' = 2(x_j x_j' + y_j y_j'),  S' = sum_j P_j',  G_j' = c2g S' - cg P_j'
+//   U' = A3' A4 + A3 A4',  V' = A1' A2 + A1 A2',  W' = q U',  Z' = conj(q) V'
+//   out_j' = base_j' + cn A_j' + i (G_j' A_j + G_j A_j') + i (conj(A_m)' {W|Z} + conj(A_m) {W'|Z'})
+// The half powers h_j = x_j x_j' + y_j y_j' are formed and G_j' = fma(-2cg, h_j, 4cg hS), which is exactly
+// fma(-cg, P_j', c2g S') (the factors of 2 are exact).  G_j, W and Z are stage()'s expressions on the same operands
+// (the compiler shares them with the base stage).  Every product and sum is spelled out with fma, __dmul_rn and
+// __dadd_rn: nothing is left to contraction, so oracle/transfer_model.py reproduces it operation for operation.
+template <bool LOSS>
+__device__ __forceinline__ void tan_wave(double xj, double yj, double dxj, double dyj, double xm, double ym, double dxm,
+                                         double dym, double G, double dG, double Cr, double Ci, double dCr, double dCi,
+                                         double cn, double tbr, double tbi, double& outr, double& outi) {
+    double r = LOSS ? fma(cn, dxj, tbr) : tbr;
+    double i = LOSS ? fma(cn, dyj, tbi) : tbi;
+    r = fma(-G, dyj, fma(-dG, yj, fma(ym, dCr, fma(dym, Cr, fma(-xm, dCi, fma(-dxm, Ci, r))))));
+    i = fma(G, dxj, fma(dG, xj, fma(xm, dCr, fma(dxm, Cr, fma(ym, dCi, fma(dym, Ci, i))))));
+    outr = r;
+    outi = i;
+}
+
+template <bool LOSS>
+__device__ __forceinline__ void stage_tan(const double (&in)[8], const double (&t)[8], const double (&tbase)[8],
+                                          double qr, double qi, double cg, double c2g, double cn, double (&out)[8]) {
+    const double x1 = in[0], y1 = in[1], x2 = in[2], y2 = in[3];
+    const double x3 = in[4], y3 = in[5], x4 = in[6], y4 = in[7];
+    const double dx1 = t[0], dy1 = t[1], dx2 = t[2], dy2 = t[3];
+    const double dx3 = t[4], dy3 = t[5], dx4 = t[6], dy4 = t[7];
+    // the base stage's G_j, W, Z (stage())
+    const double P1 = fma(y1, y1, x1 * x1);
+    const double P2 = fma(y2, y2, x2 * x2);
+    const double P3 = fma(y3, y3, x3 * x3);
+    const double P4 = fma(y4, y4, x4 * x4);
+    const double S  = (P1 + P2) + (P3 + P4);
+    const double c2 = c2g * S;
+    const double G1 = fma(-cg, P1, c2), G2 = fma(-cg, P2, c2), G3 = fma(-cg, P3, c2), G4 = fma(-cg, P4, c2);
+    const double Ur = fma(-y3, y4, x3 * x4), Ui = fma(x3, y4, y3 * x4);
+    const double Vr = fma(-y1, y2, x1 * x2), Vi = fma(x1, y2, y1 * x2);
+    const double Wr = fma(-qi, Ui, qr * Ur), Wi = fma(qr, Ui, qi * Ur);
+    const double Zr = fma(qi, Vi, qr * Vr),  Zi = fma(qr, Vi, -(qi * Vr));
+    // the tangent
+    const double h1 = fma(y1, dy1, __dmul_rn(x1, dx1));
+    const double h2 = fma(y2, dy2, __dmul_rn(x2, dx2));
+    const double h3 = fma(y3, dy3, __dmul_rn(x3, dx3));
+    const double h4 = fma(y4, dy4, __dmul_rn(x4, dx4));
+    const double hS = __dadd_rn(__dadd_rn(h1, h2), __dadd_rn(h3, h4));
+    const double c4g = __dadd_rn(c2g, c2g);
+    const double d2  = __dmul_rn(c4g, hS);
+    const double dG1 = fma(-c2g, h1, d2), dG2 = fma(-c2g, h2, d2), dG3 = fma(-c2g, h3, d2), dG4 = fma(-c2g, h4, d2);
+    const double dUr = fma(x3, dx4, fma(-y3, dy4, fma(-dy3, y4, __dmul_rn(dx3, x4))));
+    const double dUi = fma(x3, dy4, fma(y3, dx4, fma(dy3, x4, __dmul_rn(dx3, y4))));
+    const double dVr = fma(x1, dx2, fma(-y1, dy2, fma(-dy1, y2, __dmul_rn(dx1, x2))));
+    const double dVi = fma(x1, dy2, fma(y1, dx2, fma(dy1, x2, __dmul_rn(dx1, y2))));
+    const double dWr = fma(-qi, dUi, __dmul_rn(qr, dUr)), dWi = fma(qr, dUi, __dmul_rn(qi, dUr));
+    const double dZr = fma(qi, dVi, __dmul_rn(qr, dVr)),  dZi = fma(qr, dVi, -__dmul_rn(qi, dVr));
+    tan_wave<LOSS>(x1, y1, dx1, dy1, x2, y2, dx2, dy2, G1, dG1, Wr, Wi, dWr, dWi, cn, tbase[0], tbase[1], out[0], out[1]);
+    tan_wave<LOSS>(x2, y2, dx2, dy2, x1, y1, dx1, dy1, G2, dG2, Wr, Wi, dWr, dWi, cn, tbase[2], tbase[3], out[2], out[3]);
+    tan_wave<LOSS>(x3, y3, dx3, dy3, x4, y4, dx4, dy4, G3, dG3, Zr, Zi, dZr, dZi, cn, tbase[4], tbase[5], out[4], out[5]);
+    tan_wave<LOSS>(x4, y4, dx4, dy4, x3, y3, dx3, dy3, G4, dG4, Zr, Zi, dZr, dZi, cn, tbase[6], tbase[7], out[6], out[7]);
+}
+
+// The z-loop hook of fast_integrate: NoTangent (every existing kernel) adds nothing; Tangent carries one tangent
+// column t through the run.  stage<s>(in, ...) is called after stage s of a step with that stage's input state and
+// coefficients and mirrors it on the tangent, including the RK4 combination with the same exact-sum weights.
+struct NoTangent {};
+
+template <bool LOSS>
+struct Tangent {
+    double t[8], ts[8], tt[8], ta[8];
+
+    template <int S>
+    __device__ __forceinline__ void stage(const double (&in)[8], double qr, double qi, double cg, double c2g, double cn) {
+        const double third = 1.0 / 3.0, two_thirds = 2.0 / 3.0, third_c = 1.0 - two_thirds;  // as fast_integrate
+        if constexpr (S == 0) {
+            stage_tan<LOSS>(in, t, t, qr, qi, cg, c2g, cn, ts);
+#pragma unroll
+            for (int j = 0; j < 8; ++j) ta[j] = fma(third, ts[j], __dmul_rn(t[j], -third));
+        } else if constexpr (S == 1) {
+            stage_tan<LOSS>(in, ts, t, qr, qi, cg, c2g, cn, tt);
+#pragma unroll
+            for (int j = 0; j < 8; ++j) ta[j] = fma(two_thirds, tt[j], ta[j]);
+        } else if constexpr (S == 2) {
+            stage_tan<LOSS>(in, tt, t, qr, qi, cg, c2g, cn, ts);
+#pragma unroll
+            for (int j = 0; j < 8; ++j) ta[j] = fma(third_c, ts[j], ta[j]);
+        } else {
+            stage_tan<LOSS>(in, ts, ta, qr, qi, cg, c2g, cn, t);
+        }
+    }
+};
+
 // One RK4 stage on the full state or (4 doubles) on the symmetric half of one.
 template <bool LOSS>
 __device__ __forceinline__ void rk_stage(const double (&in)[8], const double (&base)[8], double qr, double qi,
@@ -306,13 +397,17 @@ __device__ __forceinline__ int32_t write_results(const Yaman4Params& p, int64_t 
 // kept, pm[1] and pm[3] are left to the caller.
 template <bool SYM>
 constexpr int kStateLen = SYM ? 4 : 8;
-template <bool TRACE, bool PMAX, bool LOSS, bool SEG = false, bool LAST = false, bool SYM = false>
+// Tan: the tangent hook (NoTangent, or Tangent<LOSS> for the transfer kernels: full state, *tan advanced with y).
+template <bool TRACE, bool PMAX, bool LOSS, bool SEG = false, bool LAST = false, bool SYM = false,
+          typename Tan = NoTangent>
 __device__ __forceinline__ int32_t fast_integrate(const Yaman4Params& p, int64_t b, double dbeta,
                                                   const Yaman4Coef& cf, double (&y)[kStateLen<SYM>], double (&pm)[4],
                                                   int i0_in = 0, int i1_in = 0, int32_t bad_in = FPA_POINT_OK,
-                                                  double* plast = nullptr) {
+                                                  double* plast = nullptr, Tan* tan = nullptr) {
     constexpr int NS = kStateLen<SYM>;
+    constexpr bool TAN = !std::is_same<Tan, NoTangent>::value;
     static_assert(!SYM || !TRACE, "the symmetric path writes no trace");
+    static_assert(!TAN || !SYM, "tangent directions leave the symmetric subspace");
     const int i0 = SEG ? i0_in : 0;
     const int i1 = SEG ? i1_in : p.n_steps;
     double* tr = nullptr;
@@ -367,16 +462,20 @@ __device__ __forceinline__ int32_t fast_integrate(const Yaman4Params& p, int64_t
         }
 #pragma unroll
         for (int j = 0; j < NS; ++j) acc[j] = fma(third, ys[j], y[j] * (-third));
+        if constexpr (TAN) tan->template stage<0>(y, qr, qi, cf.cg[0], cf.c2g[0], cf.cn[0]);
         // stage 2: yt = y + (h/2) f(z+h/2, ys)
         rk_stage<LOSS>(ys, y, qhr, qhi, cf.cg[0], cf.c2g[0], cf.cn[0], yt, Sx);
 #pragma unroll
         for (int j = 0; j < NS; ++j) acc[j] = fma(two_thirds, yt[j], acc[j]);
+        if constexpr (TAN) tan->template stage<1>(ys, qhr, qhi, cf.cg[0], cf.c2g[0], cf.cn[0]);
         // stage 3: ys = y + h f(z+h/2, yt)
         rk_stage<LOSS>(yt, y, q2r, q2i, cf.cg[1], cf.c2g[1], cf.cn[1], ys, Sx);
 #pragma unroll
         for (int j = 0; j < NS; ++j) acc[j] = fma(third_c, ys[j], acc[j]);
+        if constexpr (TAN) tan->template stage<2>(yt, q2r, q2i, cf.cg[1], cf.c2g[1], cf.cn[1]);
         // stage 4: y' = acc + (h/6) f(z+h, ys)
         rk_stage<LOSS>(ys, acc, q6r, q6i, cf.cg[2], cf.c2g[2], cf.cn[2], y, Sx);
+        if constexpr (TAN) tan->template stage<3>(ys, q6r, q6i, cf.cg[2], cf.c2g[2], cf.cn[2]);
 
         qr = qfr;
         qi = qfi;
@@ -754,6 +853,88 @@ __global__ void __launch_bounds__(THREADS, MIN_BLOCKS)
     seg_items(g, [&](int64_t b, int seg, bool last) { sweep_run_point<LOSS, X, SYM, true>(p, x, g, b, seg, last); });
 }
 
+// ------------------------------------------------------------------ small-signal transfer matrices
+// J = dA(L)/dA(0) of the discrete map fast_integrate computes (DESIGN.md §4.1d).  One thread per (point, column):
+// every lane of a point runs the point's base trajectory with the unchanged stage() calls, so A_end, Pmax, status and
+// the gain are those of the batch / sweep kernels bit for bit, and carries one tangent column beside it.  Lane
+// k = t mod nc of point b = t / nc starts from the unit vector of component col[k] (2j: Re A_j(z0), 2j+1: Im) and
+// stores jac[b, r, k] for the 8 rows r.  Lane 0 writes the point's other outputs.  Whole-run kernels only.
+struct TransferParams {
+    double*  jac;   // [B, 8, nc]
+    int      nc;    // columns per point
+    uint32_t cols;  // 4 bits per slot: bits 4k..4k+3 = the state component of slot k
+};
+
+struct BatchPoints {};  // X of the batch transfer kernel: the points are fpa_yaman4_desc's
+
+// Lane t of a transfer launch.  X = BatchPoints (batch) or SweepExtra (fused sweep; gain_lin may be NULL).
+// UNIFORM as for fast_point: 0 = gamma / alpha per point (batch only), 1 = uniform, 2 = uniform and lossless.
+template <int UNIFORM, typename X>
+__device__ __forceinline__ void transfer_point(const Yaman4Params& p, const X& x, const TransferParams& tp, int64_t t) {
+    constexpr bool SWEEP = std::is_same<X, SweepExtra>::value;
+    constexpr bool LOSS  = UNIFORM != 2;
+    const int64_t  b = t / tp.nc;
+    if (b >= p.n_points) return;
+    const int  k    = (int)(t - b * tp.nc);
+    const bool lead = k == 0;
+    double     y[8], pm[4] = {0.0, 0.0, 0.0, 0.0}, dbeta;
+    bool       run;
+    if constexpr (SWEEP) {
+        run = sweep_prologue(x, b, dbeta, lead);
+        sweep_initial_state(x, 0, y);
+    } else {
+        load_state(p, b, y);
+        dbeta = p.dbeta[b];
+        run   = !nonfinite(dbeta);
+    }
+    Tangent<LOSS> tan;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) tan.t[j] = j == (int)((tp.cols >> (4 * k)) & 15u) ? 1.0 : 0.0;
+    bool ok = false;
+    if (run) {
+        int32_t bad;
+        if constexpr (UNIFORM != 0) {
+            bad = fast_integrate<false, true, LOSS>(p, b, dbeta, p.coef, y, pm, 0, 0, FPA_POINT_OK, nullptr, &tan);
+        } else {
+            const Yaman4Coef cf = make_coef(p.gamma[b * p.gamma_stride], p.alpha[b * p.alpha_stride], p.h);
+            bad = fast_integrate<false, true, LOSS>(p, b, dbeta, cf, y, pm, 0, 0, FPA_POINT_OK, nullptr, &tan);
+        }
+        // write_results' status rule, in every lane
+        bool nf = false;
+#pragma unroll
+        for (int j = 0; j < 8; ++j) nf |= nonfinite(y[j]);
+        ok = !(p.check && (bad != FPA_POINT_OK || nf));
+        if (lead) {
+            if constexpr (SWEEP) {
+                if (x.gain_lin) sweep_epilogue(p, x, b, y, pm, bad, pm[2]);
+                else write_results(p, b, y, pm, p.Pmax != nullptr, bad);
+            } else {
+                write_results(p, b, y, pm, p.Pmax != nullptr, bad);
+            }
+        }
+    } else if (lead) {
+        if constexpr (SWEEP) {
+            if (x.gain_lin) sweep_invalid(p, x, b);
+            else write_nan_outputs(p, b);
+        } else {
+            write_nan_outputs(p, b);
+        }
+    }
+    double* J = tp.jac + b * 8 * tp.nc + k;
+#pragma unroll
+    for (int r = 0; r < 8; ++r) J[r * tp.nc] = ok ? tan.t[r] : qnan();
+}
+
+// 128 threads, 2 resident blocks per SM: the lane holds two RK4 states (base and tangent, 4 x 8 doubles each) and
+// needs ~200 registers (DESIGN.md §4.1d).
+constexpr int kTransferThreads = 128, kTransferMinBlocks = 2;
+
+template <int UNIFORM, typename X>
+__global__ void __launch_bounds__(kTransferThreads, kTransferMinBlocks)
+    yaman4_transfer_kernel(const Yaman4Params p, const X x, const TransferParams tp) {
+    transfer_point<UNIFORM>(p, x, tp, (int64_t)blockIdx.x * blockDim.x + threadIdx.x);
+}
+
 // ------------------------------------------------------------------ exact path
 // dA/dz for one point.  (pr,pi) = 2*gamma*exp(i*dbeta*z); nha = -alpha/2.
 __device__ __forceinline__ void rhs4(const double (&y)[8], double pr, double pi, double gamma,
@@ -1008,6 +1189,33 @@ int yaman4_check(const fpa_yaman4_desc* d) {
     return FPA_OK;
 }
 
+// The kernel arguments of a checked batch descriptor (yaman4_launch, yaman4_transfer_launch).
+static void batch_params(const fpa_yaman4_desc* d, bool uniform, Yaman4Params& p) {
+    p.n_points     = d->n_points;
+    p.dbeta        = d->dbeta;
+    p.gamma        = d->gamma;
+    p.alpha        = d->alpha;
+    p.A0           = d->A0;
+    p.z_grid       = d->z_grid;
+    p.A_trace      = (d->flags & FPA_OUT_TRACE) ? d->A_trace : nullptr;
+    p.A_end        = (d->flags & FPA_OUT_END) ? d->A_end : nullptr;
+    p.Pmax         = (d->flags & FPA_OUT_PMAX) ? d->Pmax : nullptr;
+    p.status       = d->status;
+    p.z0           = d->z0;
+    p.z_max        = d->z_max;
+    p.h            = (d->z_max - d->z0) / (double)d->n_steps;
+    p.gamma_stride = (int)d->gamma_stride;
+    p.alpha_stride = (int)d->alpha_stride;
+    p.A0_stride    = (int)d->A0_stride;
+    p.n_steps      = (int)d->n_steps;
+    // save_every > n_steps never fires; clamp so the countdown fits an int
+    p.save_every   = (int)(d->save_every > d->n_steps ? d->n_steps + 1 : d->save_every);
+    p.check        = (d->flags & FPA_CHECK_NAN) ? 1 : 0;
+    p.n_saved      = fpa_n_saved(d->n_steps, d->save_every);
+    p.coef         = make_coef(uniform ? d->gamma_uniform : 0.0, uniform ? d->alpha_uniform : 0.0, p.h);
+    p.lossless     = (uniform && d->alpha_uniform == 0.0) ? 1 : 0;
+}
+
 int yaman4_launch(const fpa_yaman4_desc* d, cudaStream_t st) {
     int rc = yaman4_check(d);
     if (rc != FPA_OK) return rc;
@@ -1025,29 +1233,7 @@ int yaman4_launch(const fpa_yaman4_desc* d, cudaStream_t st) {
     if (d->n_points == 0) return FPA_OK;
 
     Yaman4Params p;
-    p.n_points     = d->n_points;
-    p.dbeta        = d->dbeta;
-    p.gamma        = d->gamma;
-    p.alpha        = d->alpha;
-    p.A0           = d->A0;
-    p.z_grid       = d->z_grid;
-    p.A_trace      = trace ? d->A_trace : nullptr;
-    p.A_end        = endo ? d->A_end : nullptr;
-    p.Pmax         = pmax ? d->Pmax : nullptr;
-    p.status       = d->status;
-    p.z0           = d->z0;
-    p.z_max        = d->z_max;
-    p.h            = (d->z_max - d->z0) / (double)d->n_steps;
-    p.gamma_stride = (int)d->gamma_stride;
-    p.alpha_stride = (int)d->alpha_stride;
-    p.A0_stride    = (int)d->A0_stride;
-    p.n_steps      = (int)d->n_steps;
-    // save_every > n_steps never fires; clamp so the countdown fits an int
-    p.save_every   = (int)(d->save_every > d->n_steps ? d->n_steps + 1 : d->save_every);
-    p.check        = (d->flags & FPA_CHECK_NAN) ? 1 : 0;
-    p.n_saved      = fpa_n_saved(d->n_steps, d->save_every);
-    p.coef         = make_coef(uniform ? d->gamma_uniform : 0.0, uniform ? d->alpha_uniform : 0.0, p.h);
-    p.lossless     = (uniform && d->alpha_uniform == 0.0) ? 1 : 0;
+    batch_params(d, uniform, p);
 
     const int    threads = 128;
     const long   blocks  = (long)((p.n_points + threads - 1) / threads);
@@ -1081,7 +1267,9 @@ int sweep_grid_points(const fpa_sweep_desc* d, int64_t* n_grid) {
 
 // Checks a sweep descriptor and fills the kernel arguments for its n_grid grid points (the whole grid or the
 // sub-range) x n_phases runs each; the plain sweep is n_phases = 1.
-static int sweep_setup(const fpa_sweep_desc* d, int64_t n_phases, Yaman4Params& p, SweepExtra& x, int64_t& n_grid) {
+// transfer: the transfer sweep, whose gain_lin may be NULL (and only then p_signal 0).
+static int sweep_setup(const fpa_sweep_desc* d, int64_t n_phases, Yaman4Params& p, SweepExtra& x, int64_t& n_grid,
+                       bool transfer = false) {
     FPA_REQUIRE(d != nullptr, "sweep descriptor is NULL");
     if (d->flags & FPA_PHASE_EXACT) {
         set_error("FPA_PHASE_EXACT is not available for the fused sweep: build the table with fpa_dbeta_table_* "
@@ -1093,12 +1281,13 @@ static int sweep_setup(const fpa_sweep_desc* d, int64_t n_phases, Yaman4Params& 
     rc = sweep_grid_points(d, &n_grid);
     if (rc != FPA_OK) return rc;
     const int64_t B = n_grid * n_phases;
-    FPA_REQUIRE(d->gain_lin != nullptr || B == 0, "gain_lin must be set");
+    FPA_REQUIRE(d->gain_lin != nullptr || B == 0 || transfer, "gain_lin must be set");
     FPA_REQUIRE(d->length_scale == 1.0 || d->length_scale == 1000.0, "length_scale must be 1 or 1000");
     FPA_REQUIRE(d->z_max > 0.0, "z_max must be positive");
     FPA_REQUIRE(d->dz > 0.0, "dz must be positive");
     FPA_REQUIRE(d->save_every >= 1, "save_every must be a positive integer");
-    FPA_REQUIRE(d->p_signal > 0.0, "p_in[2] (signal seed power) must be > 0 to define gain");
+    FPA_REQUIRE(d->p_signal > 0.0 || (transfer && d->gain_lin == nullptr),
+                "p_in[2] (signal seed power) must be > 0 to define gain");
     // sweep_prologue and sweep_epilogue store these with 16-byte vector stores
     FPA_REQUIRE_ALIGNED16(d->plan.omega, "plan.omega");
     FPA_REQUIRE_ALIGNED16(d->A_end, "A_end");
@@ -1194,6 +1383,89 @@ int yaman4_phase_sweep_launch(const fpa_phase_sweep_desc* d, void* scratch, int6
     x.n_phases   = K;
     x.last_saved = d->metric == FPA_GAIN_LAST_SAVED ? 1 : 0;
     return sweep_run(p, x, scratch, scratch_bytes, st);
+}
+
+// ---- small-signal transfer matrices
+// The column mask and jac of a transfer output (the kernels store jac with 8-byte stores).
+static int transfer_params(const fpa_transfer_out* t, TransferParams& tp) {
+    FPA_REQUIRE(t != nullptr, "transfer output is NULL");
+    FPA_REQUIRE(t->columns != 0 && (t->columns >> 8) == 0, "columns must be a non-zero mask of bits 0..7 (got %#x)",
+                t->columns);
+    FPA_REQUIRE(t->jac != nullptr, "jac must be set");
+    FPA_REQUIRE_ALIGNED8(t->jac, "jac");
+    tp.jac  = t->jac;
+    tp.nc   = 0;
+    tp.cols = 0;
+    for (uint32_t c = 0; c < 8; ++c) {
+        if ((t->columns >> c) & 1u) {
+            tp.cols |= c << (4 * tp.nc);
+            ++tp.nc;
+        }
+    }
+    return FPA_OK;
+}
+
+// The checks of a batch transfer, for the device and the host entries alike: the batch descriptor's, the transfer
+// output's, and the paths the tangent kernels do not cover (FPA_ERR_UNSUPPORTED).
+int yaman4_transfer_check(const fpa_yaman4_desc* d, const fpa_transfer_out* t) {
+    if (d && ((d->flags & (FPA_OUT_TRACE | FPA_PHASE_EXACT)) || d->z_grid)) {
+        set_error("transfer matrices follow the uniform-grid fast integrator: FPA_OUT_TRACE, z_grid and "
+                  "FPA_PHASE_EXACT are not available");
+        return FPA_ERR_UNSUPPORTED;
+    }
+    int rc = yaman4_check(d);
+    if (rc != FPA_OK) return rc;
+    TransferParams tp;
+    return transfer_params(t, tp);
+}
+
+int yaman4_transfer_launch(const fpa_yaman4_desc* d, const fpa_transfer_out* t, cudaStream_t st) {
+    int rc = yaman4_transfer_check(d, t);
+    if (rc != FPA_OK) return rc;
+    const bool uniform = (d->flags & FPA_UNIFORM_PHYSICS) != 0;
+    FPA_REQUIRE(!uniform || (d->gamma_stride == 0 && d->alpha_stride == 0),
+                "FPA_UNIFORM_PHYSICS needs broadcast gamma and alpha (stride 0)");
+    FPA_REQUIRE_ALIGNED16(d->A0, "A0");
+    if (d->flags & FPA_OUT_END) FPA_REQUIRE_ALIGNED16(d->A_end, "A_end");
+    if (d->flags & FPA_OUT_PMAX) FPA_REQUIRE_ALIGNED16(d->Pmax, "Pmax");
+    if (d->n_points == 0) return FPA_OK;
+    Yaman4Params   p;
+    TransferParams tp;
+    batch_params(d, uniform, p);
+    transfer_params(t, tp);
+    const BatchPoints x{};
+    const long        blocks = (long)((p.n_points * tp.nc + kTransferThreads - 1) / kTransferThreads);
+    if (!uniform)
+        yaman4_transfer_kernel<0><<<blocks, kTransferThreads, 0, st>>>(p, x, tp);
+    else if (p.lossless)
+        yaman4_transfer_kernel<2><<<blocks, kTransferThreads, 0, st>>>(p, x, tp);
+    else
+        yaman4_transfer_kernel<1><<<blocks, kTransferThreads, 0, st>>>(p, x, tp);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return cuda_fail(e, "yaman4_transfer_kernel launch");
+    return FPA_OK;
+}
+
+int yaman4_transfer_sweep_launch(const fpa_sweep_desc* d, const fpa_transfer_out* t, cudaStream_t st) {
+    Yaman4Params   p;
+    SweepExtra     x;
+    TransferParams tp;
+    int64_t        n_grid;
+    if (d && (d->flags & FPA_PHASE_EXACT)) return sweep_setup(d, 1, p, x, n_grid);  // FPA_ERR_UNSUPPORTED
+    FPA_REQUIRE(d != nullptr, "sweep descriptor is NULL");
+    FPA_REQUIRE(d->n_peers == 0, "the transfer sweep has no peer-store gather: n_peers must be 0");
+    int rc = transfer_params(t, tp);
+    if (rc != FPA_OK) return rc;
+    rc = sweep_setup(d, 1, p, x, n_grid, true);
+    if (rc != FPA_OK || n_grid == 0) return rc;
+    const long blocks = (long)((p.n_points * tp.nc + kTransferThreads - 1) / kTransferThreads);
+    if (p.lossless)
+        yaman4_transfer_kernel<2><<<blocks, kTransferThreads, 0, st>>>(p, x, tp);
+    else
+        yaman4_transfer_kernel<1><<<blocks, kTransferThreads, 0, st>>>(p, x, tp);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return cuda_fail(e, "yaman4_transfer_kernel launch");
+    return FPA_OK;
 }
 
 int yaman4_rhs_launch(int64_t B, const double* z, const double* A, const double* gamma,

@@ -31,7 +31,7 @@ from .dispersion import DispersionParams
 from .parameters import FiberParams, SimulationGrid
 from .phase_matching import PhaseMatchingConfig, PhaseMatchingMethod, fill_plan_desc
 from .simulation import (_default_phase_matching_cfg, _length_scale_to_m, make_initial_amplitudes,
-                         run_batch_simulation)
+                         run_batch_simulation, waves_to_columns)
 
 GainMode = Literal["end", "max"]
 
@@ -57,13 +57,13 @@ def _signal_axis(lambda_signal_m) -> np.ndarray:
     return lam3
 
 
-def _powers_and_phases(p_in, phase_in):
+def _powers_and_phases(p_in, phase_in, need_seed=True):
     p0 = np.asarray(list(p_in), dtype=float)
     if p0.shape != (4,):
         raise ValueError(f"p_in must have shape (4,), got {p0.shape}")
     if not np.all(np.isfinite(p0)) or np.any(p0 < 0.0):
         raise ValueError("p_in must contain finite non-negative powers")
-    if p0[2] <= 0.0:
+    if need_seed and p0[2] <= 0.0:
         raise ValueError("p_in[2] (signal seed power) must be > 0 to define gain")
     ph0 = None
     if phase_in is not None:
@@ -165,6 +165,62 @@ def sweep_gain_2d(*, cfg: SimulationConfig, lambda_p1_m, lambda_p2_m, lambda_sig
     g = out["gain_lin"]
     with np.errstate(invalid="ignore", divide="ignore"):
         out["gain"] = g if unit == "linear" else 10.0 * np.log10(g)
+    out["n_steps"] = int(round(float(cfg.z_max) * s / (float(cfg.dz) * s)))
+    return out
+
+
+def sweep_transfer_2d(*, cfg: SimulationConfig, lambda_p1_m, lambda_p2_m, lambda_signal_m, gamma: float,
+                      alpha: float, p_in, phase_in=None, waves=(2, 3), dispersion: Optional[DispersionParams] = None,
+                      phase_matching_cfg: Optional[PhaseMatchingConfig] = None, length_unit: str = "m",
+                      device: Optional[int] = None, devices=None) -> dict:
+    """Small-signal transfer matrices on the grid of `sweep_gain_2d`: per grid point J = dA(L)/dA(0), the exact
+    derivative of the RK4 map the sweep integrates, around the run that starts from (p_in, phase_in).
+
+    Returns dict(jac [n1,n3,8,nc], columns, A_end [n1,n3,4], dbeta, valid, status, n_steps) and, when p_in[2] > 0,
+    gain_lin [n1,n3] -- bit for bit `sweep_gain_2d`'s.  Rows / columns of jac as in
+    `simulation.run_batch_transfer`; `waves` selects whole input waves.  Zero seeds are allowed (p_in[2] = 0 gives
+    the undepleted-pump linearisation); every other argument error is raised as in `sweep_gain_2d`.  Invalid plan
+    points and runs that fail under cfg.check_nan get an all-NaN J.  The small_signal module turns J into gains."""
+    lam3 = _signal_axis(lambda_signal_m)
+    lam1 = np.atleast_1d(np.asarray(lambda_p1_m, dtype=float))
+    lam2 = np.atleast_1d(np.asarray(lambda_p2_m, dtype=float))
+    p0, ph0 = _powers_and_phases(p_in, phase_in, need_seed=False)
+    mask = waves_to_columns(waves)
+    columns = tuple(c for c in range(8) if mask >> c & 1)
+
+    pm_cfg = phase_matching_cfg
+    if pm_cfg is None:
+        try:
+            pm_cfg = _default_phase_matching_cfg(dispersion=dispersion, beta_legacy=None)
+        except ValueError:
+            pm_cfg = None
+    n1, n3 = lam1.size, lam3.size
+    if pm_cfg is None or not _run_constants_ok(cfg, gamma, alpha, dispersion, pm_cfg, length_unit):
+        # every run would raise -> all NaN, as in sweep_gain_2d
+        nan = np.full((n1, n3), np.nan)
+        out = {"jac": np.full((n1, n3, 8, len(columns)), np.nan), "A_end": np.full((n1, n3, 4), np.nan + 0j),
+               "dbeta": nan, "valid": np.zeros((n1, n3), np.int32), "status": np.full((n1, n3), -1, np.int32),
+               "columns": columns, "n_steps": 0}
+        if p0[2] > 0.0:
+            out["gain_lin"] = nan.copy()
+        return out
+
+    s = _length_scale_to_m(length_unit)
+    d = _lib.SweepDesc()
+    plan, keep = _device.new_plan_desc(lam1, lam2, lam3)
+    fill_plan_desc(plan, dispersion, pm_cfg)
+    d.plan = plan
+    A0 = make_initial_amplitudes(p0, ph0)
+    for j in range(4):
+        d.A0[2 * j], d.A0[2 * j + 1] = A0[j].real, A0[j].imag
+    d.p_signal = float(p0[2])
+    d.gamma, d.alpha = float(gamma), float(alpha)
+    d.z_max, d.dz = float(cfg.z_max), float(cfg.dz)
+    d.length_scale = s
+    d.save_every = int(cfg.save_every)
+    d.flags = _lib.CHECK_NAN if cfg.check_nan else 0
+    out = _device.transfer_sweep(d, mask, device=device, devices=devices)
+    out["columns"] = columns
     out["n_steps"] = int(round(float(cfg.z_max) * s / (float(cfg.dz) * s)))
     return out
 

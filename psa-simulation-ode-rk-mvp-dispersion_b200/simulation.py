@@ -185,6 +185,43 @@ def run_batch_simulation(cfg: SimulationConfig, *, gamma, alpha, delta_beta, p_i
     return r
 
 
+def waves_to_columns(waves) -> int:
+    """Column mask of the transfer kernels for whole waves: wave w -> columns 2w (Re A_w(0)) and 2w+1 (Im)."""
+    mask = 0
+    for w in np.atleast_1d(np.asarray(waves, dtype=int)).tolist():
+        if not 0 <= w < 4:
+            raise ValueError(f"waves must be indices in 0..3, got {w}")
+        mask |= 3 << (2 * w)
+    if mask == 0:
+        raise ValueError("waves must name at least one wave")
+    return mask
+
+
+def run_batch_transfer(cfg: SimulationConfig, *, gamma, alpha, delta_beta, p_in=None, phase_in=None, A0=None,
+                       waves=(2, 3), length_unit: str = "m", device: Optional[int] = None, devices=None) -> dict:
+    """Small-signal transfer matrices of B runs (arguments as `run_batch_simulation`): J = dA(L)/dA(0), the exact
+    derivative of the RK4 map the batch integrator computes, one tangent column per real input component.
+
+    Returns dict(jac [B,8,nc], columns, A_end [B,4], status [B], n_steps).  Row r of jac is Re (r even) or Im
+    (r odd) of A_{r//2}(L); column k is the derivative with respect to input component columns[k] (2w: Re A_w(0),
+    2w+1: Im A_w(0)); `waves` selects whole waves (both quadratures).  J is dimensionless, the same in m and km.
+    A run that fails under cfg.check_nan, or whose dbeta is not finite, gets an all-NaN J."""
+    validate_config(cfg)
+    s = _length_scale_to_m(length_unit)
+    if A0 is None:
+        A0 = make_initial_amplitudes(p_in, phase_in)
+    mask = waves_to_columns(waves)
+    db = np.asarray(delta_beta, dtype=float).reshape(-1) / s
+    z_max, dz = float(cfg.z_max) * s, float(cfg.dz) * s
+    n_steps = int(round(z_max / dz))
+    r = _device.yaman4_transfer(db, np.asarray(gamma, dtype=float) / s, np.asarray(alpha, dtype=float) / s, A0,
+                                mask, z_max=z_max, n_steps=n_steps, check_nan=cfg.check_nan, device=device,
+                                devices=devices)
+    r["columns"] = tuple(c for c in range(8) if mask >> c & 1)
+    r["n_steps"] = n_steps
+    return r
+
+
 def example_zero_signal() -> tuple[np.ndarray, np.ndarray]:
     """Two 0.5 W pumps, no signal/idler, dbeta = 0 PROVIDED, km units (simulation.py:371-405)."""
     w0 = 2.0 * np.pi * constants.c / 1.55e-6
