@@ -33,8 +33,10 @@
 //    operation of stage() on wave 2 (4) is the one on wave 1 (3) with the same operands, so the state stays
 //    on that subspace for the whole fiber.  stage_sym() / fast_integrate<..., SYM> then integrate the
 //    4-double state (x1, y1, x3, y3) with the same expressions in the same operand order: 186 instead of
-//    298 FP64 instructions per lossy step and the same bits (DESIGN.md §4.1c).  The launcher decides by a
-//    memcmp of A0's bit patterns; FPA_SWEEP_SYM=0 forces the 4-wave kernels.
+//    298 FP64 instructions per lossy step and the same bits (DESIGN.md §4.1c).  The symmetric kernels run
+//    stage_sym_fast() (178 per step: exact identities that hold while |A1|^2 + |A3|^2 < 2^1023) and replay a
+//    run or segment that left that range with stage_sym().  The launcher decides by a memcmp of A0's bit
+//    patterns; FPA_SWEEP_SYM=0 forces the 4-wave kernels.
 //    Each family -- the batch (yaman4_fast_kernel) and the fused sweep (yaman4_sweep_kernel) -- has one per-point
 //    body, fast_point / sweep_run_point.  Its whole-run kernel runs it once, for the single segment [0, n_steps); its
 //    z-segment scheduler kernel (yaman4_fast_seg_kernel / yaman4_sweep_seg_kernel) runs it once per work item through
@@ -165,6 +167,52 @@ __device__ __forceinline__ void stage_sym(const double (&in)[4], const double (&
     const double Vr = fma(-y1, y1, x1 * x1), Vi = fma(x1, y1, y1 * x1);  // A1*A2
     const double Wr = fma(-qi, Ui, qr * Ur), Wi = fma(qr, Ui, qi * Ur);
     const double Zr = fma(qi, Vi, qr * Vr),  Zi = fma(qr, Vi, -(qi * Vr));
+    if (LOSS) {
+        out[0] = fma(-G1, y1, fma(y1, Wr, fma(-x1, Wi, fma(cn, x1, base[0]))));
+        out[1] = fma(G1, x1, fma(x1, Wr, fma(y1, Wi, fma(cn, y1, base[1]))));
+        out[2] = fma(-G3, y3, fma(y3, Zr, fma(-x3, Zi, fma(cn, x3, base[2]))));
+        out[3] = fma(G3, x3, fma(x3, Zr, fma(y3, Zi, fma(cn, y3, base[3]))));
+    } else {
+        out[0] = fma(-G1, y1, fma(y1, Wr, fma(-x1, Wi, base[0])));
+        out[1] = fma(G1, x1, fma(x1, Wr, fma(y1, Wi, base[1])));
+        out[2] = fma(-G3, y3, fma(y3, Zr, fma(-x3, Zi, base[2])));
+        out[3] = fma(G3, x3, fma(x3, Zr, fma(y3, Zi, base[3])));
+    }
+}
+
+// stage_sym() with fewer FP64 instructions, the same bits whenever T = P1 + P3 < 2^1023 (DESIGN.md §4.1c):
+//  * S = (P1 + P1) + (P3 + P3) is exactly 2T (doublings are exact, scaling by 2 commutes with rounding), so
+//    c2g * S and c4g * T = (2 c2g) * T are products of the same real numbers: 2 adds fewer.
+//  * DBL (stage 2, whose doubled phase (q2r, q2i) = 2 (qr, qi) the z-loop forms anyway for stage 3): with m = y x,
+//    fma(x, y, m) is exactly 2m (m's rounding error is below half the spacing at 2m; a subnormal tie rounds to the
+//    even 2m), so fma(-qi, Ui, .) == fma(-q2i, m3, .) and the same for Wi, Zr, Zi: Ui and Vi are not formed.
+// Both fail only when a doubling overflows, which needs T >= 2^1023.  The high word of T (>= +0 or NaN) is folded
+// into `guard` by an unsigned max: guard >= 0x7FE00000 flags T >= 2^1023, inf or NaN, and the caller then replays
+// the run with stage_sym().
+template <bool LOSS, bool DBL>
+__device__ __forceinline__ void stage_sym_fast(const double (&in)[4], const double (&base)[4], double qr, double qi,
+                                               double q2r, double q2i, double cg, double c4g, double cn,
+                                               double (&out)[4], unsigned& guard) {
+    const double x1 = in[0], y1 = in[1], x3 = in[2], y3 = in[3];
+    const double P1 = fma(y1, y1, x1 * x1);
+    const double P3 = fma(y3, y3, x3 * x3);
+    const double T  = P1 + P3;
+    const unsigned hiT = (unsigned)__double2hiint(T);
+    guard = hiT > guard ? hiT : guard;
+    const double c2 = c4g * T;
+    const double G1 = fma(-cg, P1, c2);
+    const double G3 = fma(-cg, P3, c2);
+    const double Ur = fma(-y3, y3, x3 * x3), m3 = y3 * x3;
+    const double Vr = fma(-y1, y1, x1 * x1), m1 = y1 * x1;
+    double Wr, Wi, Zr, Zi;
+    if (DBL) {
+        Wr = fma(-q2i, m3, qr * Ur), Wi = fma(q2r, m3, qi * Ur);
+        Zr = fma(q2i, m1, qr * Vr),  Zi = fma(q2r, m1, -(qi * Vr));
+    } else {
+        const double Ui = fma(x3, y3, m3), Vi = fma(x1, y1, m1);
+        Wr = fma(-qi, Ui, qr * Ur), Wi = fma(qr, Ui, qi * Ur);
+        Zr = fma(qi, Vi, qr * Vr),  Zi = fma(qr, Vi, -(qi * Vr));
+    }
     if (LOSS) {
         out[0] = fma(-G1, y1, fma(y1, Wr, fma(-x1, Wi, fma(cn, x1, base[0]))));
         out[1] = fma(G1, x1, fma(x1, Wr, fma(y1, Wi, fma(cn, y1, base[1]))));
@@ -395,10 +443,22 @@ __device__ __forceinline__ int32_t write_results(const Yaman4Params& p, int64_t 
 // it, so a segmented run is bit-identical to a whole one.  LAST: *plast follows the last saved sample (save_sample).
 // SYM: y is the symmetric half (x1, y1, x3, y3) of a state with A1 == A2, A3 == A4 (stage_sym); pm[0] and pm[2] are
 // kept, pm[1] and pm[3] are left to the caller.
+// GUARD (SYM only): the stages are stage_sym_fast(), and no step runs the finite check.  Returns kSymReplay when a
+// stage's guard tripped (some T >= 2^1023, inf or NaN: the only states where stage_sym_fast() may differ from
+// stage_sym(), and the only ones where the finite check could have fired); the caller then replays the range with
+// GUARD = false.  Otherwise the results are those of GUARD = false, and `bad` is returned as given.
 template <bool SYM>
 constexpr int kStateLen = SYM ? 4 : 8;
+constexpr int32_t kSymReplay = -2;
+// (double)i, the same bits, through an asm statement: the compiler then cannot keep a floating-point copy of the loop
+// counter (one DADD per step) for the re-sync block, which needs it every kResync steps only.
+__device__ __forceinline__ double int_to_double_opaque(int i) {
+    double d;
+    asm("cvt.rn.f64.s32 %0, %1;" : "=d"(d) : "r"(i));
+    return d;
+}
 // Tan: the tangent hook (NoTangent, or Tangent<LOSS> for the transfer kernels: full state, *tan advanced with y).
-template <bool TRACE, bool PMAX, bool LOSS, bool SEG = false, bool LAST = false, bool SYM = false,
+template <bool TRACE, bool PMAX, bool LOSS, bool SEG = false, bool LAST = false, bool SYM = false, bool GUARD = false,
           typename Tan = NoTangent>
 __device__ __forceinline__ int32_t fast_integrate(const Yaman4Params& p, int64_t b, double dbeta,
                                                   const Yaman4Coef& cf, double (&y)[kStateLen<SYM>], double (&pm)[4],
@@ -408,6 +468,7 @@ __device__ __forceinline__ int32_t fast_integrate(const Yaman4Params& p, int64_t
     constexpr bool TAN = !std::is_same<Tan, NoTangent>::value;
     static_assert(!SYM || !TRACE, "the symmetric path writes no trace");
     static_assert(!TAN || !SYM, "tangent directions leave the symmetric subspace");
+    static_assert(!GUARD || SYM, "the guarded stages are those of the symmetric path");
     const int i0 = SEG ? i0_in : 0;
     const int i1 = SEG ? i1_in : p.n_steps;
     double* tr = nullptr;
@@ -435,11 +496,15 @@ __device__ __forceinline__ int32_t fast_integrate(const Yaman4Params& p, int64_t
     // ys2 weights cancel exactly (same constant); 1 - fl(2/3) is exactly representable, so the ys4 weight
     // third_c = 1 - fl(2/3) makes two_thirds + third_c == 1 with no rounding.
     const double third = 1.0 / 3.0, two_thirds = 2.0 / 3.0, third_c = 1.0 - two_thirds;
+    unsigned     guard = 0;
+    // 4*c*gamma of stage_sym_fast(), in registers: a field of Yaman4Coef would grow the parameter block, and with it
+    // the machine code of every kernel.  It is finite: sweep_symmetric() sends any other sweep to the 4-wave kernels.
+    const double c4g[3] = {cf.c2g[0] + cf.c2g[0], cf.c2g[1] + cf.c2g[1], cf.c2g[2] + cf.c2g[2]};
 
     for (int i = i0; i < i1; ++i) {
         if ((i & (kResync - 1)) == 0) {
             double s, c;
-            sincos(dbeta * fma((double)i, h, z0), &s, &c);
+            sincos(dbeta * fma(GUARD ? int_to_double_opaque(i) : (double)i, h, z0), &s, &c);
             qr = cf.q0 * c;
             qi = cf.q0 * s;
         }
@@ -451,30 +516,43 @@ __device__ __forceinline__ int32_t fast_integrate(const Yaman4Params& p, int64_t
 
         double ys[NS], yt[NS], acc[NS], S, Sx;
         // stage 1: ys = y + (h/2) f(z, y)
-        rk_stage<LOSS>(y, y, qr, qi, cf.cg[0], cf.c2g[0], cf.cn[0], ys, S);
-        // S = sum |A|^2 of the state that step i-1 produced: a non-finite component makes S
-        // non-finite, so the exact per-component test runs only then (integrators.py:132-135).
-        if (nonfinite(S) && bad == FPA_POINT_OK && i > 0) {
-            bool nf = false;
+        if constexpr (GUARD) {
+            stage_sym_fast<LOSS, false>(y, y, qr, qi, q2r, q2i, cf.cg[0], c4g[0], cf.cn[0], ys, guard);
+        } else {
+            rk_stage<LOSS>(y, y, qr, qi, cf.cg[0], cf.c2g[0], cf.cn[0], ys, S);
+            // S = sum |A|^2 of the state that step i-1 produced: a non-finite component makes S
+            // non-finite, so the exact per-component test runs only then (integrators.py:132-135).
+            if (nonfinite(S) && bad == FPA_POINT_OK && i > 0) {
+                bool nf = false;
 #pragma unroll
-            for (int j = 0; j < NS; ++j) nf |= nonfinite(y[j]);
-            if (nf) bad = i - 1;
+                for (int j = 0; j < NS; ++j) nf |= nonfinite(y[j]);
+                if (nf) bad = i - 1;
+            }
         }
 #pragma unroll
         for (int j = 0; j < NS; ++j) acc[j] = fma(third, ys[j], y[j] * (-third));
         if constexpr (TAN) tan->template stage<0>(y, qr, qi, cf.cg[0], cf.c2g[0], cf.cn[0]);
         // stage 2: yt = y + (h/2) f(z+h/2, ys)
-        rk_stage<LOSS>(ys, y, qhr, qhi, cf.cg[0], cf.c2g[0], cf.cn[0], yt, Sx);
+        if constexpr (GUARD)
+            stage_sym_fast<LOSS, true>(ys, y, qhr, qhi, q2r, q2i, cf.cg[0], c4g[0], cf.cn[0], yt, guard);
+        else
+            rk_stage<LOSS>(ys, y, qhr, qhi, cf.cg[0], cf.c2g[0], cf.cn[0], yt, Sx);
 #pragma unroll
         for (int j = 0; j < NS; ++j) acc[j] = fma(two_thirds, yt[j], acc[j]);
         if constexpr (TAN) tan->template stage<1>(ys, qhr, qhi, cf.cg[0], cf.c2g[0], cf.cn[0]);
         // stage 3: ys = y + h f(z+h/2, yt)
-        rk_stage<LOSS>(yt, y, q2r, q2i, cf.cg[1], cf.c2g[1], cf.cn[1], ys, Sx);
+        if constexpr (GUARD)
+            stage_sym_fast<LOSS, false>(yt, y, q2r, q2i, q2r, q2i, cf.cg[1], c4g[1], cf.cn[1], ys, guard);
+        else
+            rk_stage<LOSS>(yt, y, q2r, q2i, cf.cg[1], cf.c2g[1], cf.cn[1], ys, Sx);
 #pragma unroll
         for (int j = 0; j < NS; ++j) acc[j] = fma(third_c, ys[j], acc[j]);
         if constexpr (TAN) tan->template stage<2>(yt, q2r, q2i, cf.cg[1], cf.c2g[1], cf.cn[1]);
         // stage 4: y' = acc + (h/6) f(z+h, ys)
-        rk_stage<LOSS>(ys, acc, q6r, q6i, cf.cg[2], cf.c2g[2], cf.cn[2], y, Sx);
+        if constexpr (GUARD)
+            stage_sym_fast<LOSS, false>(ys, acc, q6r, q6i, q2r, q2i, cf.cg[2], c4g[2], cf.cn[2], y, guard);
+        else
+            rk_stage<LOSS>(ys, acc, q6r, q6i, cf.cg[2], cf.c2g[2], cf.cn[2], y, Sx);
         if constexpr (TAN) tan->template stage<3>(ys, q6r, q6i, cf.cg[2], cf.c2g[2], cf.cn[2]);
 
         qr = qfr;
@@ -485,6 +563,7 @@ __device__ __forceinline__ int32_t fast_integrate(const Yaman4Params& p, int64_t
             save_sample<LAST>(y, tr, pm, TRACE, PMAX, plast);
         }
     }
+    if (GUARD && guard >= 0x7FE00000u) return kSymReplay;
     return bad;
 }
 
@@ -824,7 +903,21 @@ __device__ __forceinline__ void sweep_run_point(const Yaman4Params& p, const X& 
     if (run) {
         const int i0 = seg * g.seg_steps;
         const int i1 = last ? p.n_steps : i0 + g.seg_steps;
-        bad = fast_integrate<false, true, LOSS, SEG, PHASE, SYM>(p, b, db_run, p.coef, y, pm, i0, i1, bad, &plast);
+        if constexpr (SYM) {
+            // The guarded loop; a range where it tripped runs again from its start (A0, or the record, which is only
+            // overwritten after the range) with stage_sym(), and the outputs are the replay's.
+            bad = fast_integrate<false, true, LOSS, SEG, false, true, true>(p, b, db_run, p.coef, y, pm, i0, i1, bad);
+            if (bad == kSymReplay) {
+                bad = FPA_POINT_OK;
+                if (seg == 0)
+                    sweep_initial_state(x, 0, y);
+                else
+                    rec.load<true, false>(y, pm, plast, bad);
+                bad = fast_integrate<false, true, LOSS, SEG, false, true>(p, b, db_run, p.coef, y, pm, i0, i1, bad);
+            }
+        } else {
+            bad = fast_integrate<false, true, LOSS, SEG, PHASE>(p, b, db_run, p.coef, y, pm, i0, i1, bad, &plast);
+        }
         if (last) {
             if constexpr (SYM) {
                 double yf[8];
@@ -1341,10 +1434,13 @@ static int sweep_run(const Yaman4Params& p, const X& x, void* scratch, int64_t s
 }
 
 // A0 has A1 == A2 and A3 == A4 BIT FOR BIT (a value test would take -0.0 for 0.0, and the runs would then differ in
-// the sign of a zero); FPA_SWEEP_SYM=0 turns the symmetric kernels off (tests, A/B timing).
-static bool sweep_symmetric(const SweepExtra& x) {
+// the sign of a zero); FPA_SWEEP_SYM=0 turns the symmetric kernels off (tests, A/B timing).  The symmetric kernels'
+// 4*c*gamma must be finite (stage_sym_fast): an absurd gamma*h takes the 4-wave kernels, which compute the same bits.
+static bool sweep_symmetric(const Yaman4Params& p, const SweepExtra& x) {
+    bool c4g_finite = true;
+    for (int s = 0; s < 3; ++s) c4g_finite &= std::isfinite(p.coef.c2g[s] + p.coef.c2g[s]);
     return env_int("FPA_SWEEP_SYM", 1) != 0 && memcmp(&x.A0[0], &x.A0[2], 2 * sizeof(double)) == 0 &&
-           memcmp(&x.A0[4], &x.A0[6], 2 * sizeof(double)) == 0;
+           memcmp(&x.A0[4], &x.A0[6], 2 * sizeof(double)) == 0 && c4g_finite;
 }
 
 int yaman4_sweep_launch(const fpa_sweep_desc* d, void* scratch, int64_t scratch_bytes, cudaStream_t st) {
@@ -1353,7 +1449,7 @@ int yaman4_sweep_launch(const fpa_sweep_desc* d, void* scratch, int64_t scratch_
     int64_t      n_grid;
     int rc = sweep_setup(d, 1, p, x, n_grid);
     if (rc != FPA_OK || n_grid == 0) return rc;
-    if (sweep_symmetric(x)) return sweep_run<SweepExtra, true>(p, x, scratch, scratch_bytes, st);
+    if (sweep_symmetric(p, x)) return sweep_run<SweepExtra, true>(p, x, scratch, scratch_bytes, st);
     return sweep_run(p, x, scratch, scratch_bytes, st);
 }
 
