@@ -333,7 +333,10 @@ int fpa_yaman4_phase_sweep_dev(const fpa_phase_sweep_desc* d, void* scratch, int
  * FPA_PHASE_EXACT give FPA_ERR_UNSUPPORTED; `scratch` is ignored.
  * Sweep: the descriptor and units of fpa_yaman4_sweep_*; n_peers must be 0; FPA_PHASE_EXACT gives
  * FPA_ERR_UNSUPPORTED.  gain_lin may be NULL, and only then may p_signal be 0: a zero seed gives the undepleted-pump
- * linearisation.  The multi-device entry splits the flattened grid like fpa_yaman4_sweep_multi_host.
+ * linearisation.
+ * The multi-device entries split the work over several devices of one box from ONE process, the batch's points
+ * like fpa_yaman4_rk4_batch_multi_host and the sweep's flattened grid like fpa_yaman4_sweep_multi_host; results
+ * are bit-identical to the single-device call for any device list.
  * A point that is not integrated (invalid plan point, non-finite dbeta) and, under FPA_CHECK_NAN, a point whose
  * status is not FPA_POINT_OK get an all-NaN J.  J is dimensionless, the same in m and km units.
  */
@@ -345,6 +348,8 @@ typedef struct fpa_transfer_out {
 
 int fpa_yaman4_transfer_batch_dev (const fpa_yaman4_desc* d, const fpa_transfer_out* t, void* stream);
 int fpa_yaman4_transfer_batch_host(const fpa_yaman4_desc* d, const fpa_transfer_out* t, int device);
+int fpa_yaman4_transfer_batch_multi_host(const fpa_yaman4_desc* d, const fpa_transfer_out* t,
+                                         int n_devices, const int* devices);
 int fpa_yaman4_transfer_sweep_dev (const fpa_sweep_desc* d, const fpa_transfer_out* t, void* stream);
 int fpa_yaman4_transfer_sweep_host(const fpa_sweep_desc* d, const fpa_transfer_out* t, int device);
 int fpa_yaman4_transfer_sweep_multi_host(const fpa_sweep_desc* d, const fpa_transfer_out* t,

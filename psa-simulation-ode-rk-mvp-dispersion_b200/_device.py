@@ -53,25 +53,23 @@ def result_array(shape, dtype, pinned: bool = True) -> np.ndarray:
     return np.empty(shape, dtype=dtype)
 
 
-def _run_host(host, multi_host, desc, device, devices) -> None:
+def _run_host(host, multi_host, desc, device, devices, transfer=None) -> None:
     """`multi_host` over `devices` when they are several, else `host` on `device` (or the one entry of
-    `devices`, or the process default)."""
+    `devices`, or the process default).  `transfer`: the TransferOut the transfer entries take after the descriptor."""
+    args = (C.byref(desc),) if transfer is None else (C.byref(desc), C.byref(transfer))
     if devices is not None and len(devices) > 1:
         ids = (C.c_int * len(devices))(*[int(v) for v in devices])
-        _lib.check(multi_host(C.byref(desc), len(devices), ids))
+        _lib.check(multi_host(*args, len(devices), ids))
         return
     dev = _lib.get_device() if device is None else int(device)
     if devices is not None and len(devices) == 1:
         dev = int(devices[0])
-    _lib.check(host(C.byref(desc), dev))
+    _lib.check(host(*args, dev))
 
 
-def yaman4_batch(dbeta, gamma, alpha, A0, *, z0=0.0, z_max, n_steps, save_every=1, z_grid=None,
-                 trace=False, end=True, pmax=False, check_nan=True, phase_exact=False,
-                 device: Optional[int] = None, devices=None) -> dict:
-    """B scan points through `fpa_yaman4_rk4_batch_host` (`devices=[...]`: split over several GPUs
-    of the box by `fpa_yaman4_rk4_batch_multi_host`, bit-identical).  Returns a dict with the requested
-    outputs: A_trace [B,n_saved,4] c128, A_end [B,4] c128, Pmax [B,4] f64, status [B] i32."""
+def _yaman4_desc(dbeta, gamma, alpha, A0, *, z0, z_max, n_steps, save_every, z_grid, flags):
+    """Yaman4Desc over the inputs of B = dbeta.size points (gamma, alpha, A0 broadcast or per point), outputs unset.
+    Returns (desc, the arrays it points at)."""
     dbeta = f64(dbeta).reshape(-1)
     B = dbeta.size
     gam, gs = _per_point(gamma, B, 1, "gamma")
@@ -82,20 +80,11 @@ def yaman4_batch(dbeta, gamma, alpha, A0, *, z0=0.0, z_max, n_steps, save_every=
         raise ValueError("n_steps must be >= 1")
     if save_every <= 0:
         raise ValueError("save_every must be a positive integer")
-    ns = n_saved(n_steps, save_every)
     grid = None
     if z_grid is not None:
         grid = f64(z_grid).reshape(-1)
         if grid.size != n_steps + 1:
             raise ValueError("z_grid must hold n_steps+1 values")
-    big = B >= 4096            # single runs and small batches: not worth page-locking
-    out = {"status": result_array(B, np.int32, big)}
-    if trace:
-        out["A_trace"] = result_array((B, ns, 4), np.complex128, big and B * ns * 64 <= (1 << 30))
-    if end:
-        out["A_end"] = result_array((B, 4), np.complex128, big)
-    if pmax:
-        out["Pmax"] = result_array((B, 4), np.float64, big)
     d = _lib.Yaman4Desc()
     d.n_points = B
     d.dbeta = ptr(dbeta)
@@ -105,11 +94,28 @@ def yaman4_batch(dbeta, gamma, alpha, A0, *, z0=0.0, z_max, n_steps, save_every=
     d.z0, d.z_max = float(z0), float(z_max)
     d.n_steps, d.save_every = n_steps, save_every
     d.z_grid = ptr(grid)
-    d.flags = _flags(trace, end, pmax, check_nan, phase_exact)
-    d.A_trace = ptr(out.get("A_trace"))
-    d.A_end = ptr(out.get("A_end"))
-    d.Pmax = ptr(out.get("Pmax"))
-    d.status = ptr(out["status"])
+    d.flags = flags
+    return d, (dbeta, gam, alp, a0, grid)
+
+
+def yaman4_batch(dbeta, gamma, alpha, A0, *, z0=0.0, z_max, n_steps, save_every=1, z_grid=None,
+                 trace=False, end=True, pmax=False, check_nan=True, phase_exact=False,
+                 device: Optional[int] = None, devices=None) -> dict:
+    """B scan points through `fpa_yaman4_rk4_batch_host` (`devices=[...]`: split over several GPUs
+    of the box by `fpa_yaman4_rk4_batch_multi_host`, bit-identical).  Returns a dict with the requested
+    outputs: A_trace [B,n_saved,4] c128, A_end [B,4] c128, Pmax [B,4] f64, status [B] i32."""
+    d, keep = _yaman4_desc(dbeta, gamma, alpha, A0, z0=z0, z_max=z_max, n_steps=n_steps, save_every=save_every,
+                           z_grid=z_grid, flags=_flags(trace, end, pmax, check_nan, phase_exact))
+    B, ns = d.n_points, n_saved(d.n_steps, d.save_every)
+    big = B >= 4096            # single runs and small batches: not worth page-locking
+    out = {"status": result_array(B, np.int32, big)}
+    if trace:
+        out["A_trace"] = result_array((B, ns, 4), np.complex128, big and B * ns * 64 <= (1 << 30))
+    if end:
+        out["A_end"] = result_array((B, 4), np.complex128, big)
+    if pmax:
+        out["Pmax"] = result_array((B, 4), np.float64, big)
+    d.A_trace, d.A_end, d.Pmax, d.status = (ptr(out.get(k)) for k in ("A_trace", "A_end", "Pmax", "status"))
     L = _lib.lib()
     _run_host(L.fpa_yaman4_rk4_batch_host, L.fpa_yaman4_rk4_batch_multi_host, d, device, devices)
     return out
@@ -130,53 +136,18 @@ def transfer_out(columns: int, n_points: int, pinned: bool = False):
 def yaman4_transfer(dbeta, gamma, alpha, A0, columns, *, z0=0.0, z_max, n_steps, pmax=False, check_nan=True,
                     device: Optional[int] = None, devices=None) -> dict:
     """Transfer matrices of B points through `fpa_yaman4_transfer_batch_host`: jac [B,8,nc], A_end [B,4],
-    status [B] (and Pmax [B,4]).  `devices=[...]`: contiguous shares of the points, one host thread per device
-    (ctypes releases the GIL during each call, so the devices run at once); results identical to one device."""
-    dbeta = f64(dbeta).reshape(-1)
-    B = dbeta.size
-    gam, gs = _per_point(gamma, B, 1, "gamma")
-    alp, as_ = _per_point(alpha, B, 1, "alpha")
-    a0, a0s = _per_point(A0, B, 4, "A0", c128)
-    n_steps = int(n_steps)
-    if n_steps < 1:
-        raise ValueError("n_steps must be >= 1")
+    status [B] (and Pmax [B,4]).  `devices=[...]`: split over several GPUs of the box by
+    `fpa_yaman4_transfer_batch_multi_host`, bit-identical."""
+    d, keep = _yaman4_desc(dbeta, gamma, alpha, A0, z0=z0, z_max=z_max, n_steps=n_steps, save_every=1, z_grid=None,
+                           flags=_flags(False, True, pmax, check_nan, False))
+    B = d.n_points
     t, jac = transfer_out(columns, B)
     out = {"jac": jac, "A_end": np.empty((B, 4), np.complex128), "status": np.empty(B, np.int32)}
     if pmax:
         out["Pmax"] = np.empty((B, 4))
-    devs = [(_lib.get_device() if device is None else int(device))] if not devices else [int(v) for v in devices]
-    nc = jac.shape[2]
+    d.A_end, d.Pmax, d.status = (ptr(out.get(k)) for k in ("A_end", "Pmax", "status"))
     L = _lib.lib()
-
-    def part(k):
-        lo, hi = (B * k) // len(devs), (B * (k + 1)) // len(devs)
-        if hi <= lo:
-            return _lib.OK, ""
-        d = _lib.Yaman4Desc()
-        d.n_points = hi - lo
-        d.dbeta = ptr(dbeta) + 8 * lo
-        d.gamma, d.gamma_stride = ptr(gam) + 8 * lo * gs, gs
-        d.alpha, d.alpha_stride = ptr(alp) + 8 * lo * as_, as_
-        d.A0, d.A0_stride = ptr(a0) + 16 * 4 * lo * a0s, a0s
-        d.z0, d.z_max, d.n_steps, d.save_every = float(z0), float(z_max), n_steps, 1
-        d.flags = _flags(False, True, pmax, check_nan, False)
-        d.A_end = ptr(out["A_end"]) + 64 * lo
-        d.Pmax = ptr(out["Pmax"]) + 32 * lo if pmax else None
-        d.status = ptr(out["status"]) + 4 * lo
-        tp = _lib.TransferOut()
-        tp.columns, tp.jac = t.columns, ptr(jac) + 8 * 8 * nc * lo
-        rc = L.fpa_yaman4_transfer_batch_host(C.byref(d), C.byref(tp), devs[k])
-        return rc, (_lib.last_error() if rc != _lib.OK else "")
-
-    if len(devs) == 1:
-        _lib.check(part(0)[0])
-    else:
-        from concurrent.futures import ThreadPoolExecutor
-        with ThreadPoolExecutor(len(devs)) as ex:
-            res = list(ex.map(part, range(len(devs))))
-        for rc, msg in res:
-            if rc != _lib.OK:
-                raise {_lib.ERR_INVALID: ValueError, _lib.ERR_UNSUPPORTED: NotImplementedError}.get(rc, _lib.FpaError)(msg)
+    _run_host(L.fpa_yaman4_transfer_batch_host, L.fpa_yaman4_transfer_batch_multi_host, d, device, devices, t)
     return out
 
 
@@ -187,25 +158,13 @@ def transfer_sweep(desc, columns, *, device: Optional[int] = None, devices=None)
     G = n1 * n3
     big = G >= 4096
     t, jac = transfer_out(columns, G, big)
-    out = {"jac": jac.reshape(n1, n3, 8, -1), "A_end": result_array((n1, n3, 4), np.complex128, big),
-           "dbeta": result_array((n1, n3), np.float64, big), "valid": result_array((n1, n3), np.int32, big),
-           "status": result_array((n1, n3), np.int32, big)}
-    if desc.p_signal > 0.0:
-        out["gain_lin"] = result_array((n1, n3), np.float64, big)
-    desc.plan.dbeta, desc.plan.valid, desc.plan.omega = ptr(out["dbeta"]), ptr(out["valid"]), None
-    desc.gain_lin, desc.status = ptr(out.get("gain_lin")), ptr(out["status"])
-    desc.Pmax, desc.A_end = None, ptr(out["A_end"])
+    out = {"jac": jac.reshape(n1, n3, 8, -1), "A_end": result_array((n1, n3, 4), np.complex128, big)}
+    gain = {"gain_lin": np.float64} if desc.p_signal > 0.0 else {}
+    _sweep_outputs(desc, out, (n1, n3), big, dbeta=np.float64, valid=np.int32, status=np.int32, **gain)
     if G == 0:
         return out
     L = _lib.lib()
-    if devices is not None and len(devices) > 1:
-        ids = (C.c_int * len(devices))(*[int(v) for v in devices])
-        _lib.check(L.fpa_yaman4_transfer_sweep_multi_host(C.byref(desc), C.byref(t), len(devices), ids))
-    else:
-        dev = _lib.get_device() if device is None else int(device)
-        if devices is not None and len(devices) == 1:
-            dev = int(devices[0])
-        _lib.check(L.fpa_yaman4_transfer_sweep_host(C.byref(desc), C.byref(t), dev))
+    _run_host(L.fpa_yaman4_transfer_sweep_host, L.fpa_yaman4_transfer_sweep_multi_host, desc, device, devices, t)
     return out
 
 
@@ -273,6 +232,22 @@ def dbeta_table(plan, *, want_omega=False, device: Optional[int] = None) -> dict
     return out
 
 
+def _sweep_outputs(w, out, shape, pinned, given=None, **dtypes) -> None:
+    """Add to `out` one array of `shape` per `dtypes` entry (name -> dtype): `given`'s array of that name, which must
+    be C-contiguous with that shape and dtype, else `result_array(shape, dtype, pinned)`.  Then point the SweepDesc
+    `w` at out's plan outputs dbeta / valid (omega stays NULL), gain_lin, status, Pmax and A_end (NULL where `out`
+    has none)."""
+    for key, dtype in dtypes.items():
+        arr = (given or {}).get(key)
+        if arr is None:
+            arr = result_array(shape, dtype, pinned)
+        elif arr.shape != shape or arr.dtype != dtype or not arr.flags["C_CONTIGUOUS"]:
+            raise ValueError(f"out[{key!r}] must be a C-contiguous {np.dtype(dtype)} array of shape {shape}")
+        out[key] = arr
+    w.plan.dbeta, w.plan.valid, w.plan.omega = ptr(out["dbeta"]), ptr(out["valid"]), None
+    w.gain_lin, w.status, w.Pmax, w.A_end = (ptr(out.get(k)) for k in ("gain_lin", "status", "Pmax", "A_end"))
+
+
 def sweep(desc, *, want_pmax=False, want_end=False, device: Optional[int] = None,
           out: Optional[dict] = None, devices=None) -> dict:
     """Run `fpa_yaman4_sweep_host` on a SweepDesc whose plan axes / physics are filled.
@@ -282,23 +257,13 @@ def sweep(desc, *, want_pmax=False, want_end=False, device: Optional[int] = None
     `devices`: CUDA ordinals to split the flattened grid over from this one process
     (`fpa_yaman4_sweep_multi_host`)."""
     n1, n3 = desc.plan.n1, desc.plan.n3
-    given = out or {}
-    out = {}
-    for key, dtype in (("gain_lin", np.float64), ("dbeta", np.float64), ("valid", np.int32),
-                       ("status", np.int32)):
-        arr = given.get(key)
-        if arr is None:
-            arr = result_array((n1, n3), dtype, n1 * n3 >= 4096)
-        elif arr.shape != (n1, n3) or arr.dtype != dtype or not arr.flags["C_CONTIGUOUS"]:
-            raise ValueError(f"out[{key!r}] must be a C-contiguous {np.dtype(dtype)} array of shape {(n1, n3)}")
-        out[key] = arr
+    given, out = out, {}
     if want_pmax:
         out["Pmax"] = np.empty((n1, n3, 4))
     if want_end:
         out["A_end"] = np.empty((n1, n3, 4), dtype=np.complex128)
-    desc.plan.dbeta, desc.plan.valid, desc.plan.omega = ptr(out["dbeta"]), ptr(out["valid"]), None
-    desc.gain_lin, desc.status = ptr(out["gain_lin"]), ptr(out["status"])
-    desc.Pmax, desc.A_end = ptr(out.get("Pmax")), ptr(out.get("A_end"))
+    _sweep_outputs(desc, out, (n1, n3), n1 * n3 >= 4096, given, gain_lin=np.float64, dbeta=np.float64,
+                   valid=np.int32, status=np.int32)
     if n1 * n3 == 0:
         return out
     L = _lib.lib()
@@ -314,17 +279,14 @@ def phase_sweep(desc, *, want_map: bool = True, device: Optional[int] = None, de
     (`fpa_yaman4_phase_sweep_multi_host`)."""
     n1, n3, K = desc.sweep.plan.n1, desc.sweep.plan.n3, int(desc.n_phases)
     big = n1 * n3 * K >= 4096
-    out = {"dbeta": result_array((n1, n3), np.float64, big), "valid": result_array((n1, n3), np.int32, big),
-           "status": result_array((n1, n3, K), np.int32, big)}
+    out = {"status": result_array((n1, n3, K), np.int32, big)}
     if want_map:
         out["gain_lin"] = result_array((n1, n3, K), np.float64, big)
-    for key, dtype in (("gain_max", np.float64), ("gain_min", np.float64), ("idx_max", np.int32),
-                       ("idx_min", np.int32), ("n_finite", np.int32)):
-        out[key] = result_array((n1, n3), dtype, big)
+    reductions = {"gain_max": np.float64, "gain_min": np.float64, "idx_max": np.int32, "idx_min": np.int32,
+                  "n_finite": np.int32}
+    _sweep_outputs(desc.sweep, out, (n1, n3), big, dbeta=np.float64, valid=np.int32, **reductions)
+    for key in reductions:
         setattr(desc, key, ptr(out[key]))
-    w = desc.sweep
-    w.plan.dbeta, w.plan.valid, w.plan.omega = ptr(out["dbeta"]), ptr(out["valid"]), None
-    w.gain_lin, w.status, w.Pmax, w.A_end = ptr(out.get("gain_lin")), ptr(out["status"]), None, None
     if n1 * n3 == 0:
         return out
     L = _lib.lib()

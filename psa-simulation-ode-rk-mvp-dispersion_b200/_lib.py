@@ -147,6 +147,8 @@ SIGNATURES = {
     "fpa_yaman4_phase_sweep_dev": (C.c_int, [C.POINTER(PhaseSweepDesc), C.c_void_p, C.c_int64, C.c_void_p]),
     "fpa_yaman4_transfer_batch_dev": (C.c_int, [C.POINTER(Yaman4Desc), C.POINTER(TransferOut), C.c_void_p]),
     "fpa_yaman4_transfer_batch_host": (C.c_int, [C.POINTER(Yaman4Desc), C.POINTER(TransferOut), C.c_int]),
+    "fpa_yaman4_transfer_batch_multi_host": (C.c_int, [C.POINTER(Yaman4Desc), C.POINTER(TransferOut), C.c_int,
+                                                       C.POINTER(C.c_int)]),
     "fpa_yaman4_transfer_sweep_dev": (C.c_int, [C.POINTER(SweepDesc), C.POINTER(TransferOut), C.c_void_p]),
     "fpa_yaman4_transfer_sweep_host": (C.c_int, [C.POINTER(SweepDesc), C.POINTER(TransferOut), C.c_int]),
     "fpa_yaman4_transfer_sweep_multi_host": (C.c_int, [C.POINTER(SweepDesc), C.POINTER(TransferOut), C.c_int,

@@ -330,6 +330,24 @@ static int batch_host_launch(const fpa_yaman4_desc* d, int device, Pending* p) {
     return batch_host_launch(d, device, p, nullptr);
 }
 
+// Part k of a batch: a contiguous range of the points, sizes differing by at most one.
+static fpa_yaman4_desc batch_part(const fpa_yaman4_desc* d, int n_devices, int k, int64_t* lo) {
+    int64_t hi;
+    balanced_range(d->n_points, n_devices, k, lo, &hi);
+    const int64_t   ns   = fpa_n_saved(d->n_steps, d->save_every);
+    fpa_yaman4_desc part = *d;
+    part.n_points = hi - *lo;
+    part.dbeta    = d->dbeta + *lo;
+    part.gamma    = d->gamma + *lo * d->gamma_stride;
+    part.alpha    = d->alpha + *lo * d->alpha_stride;
+    part.A0       = d->A0 + *lo * d->A0_stride * 8;
+    if (d->A_trace) part.A_trace = d->A_trace + *lo * ns * 8;
+    if (d->A_end) part.A_end = d->A_end + *lo * 8;
+    if (d->Pmax) part.Pmax = d->Pmax + *lo * 4;
+    if (d->status) part.status = d->status + *lo;
+    return part;
+}
+
 // ----------------------------------------------------------------- sweeps
 // Phase sweep: the sweep kernel, then the per-grid-point reductions over its gain map on the same stream.
 static int phase_sweep_dev(const fpa_phase_sweep_desc* d, void* scratch, int64_t scratch_bytes, cudaStream_t st) {
@@ -599,22 +617,10 @@ int fpa_yaman4_rk4_batch_multi_host(const fpa_yaman4_desc* d, int n_devices, con
     FPA_TRY(yaman4_check(d));
     FPA_TRY(check_devices(n_devices, devices));
     if (n_devices == 1) return fpa_yaman4_rk4_batch_host(d, devices[0]);
-    const int64_t ns = fpa_n_saved(d->n_steps, d->save_every);
     return run_on_devices(n_devices, devices, [&](int k, Pending* p) {
-        int64_t lo, hi;
-        balanced_range(d->n_points, n_devices, k, &lo, &hi);
-        if (hi <= lo) return (int)FPA_OK;
-        fpa_yaman4_desc part = *d;
-        part.n_points = hi - lo;
-        part.dbeta    = d->dbeta + lo;
-        part.gamma    = d->gamma + lo * d->gamma_stride;
-        part.alpha    = d->alpha + lo * d->alpha_stride;
-        part.A0       = d->A0 + lo * d->A0_stride * 8;
-        if (d->A_trace) part.A_trace = d->A_trace + lo * ns * 8;
-        if (d->A_end) part.A_end = d->A_end + lo * 8;
-        if (d->Pmax) part.Pmax = d->Pmax + lo * 4;
-        if (d->status) part.status = d->status + lo;
-        return batch_host_launch(&part, devices[k], p);
+        int64_t               lo;
+        const fpa_yaman4_desc part = batch_part(d, n_devices, k, &lo);
+        return part.n_points > 0 ? batch_host_launch(&part, devices[k], p) : (int)FPA_OK;
     });
 }
 
@@ -711,6 +717,21 @@ int fpa_yaman4_transfer_batch_host(const fpa_yaman4_desc* d, const fpa_transfer_
     Pending p;
     FPA_TRY(batch_host_launch(d, device, &p, t));
     return finish(p, device);
+}
+
+int fpa_yaman4_transfer_batch_multi_host(const fpa_yaman4_desc* d, const fpa_transfer_out* t, int n_devices,
+                                         const int* devices) {
+    FPA_TRY(yaman4_transfer_check(d, t));
+    FPA_TRY(check_devices(n_devices, devices));
+    if (n_devices == 1) return fpa_yaman4_transfer_batch_host(d, t, devices[0]);
+    const int64_t nc = __builtin_popcount(t->columns);
+    return run_on_devices(n_devices, devices, [&](int k, Pending* p) {
+        int64_t               lo;
+        const fpa_yaman4_desc part = batch_part(d, n_devices, k, &lo);
+        fpa_transfer_out      tp   = *t;
+        tp.jac += lo * 8 * nc;
+        return part.n_points > 0 ? batch_host_launch(&part, devices[k], p, &tp) : (int)FPA_OK;
+    });
 }
 
 int fpa_yaman4_transfer_sweep_dev(const fpa_sweep_desc* d, const fpa_transfer_out* t, void* stream) {

@@ -30,7 +30,7 @@ from .config import SimulationConfig, custom_simulation_config, validate_config
 from .dispersion import DispersionParams
 from .parameters import FiberParams, SimulationGrid
 from .phase_matching import PhaseMatchingConfig, PhaseMatchingMethod, fill_plan_desc
-from .simulation import (_default_phase_matching_cfg, _length_scale_to_m, make_initial_amplitudes,
+from .simulation import (_default_phase_matching_cfg, _length_scale_to_m, _n_steps, make_initial_amplitudes,
                          run_batch_simulation, waves_to_columns)
 
 GainMode = Literal["end", "max"]
@@ -111,6 +111,57 @@ def _run_constants_ok(cfg, gamma, alpha, dispersion, pm_cfg, length_unit) -> boo
         return False
 
 
+def _sweep_args(lambda_p1_m, lambda_p2_m, lambda_signal_m, p_in, phase_in, need_seed=True):
+    """The wavelength axes (lam1, lam2, lam3) and the checked (p0, ph0) of a wavelength sweep."""
+    lam3 = _signal_axis(lambda_signal_m)
+    lam1 = np.atleast_1d(np.asarray(lambda_p1_m, dtype=float))
+    lam2 = np.atleast_1d(np.asarray(lambda_p2_m, dtype=float))
+    return (lam1, lam2, lam3), *_powers_and_phases(p_in, phase_in, need_seed)
+
+
+def _sweep_setup(w, axes, *, cfg, gamma, alpha, p0, dispersion, phase_matching_cfg, length_unit, device,
+                 phases=None, report_dbeta=True):
+    """What the wavelength sweeps share once their own arguments are checked.  Fills the SweepDesc `w` (plan, seed
+    power, physics, units, save_every, flags; not A0) and returns (arrays `w` points at, None).
+
+    When every run would raise (no phase-matching config, or a per-run check of the reference fails), `w` is left
+    alone and it returns (None, the all-NaN part every sweep reports then): dbeta [n1,n3], valid, status [n1,n3]
+    (or [n1,n3,phases]) and n_steps = 0.  With `report_dbeta`, dbeta is still computed there when the plan allows."""
+    pm_cfg = phase_matching_cfg
+    if pm_cfg is None:
+        try:
+            pm_cfg = _default_phase_matching_cfg(dispersion=dispersion, beta_legacy=None)
+        except ValueError:
+            pm_cfg = None
+    n1, n3 = axes[0].size, axes[2].size
+    if pm_cfg is None or not _run_constants_ok(cfg, gamma, alpha, dispersion, pm_cfg, length_unit):
+        shape = (n1, n3) if phases is None else (n1, n3, phases)
+        nan = {"dbeta": np.full((n1, n3), np.nan), "valid": np.zeros((n1, n3), np.int32),
+               "status": np.full(shape, -1, np.int32), "n_steps": 0}
+        if report_dbeta and isinstance(pm_cfg, PhaseMatchingConfig) and (
+                dispersion is not None or pm_cfg.method == PhaseMatchingMethod.PROVIDED):
+            plan, _ = _device.new_plan_desc(*axes)
+            fill_plan_desc(plan, dispersion, pm_cfg)
+            nan["dbeta"] = _device.dbeta_table(plan, device=device)["dbeta"]
+        return None, nan
+    plan, keep = _device.new_plan_desc(*axes)
+    fill_plan_desc(plan, dispersion, pm_cfg)
+    w.plan = plan
+    w.p_signal = float(p0[2])
+    w.gamma, w.alpha = float(gamma), float(alpha)
+    w.z_max, w.dz = float(cfg.z_max), float(cfg.dz)
+    w.length_scale = _length_scale_to_m(length_unit)
+    w.save_every = int(cfg.save_every)
+    w.flags = _lib.CHECK_NAN if cfg.check_nan else 0
+    return keep, None
+
+
+def _set_A0(d, p0, ph0):
+    A0 = make_initial_amplitudes(p0, ph0)
+    for j in range(4):
+        d.A0[2 * j], d.A0[2 * j + 1] = A0[j].real, A0[j].imag
+
+
 def sweep_gain_2d(*, cfg: SimulationConfig, lambda_p1_m, lambda_p2_m, lambda_signal_m, gamma: float,
                   alpha: float, p_in, phase_in=None, dispersion: Optional[DispersionParams] = None,
                   phase_matching_cfg: Optional[PhaseMatchingConfig] = None, length_unit: str = "m",
@@ -121,51 +172,20 @@ def sweep_gain_2d(*, cfg: SimulationConfig, lambda_p1_m, lambda_p2_m, lambda_sig
     status, n_steps).  One C-ABI call: axes up, results down.  `out` may hold preallocated
     (pinned) arrays for gain_lin / dbeta / valid / status.  `devices=[0, 1, ...]` splits the pump
     rows over several GPUs of the box from this one process (bit-identical results)."""
-    lam3 = _signal_axis(lambda_signal_m)
-    lam1 = np.atleast_1d(np.asarray(lambda_p1_m, dtype=float))
-    lam2 = np.atleast_1d(np.asarray(lambda_p2_m, dtype=float))
-    p0, ph0 = _powers_and_phases(p_in, phase_in)
+    axes, p0, ph0 = _sweep_args(lambda_p1_m, lambda_p2_m, lambda_signal_m, p_in, phase_in)
     unit = _norm_choice(gain_unit, ("db", "linear"), "gain_unit must be 'dB' or 'linear'")
-
-    pm_cfg = phase_matching_cfg
-    if pm_cfg is None:
-        try:
-            pm_cfg = _default_phase_matching_cfg(dispersion=dispersion, beta_legacy=None)
-        except ValueError:
-            pm_cfg = None
-    n1, n3 = lam1.size, lam3.size
-    if pm_cfg is None or not _run_constants_ok(cfg, gamma, alpha, dispersion, pm_cfg, length_unit):
-        # every run would raise -> all NaN; dbeta is still reported when it can be computed
-        nan = np.full((n1, n3), np.nan)
-        out = {"gain": nan, "gain_lin": nan.copy(), "dbeta": nan.copy(),
-               "valid": np.zeros((n1, n3), np.int32), "status": np.full((n1, n3), -1, np.int32),
-               "n_steps": 0}
-        if isinstance(pm_cfg, PhaseMatchingConfig) and (dispersion is not None or
-                                                        pm_cfg.method == PhaseMatchingMethod.PROVIDED):
-            plan, keep = _device.new_plan_desc(lam1, lam2, lam3)
-            fill_plan_desc(plan, dispersion, pm_cfg)
-            out["dbeta"] = _device.dbeta_table(plan, device=device)["dbeta"]
-        return out
-
-    s = _length_scale_to_m(length_unit)
     d = _lib.SweepDesc()
-    plan, keep = _device.new_plan_desc(lam1, lam2, lam3)
-    fill_plan_desc(plan, dispersion, pm_cfg)
-    d.plan = plan
-    A0 = make_initial_amplitudes(p0, ph0)
-    for j in range(4):
-        d.A0[2 * j], d.A0[2 * j + 1] = A0[j].real, A0[j].imag
-    d.p_signal = float(p0[2])
-    d.gamma, d.alpha = float(gamma), float(alpha)
-    d.z_max, d.dz = float(cfg.z_max), float(cfg.dz)
-    d.length_scale = s
-    d.save_every = int(cfg.save_every)
-    d.flags = _lib.CHECK_NAN if cfg.check_nan else 0
+    keep, nan = _sweep_setup(d, axes, cfg=cfg, gamma=gamma, alpha=alpha, p0=p0, dispersion=dispersion,
+                             phase_matching_cfg=phase_matching_cfg, length_unit=length_unit, device=device)
+    if keep is None:
+        g = np.full(nan["valid"].shape, np.nan)
+        return {"gain": g, "gain_lin": g.copy(), **nan}
+    _set_A0(d, p0, ph0)
     out = _device.sweep(d, want_pmax=want_pmax, device=device, out=out, devices=devices)
     g = out["gain_lin"]
     with np.errstate(invalid="ignore", divide="ignore"):
         out["gain"] = g if unit == "linear" else 10.0 * np.log10(g)
-    out["n_steps"] = int(round(float(cfg.z_max) * s / (float(cfg.dz) * s)))
+    out["n_steps"] = _n_steps(cfg, _length_scale_to_m(length_unit))
     return out
 
 
@@ -181,47 +201,24 @@ def sweep_transfer_2d(*, cfg: SimulationConfig, lambda_p1_m, lambda_p2_m, lambda
     `simulation.run_batch_transfer`; `waves` selects whole input waves.  Zero seeds are allowed (p_in[2] = 0 gives
     the undepleted-pump linearisation); every other argument error is raised as in `sweep_gain_2d`.  Invalid plan
     points and runs that fail under cfg.check_nan get an all-NaN J.  The small_signal module turns J into gains."""
-    lam3 = _signal_axis(lambda_signal_m)
-    lam1 = np.atleast_1d(np.asarray(lambda_p1_m, dtype=float))
-    lam2 = np.atleast_1d(np.asarray(lambda_p2_m, dtype=float))
-    p0, ph0 = _powers_and_phases(p_in, phase_in, need_seed=False)
+    axes, p0, ph0 = _sweep_args(lambda_p1_m, lambda_p2_m, lambda_signal_m, p_in, phase_in, need_seed=False)
     mask = waves_to_columns(waves)
     columns = tuple(c for c in range(8) if mask >> c & 1)
-
-    pm_cfg = phase_matching_cfg
-    if pm_cfg is None:
-        try:
-            pm_cfg = _default_phase_matching_cfg(dispersion=dispersion, beta_legacy=None)
-        except ValueError:
-            pm_cfg = None
-    n1, n3 = lam1.size, lam3.size
-    if pm_cfg is None or not _run_constants_ok(cfg, gamma, alpha, dispersion, pm_cfg, length_unit):
-        # every run would raise -> all NaN, as in sweep_gain_2d
-        nan = np.full((n1, n3), np.nan)
-        out = {"jac": np.full((n1, n3, 8, len(columns)), np.nan), "A_end": np.full((n1, n3, 4), np.nan + 0j),
-               "dbeta": nan, "valid": np.zeros((n1, n3), np.int32), "status": np.full((n1, n3), -1, np.int32),
-               "columns": columns, "n_steps": 0}
-        if p0[2] > 0.0:
-            out["gain_lin"] = nan.copy()
-        return out
-
-    s = _length_scale_to_m(length_unit)
     d = _lib.SweepDesc()
-    plan, keep = _device.new_plan_desc(lam1, lam2, lam3)
-    fill_plan_desc(plan, dispersion, pm_cfg)
-    d.plan = plan
-    A0 = make_initial_amplitudes(p0, ph0)
-    for j in range(4):
-        d.A0[2 * j], d.A0[2 * j + 1] = A0[j].real, A0[j].imag
-    d.p_signal = float(p0[2])
-    d.gamma, d.alpha = float(gamma), float(alpha)
-    d.z_max, d.dz = float(cfg.z_max), float(cfg.dz)
-    d.length_scale = s
-    d.save_every = int(cfg.save_every)
-    d.flags = _lib.CHECK_NAN if cfg.check_nan else 0
+    keep, nan = _sweep_setup(d, axes, cfg=cfg, gamma=gamma, alpha=alpha, p0=p0, dispersion=dispersion,
+                             phase_matching_cfg=phase_matching_cfg, length_unit=length_unit, device=device,
+                             report_dbeta=False)
+    if keep is None:
+        n1, n3 = nan["valid"].shape
+        out = {"jac": np.full((n1, n3, 8, len(columns)), np.nan), "A_end": np.full((n1, n3, 4), np.nan + 0j),
+               **nan, "columns": columns}
+        if p0[2] > 0.0:
+            out["gain_lin"] = np.full((n1, n3), np.nan)
+        return out
+    _set_A0(d, p0, ph0)
     out = _device.transfer_sweep(d, mask, device=device, devices=devices)
     out["columns"] = columns
-    out["n_steps"] = int(round(float(cfg.z_max) * s / (float(cfg.dz) * s)))
+    out["n_steps"] = _n_steps(cfg, _length_scale_to_m(length_unit))
     return out
 
 
@@ -272,10 +269,7 @@ def sweep_phase_gain_2d(*, cfg: SimulationConfig, lambda_p1_m, lambda_p2_m, lamb
     nanargmin, -1 where all K are NaN), phase_at_max / phase_at_min (phase_axis at those indices, NaN there),
     n_finite, extinction_db = 10 log10(gain_max / gain_min), dbeta, valid; relative_phase [K] = the theta_k of
     each phase index; n_steps).  A single plan (n1 = n3 = 1) is the G(theta) curve of one amplifier."""
-    lam3 = _signal_axis(lambda_signal_m)
-    lam1 = np.atleast_1d(np.asarray(lambda_p1_m, dtype=float))
-    lam2 = np.atleast_1d(np.asarray(lambda_p2_m, dtype=float))
-    p0, _ = _powers_and_phases(p_in, phase_in)
+    axes, p0, _ = _sweep_args(lambda_p1_m, lambda_p2_m, lambda_signal_m, p_in, phase_in)
     table, _, theta = phase_sweep_inputs(p_in, phase_in, phase_axis, phase_weights)
     ax = np.asarray(phase_axis, dtype=float)
     K = ax.size
@@ -283,43 +277,21 @@ def sweep_phase_gain_2d(*, cfg: SimulationConfig, lambda_p1_m, lambda_p2_m, lamb
     if gain_metric not in ("end", "max"):
         raise ValueError(f"Unknown gain_metric={gain_metric!r}. Use 'end' or 'max'.")
 
-    pm_cfg = phase_matching_cfg
-    if pm_cfg is None:
-        try:
-            pm_cfg = _default_phase_matching_cfg(dispersion=dispersion, beta_legacy=None)
-        except ValueError:
-            pm_cfg = None
-    n1, n3 = lam1.size, lam3.size
-    if pm_cfg is None or not _run_constants_ok(cfg, gamma, alpha, dispersion, pm_cfg, length_unit):
-        # every run would raise -> all NaN; dbeta is still reported when it can be computed
-        nan = np.full((n1, n3), np.nan)
-        out = {"gain_lin": np.full((n1, n3, K), np.nan), "gain_max": nan, "gain_min": nan.copy(),
+    d = _lib.PhaseSweepDesc()
+    keep, nan = _sweep_setup(d.sweep, axes, cfg=cfg, gamma=gamma, alpha=alpha, p0=p0, dispersion=dispersion,
+                             phase_matching_cfg=phase_matching_cfg, length_unit=length_unit, device=device, phases=K)
+    if keep is None:
+        n1, n3 = nan["valid"].shape
+        g = np.full((n1, n3), np.nan)
+        out = {"gain_lin": np.full((n1, n3, K), np.nan), "gain_max": g, "gain_min": g.copy(),
                "idx_max": np.full((n1, n3), -1, np.int32), "idx_min": np.full((n1, n3), -1, np.int32),
-               "n_finite": np.zeros((n1, n3), np.int32), "dbeta": nan.copy(),
-               "valid": np.zeros((n1, n3), np.int32), "status": np.full((n1, n3, K), -1, np.int32), "n_steps": 0}
-        if isinstance(pm_cfg, PhaseMatchingConfig) and (dispersion is not None or
-                                                        pm_cfg.method == PhaseMatchingMethod.PROVIDED):
-            plan, keep = _device.new_plan_desc(lam1, lam2, lam3)
-            fill_plan_desc(plan, dispersion, pm_cfg)
-            out["dbeta"] = _device.dbeta_table(plan, device=device)["dbeta"]
+               "n_finite": np.zeros((n1, n3), np.int32), **nan}
     else:
-        s = _length_scale_to_m(length_unit)
-        d = _lib.PhaseSweepDesc()
-        plan, keep = _device.new_plan_desc(lam1, lam2, lam3)
-        fill_plan_desc(plan, dispersion, pm_cfg)
-        w = d.sweep
-        w.plan = plan
-        w.p_signal = float(p0[2])
-        w.gamma, w.alpha = float(gamma), float(alpha)
-        w.z_max, w.dz = float(cfg.z_max), float(cfg.dz)
-        w.length_scale = s
-        w.save_every = int(cfg.save_every)
-        w.flags = _lib.CHECK_NAN if cfg.check_nan else 0
         d.n_phases = K
         d.A0_table = _lib.ptr(table)
         d.metric = _lib.GAIN_LAST_SAVED if gain_metric == "end" else _lib.GAIN_MAX_SAVED
         out = _device.phase_sweep(d, device=device, devices=devices)
-        out["n_steps"] = int(round(float(cfg.z_max) * s / (float(cfg.dz) * s)))
+        out["n_steps"] = _n_steps(cfg, _length_scale_to_m(length_unit))
     g = out["gain_lin"]
     with np.errstate(invalid="ignore", divide="ignore"):
         out["gain"] = g if unit == "linear" else 10.0 * np.log10(g)
@@ -529,8 +501,7 @@ def sweep_dbeta_gain(*, cfg: SimulationConfig, delta_beta, gamma: float, alpha: 
         raise ValueError(f"Unknown gain_mode={gain_mode!r}. Use 'end' or 'max'.")
     p0 = np.asarray(list(p_in), dtype=float)
     A0 = make_initial_amplitudes(p0, phase_in)
-    s = _length_scale_to_m(length_unit)
-    n_steps = int(round(float(cfg.z_max) * s / (float(cfg.dz) * s)))
+    n_steps = _n_steps(cfg, _length_scale_to_m(length_unit))
     ragged = gain_mode == "end" and n_steps % int(cfg.save_every) != 0
     r = run_batch_simulation(cfg, gamma=gamma, alpha=alpha, delta_beta=delta_beta, A0=A0,
                              length_unit=length_unit, outputs=("trace",) if ragged else ("end", "pmax"),

@@ -36,6 +36,13 @@ def _length_scale_to_m(length_unit: str) -> float:
     raise ValueError(f"Unsupported length_unit={length_unit!r}. Use 'm' or 'km'.")
 
 
+def _n_steps(cfg: SimulationConfig, s: float) -> int:
+    """RK4 steps of a run over cfg.z_max in steps of cfg.dz, both per length unit with `s` metres each: both are
+    scaled to metres before they are divided, so the count is the one the runner's metre-valued z_max and dz give
+    (z_max / dz unscaled can round differently when s != 1)."""
+    return int(round(float(cfg.z_max) * s / (float(cfg.dz) * s)))
+
+
 def _to_omega_array(omega) -> np.ndarray:
     return four(omega, "omega", positive_only=True)
 
@@ -156,6 +163,18 @@ def run_single_simulation(cfg: SimulationConfig, *, gamma: float, alpha: float,
     return z_m / _length_scale_to_m(out_unit), A
 
 
+def _batch_inputs(cfg, gamma, alpha, delta_beta, p_in, phase_in, A0, length_unit):
+    """The checks and unit scaling both batch runners start with: (s, A0, dbeta [B], gamma, alpha, z_max, n_steps),
+    dbeta / gamma / alpha per metre, z_max in metres, s = metres per length_unit."""
+    validate_config(cfg)
+    s = _length_scale_to_m(length_unit)
+    if A0 is None:
+        A0 = make_initial_amplitudes(p_in, phase_in)
+    db = np.asarray(delta_beta, dtype=float).reshape(-1) / s
+    return (s, A0, db, np.asarray(gamma, dtype=float) / s, np.asarray(alpha, dtype=float) / s,
+            float(cfg.z_max) * s, _n_steps(cfg, s))
+
+
 def run_batch_simulation(cfg: SimulationConfig, *, gamma, alpha, delta_beta, p_in=None, phase_in=None,
                          A0=None, length_unit: str = "m", outputs: Sequence[str] = ("end", "pmax"),
                          phase_exact: bool = False, device: Optional[int] = None, devices=None) -> dict:
@@ -166,16 +185,9 @@ def run_batch_simulation(cfg: SimulationConfig, *, gamma, alpha, delta_beta, p_i
     'trace' (A[B,n_saved,4] and z[n_saved]).  `status[B]` = first non-finite step or -1; with
     cfg.check_nan nothing is raised here -- bad points are the caller's to mask (the sweeps
     turn them into NaN like the reference, scan_mismtach.py:736-738)."""
-    validate_config(cfg)
-    s = _length_scale_to_m(length_unit)
-    if A0 is None:
-        A0 = make_initial_amplitudes(p_in, phase_in)
-    db = np.asarray(delta_beta, dtype=float).reshape(-1) / s
-    z_max, dz = float(cfg.z_max) * s, float(cfg.dz) * s
-    n_steps = int(round(z_max / dz))
+    s, A0, db, gam, alp, z_max, n_steps = _batch_inputs(cfg, gamma, alpha, delta_beta, p_in, phase_in, A0, length_unit)
     want = {str(o).lower() for o in outputs}
-    r = _device.yaman4_batch(db, np.asarray(gamma, dtype=float) / s, np.asarray(alpha, dtype=float) / s,
-                             A0, z_max=z_max, n_steps=n_steps, save_every=cfg.save_every,
+    r = _device.yaman4_batch(db, gam, alp, A0, z_max=z_max, n_steps=n_steps, save_every=cfg.save_every,
                              trace="trace" in want, end="end" in want, pmax="pmax" in want,
                              check_nan=cfg.check_nan, phase_exact=phase_exact, device=device, devices=devices)
     if "trace" in want:
@@ -206,17 +218,10 @@ def run_batch_transfer(cfg: SimulationConfig, *, gamma, alpha, delta_beta, p_in=
     (r odd) of A_{r//2}(L); column k is the derivative with respect to input component columns[k] (2w: Re A_w(0),
     2w+1: Im A_w(0)); `waves` selects whole waves (both quadratures).  J is dimensionless, the same in m and km.
     A run that fails under cfg.check_nan, or whose dbeta is not finite, gets an all-NaN J."""
-    validate_config(cfg)
-    s = _length_scale_to_m(length_unit)
-    if A0 is None:
-        A0 = make_initial_amplitudes(p_in, phase_in)
+    s, A0, db, gam, alp, z_max, n_steps = _batch_inputs(cfg, gamma, alpha, delta_beta, p_in, phase_in, A0, length_unit)
     mask = waves_to_columns(waves)
-    db = np.asarray(delta_beta, dtype=float).reshape(-1) / s
-    z_max, dz = float(cfg.z_max) * s, float(cfg.dz) * s
-    n_steps = int(round(z_max / dz))
-    r = _device.yaman4_transfer(db, np.asarray(gamma, dtype=float) / s, np.asarray(alpha, dtype=float) / s, A0,
-                                mask, z_max=z_max, n_steps=n_steps, check_nan=cfg.check_nan, device=device,
-                                devices=devices)
+    r = _device.yaman4_transfer(db, gam, alp, A0, mask, z_max=z_max, n_steps=n_steps, check_nan=cfg.check_nan,
+                                device=device, devices=devices)
     r["columns"] = tuple(c for c in range(8) if mask >> c & 1)
     r["n_steps"] = n_steps
     return r

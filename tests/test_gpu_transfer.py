@@ -203,8 +203,9 @@ def test_entries_and_device_splits_agree(gpu, golden):
     # batch: host against _dev
     db, A0, gam, alp = _batch_inputs(B=50)
     rb = gpu._device.yaman4_transfer(db, gam, alp, A0, 0xFF, z_max=20.0, n_steps=64)
-    rb2 = gpu._device.yaman4_transfer(db, gam, alp, A0, 0xFF, z_max=20.0, n_steps=64, devices=[0, 0, 0])
-    assert rb["jac"].tobytes() == rb2["jac"].tobytes()
+    for devs in [[0, 0, 0]] + ([[0, 1]] if L.device_count() > 1 else []):
+        rb2 = gpu._device.yaman4_transfer(db, gam, alp, A0, 0xFF, z_max=20.0, n_steps=64, devices=devs)
+        assert rb["jac"].tobytes() == rb2["jac"].tobytes(), devs
     bd = L.Yaman4Desc()
     ins = {k: torch.from_numpy(np.ascontiguousarray(v)).to(dev) for k, v in
            (("db", db), ("gam", gam), ("alp", alp), ("A0", A0.astype(np.complex128)))}

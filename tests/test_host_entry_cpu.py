@@ -22,6 +22,15 @@ def _batch(L, keep):
     return d
 
 
+def _transfer(L, keep):
+    """A transfer batch: the batch descriptor without its trace, and all eight columns."""
+    d = _batch(L, keep)
+    d.flags = L.OUT_END | L.OUT_PMAX | L.CHECK_NAN
+    jac = np.empty((3, 8, 8))
+    keep.append(jac)
+    return d, L.TransferOut(columns=0xFF, jac=L.ptr(jac))
+
+
 def _sweep(L, keep, d=None):
     lam1, lam2, lam3 = np.array([1550e-9, 1551e-9]), np.array([1558e-9]), np.linspace(1540e-9, 1565e-9, 4)
     out = dict(gain_lin=np.empty(8), status=np.empty(8, np.int32), db=np.empty(8), va=np.empty(8, np.int32))
@@ -61,9 +70,10 @@ def _nwave(L, keep):
     return d, slots
 
 
-def _host_and_multi(lib, host, multi):
+def _host_and_multi(lib, host, multi, *extra):
+    """Calls of the host and the multi-host entry on one descriptor; `extra` follows it (a TransferOut)."""
     ids = (C.c_int * 2)(0, 0)
-    return [lambda d: getattr(lib, host)(d, 0), lambda d: getattr(lib, multi)(d, 2, ids)]
+    return [lambda d: getattr(lib, host)(d, *extra, 0), lambda d: getattr(lib, multi)(d, *extra, 2, ids)]
 
 
 def _refused(L, rc, word):
@@ -86,6 +96,18 @@ def test_batch_refusals(fpa, field, value, word, multi):
     d = _batch(L, keep)
     setattr(d, field, value)
     call = _host_and_multi(L.lib(), "fpa_yaman4_rk4_batch_host", "fpa_yaman4_rk4_batch_multi_host")[multi]
+    _refused(L, call(C.byref(d)), word)
+
+
+@pytest.mark.parametrize("field, value, word",
+                         [c for c in BATCH_CASES if c[0] != "A_trace"] + [("columns", 0, "columns")])
+@pytest.mark.parametrize("multi", [False, True])
+def test_transfer_batch_refusals(fpa, field, value, word, multi):
+    L, keep = fpa._lib, []
+    d, t = _transfer(L, keep)
+    setattr(t if field == "columns" else d, field, value)
+    call = _host_and_multi(L.lib(), "fpa_yaman4_transfer_batch_host", "fpa_yaman4_transfer_batch_multi_host",
+                           C.byref(t))[multi]
     _refused(L, call(C.byref(d)), word)
 
 
@@ -141,12 +163,14 @@ def test_multi_host_device_lists(fpa, n_devices, word):
     L, keep, lib = fpa._lib, [], fpa._lib.lib()
     ids = (C.c_int * 65)()
     d, _ = _nwave(L, keep)
-    for entry, desc in (("fpa_yaman4_rk4_batch_multi_host", _batch(L, keep)),
-                        ("fpa_yaman4_sweep_multi_host", _sweep(L, keep)),
-                        ("fpa_yaman4_phase_sweep_multi_host", _phase(L, keep)),
-                        ("fpa_nwave_rk4_batch_multi_host", d)):
-        _refused(L, getattr(lib, entry)(C.byref(desc), n_devices, ids), word)
-        _refused(L, getattr(lib, entry)(C.byref(desc), 2, None), word)
+    td, t = _transfer(L, keep)
+    for entry, args in (("fpa_yaman4_rk4_batch_multi_host", (C.byref(_batch(L, keep)),)),
+                        ("fpa_yaman4_sweep_multi_host", (C.byref(_sweep(L, keep)),)),
+                        ("fpa_yaman4_phase_sweep_multi_host", (C.byref(_phase(L, keep)),)),
+                        ("fpa_nwave_rk4_batch_multi_host", (C.byref(d),)),
+                        ("fpa_yaman4_transfer_batch_multi_host", (C.byref(td), C.byref(t)))):
+        _refused(L, getattr(lib, entry)(*args, n_devices, ids), word)
+        _refused(L, getattr(lib, entry)(*args, 2, None), word)
 
 
 def test_multi_host_sweeps_split_the_whole_grid(fpa):
