@@ -156,3 +156,74 @@ def march(A0, gamma, alpha, beta, table, rows, *, z_max, n_steps, save_every=1, 
         return np.array(zs), np.array(ys), status
     return np.array(zs), np.array(ys)
 
+
+def _require_extended_precision():
+    if np.finfo(np.longdouble).nmant < 63:
+        raise RuntimeError(f"numpy's longdouble has {np.finfo(np.longdouble).nmant} mantissa bits on this platform; "
+                           "the extended-precision reference needs at least 63 (x87 80-bit or wider)")
+
+
+def nwave_rhs_ld(z, A, gamma, alpha, beta, tab, starts, nonempty):
+    """nwave_rhs_fast in long double: A clongdouble [N]; z, gamma, alpha, beta longdouble; tab [T,4] int (k, l, m,
+    weight); starts = row_ptr[:-1] of the rows in `nonempty`.  The phase of an entry is taken as the product of the
+    per-wave factors exp(i*b_j*z), the same number to long-double rounding as exp(i*(b_k + b_l - b_m - b_n)*z)."""
+    ph = beta * z
+    E = np.empty(A.size, dtype=np.clongdouble)
+    E.real, E.imag = np.cos(ph), np.sin(ph)
+    At = A * E
+    P = A.real * A.real + A.imag * A.imag
+    S = P.sum()
+    out = (-alpha / 2) * A + (1j * gamma) * ((2 * S - P) * A)
+    if tab.shape[0]:
+        k, l, m = tab[:, 0], tab[:, 1], tab[:, 2]
+        terms = (At[k] * At[l]) * (np.conj(At[m]) * tab[:, 3].astype(np.longdouble))
+        acc = np.zeros(A.size, dtype=np.clongdouble)
+        acc[nonempty] = np.add.reduceat(terms, starts)
+        out = out + (1j * gamma) * (np.conj(E) * acc)
+    return out
+
+
+def march_ld(A0, gamma, alpha, beta, table, rows, *, z_max, n_steps, save_every=1, z0=0.0, check=False):
+    """march() in extended precision: the same RK4 on the same FP64 abscissae linspace(z0, z_max, n_steps+1), with
+    the saving rule and the status of march().  The FP64 inputs a kernel gets (A0, gamma, alpha, beta) are promoted
+    as they are, so the only difference from a kernel's result is the kernel's own rounding.  Returns long-double
+    states (clongdouble [n_saved, N]); z_saved holds the FP64 abscissae.
+
+    Needs numpy's longdouble to carry at least 63 mantissa bits (x86-64 Linux: the x87 80-bit format, 64 bits);
+    anywhere else it raises instead of silently computing in FP64."""
+    _require_extended_precision()
+    LD = np.longdouble
+    beta = np.asarray(beta, dtype=float).astype(LD)
+    gamma, alpha, z0 = LD(float(gamma)), LD(float(alpha)), float(z0)
+    rows = np.asarray(rows, dtype=np.int64)
+    tab = np.asarray(table, dtype=np.int64).reshape(-1, 4)
+    nonempty = np.flatnonzero(np.diff(rows) > 0)
+    starts = rows[nonempty]
+
+    def f(z, y):
+        return nwave_rhs_ld(z, y, gamma, alpha, beta, tab, starts, nonempty)
+
+    grid = np.linspace(z0, z_max, n_steps + 1)
+    zl = grid.astype(LD)
+    y = np.asarray(A0, dtype=np.complex128).astype(np.clongdouble)
+    zs, ys = [grid[0]], [y.copy()]
+    status = -1
+    half, sixth = LD(1) / 2, LD(1) / 6
+    with np.errstate(over="ignore", invalid="ignore") if check else contextlib.nullcontext():
+        for i in range(n_steps):
+            z, h = zl[i], zl[i + 1] - zl[i]
+            k1 = f(z, y)
+            k2 = f(z + half * h, y + (half * h) * k1)
+            k3 = f(z + half * h, y + (half * h) * k2)
+            k4 = f(z + h, y + h * k3)
+            y = y + (h * sixth) * (k1 + 2 * k2 + 2 * k3 + k4)
+            if (i + 1) % save_every == 0:
+                zs.append(grid[i + 1])
+                ys.append(y.copy())
+            if check and not np.all(np.isfinite(y)):
+                status = i
+                break
+    if check:
+        return np.array(zs), np.array(ys), status
+    return np.array(zs), np.array(ys)
+

@@ -5,6 +5,7 @@ import numpy as np
 import pytest
 
 from conftest import rel_err
+from test_nwave_lines_cpu import assert_lines
 
 pytestmark = pytest.mark.gpu
 
@@ -54,7 +55,7 @@ def test_n21_dual_pump_plan_vs_oracle(gpu, nw_oracle, golden):
         A = r["A_trace"][0]
         assert A.shape == (41, 21)
         assert np.max(np.abs(A - A_ref)) / np.max(np.abs(A_ref)) < 1e-11, form
-        assert rel_err(np.abs(A[-1, seeded]) ** 2, np.abs(A_ref[-1, seeded]) ** 2) < 1e-10, form
+        assert_lines(A, A_ref, 1e-11, f"N = 21 {form}")      # every line, the 11 exact zeros included
         assert np.array_equal(r["A_end"][0], A[-1])
     # cascaded FWM populated lines that started empty
     assert (np.abs(A[-1, ~seeded]) ** 2).max() > 1e-12
@@ -94,10 +95,11 @@ def test_n64_comb_batch_vs_oracle(gpu, nw_oracle):
         for b in range(3):
             A_ref = refs[b]
             assert np.max(np.abs(r["A_trace"][b] - A_ref)) / np.max(np.abs(A_ref)) < 1e-12, form
-            # the 1e-12 W lines sit 12 decades below the pumps: their power is compared on the scale
-            # of the sum they are a small difference of (|A_pump|^3 * gamma * z)
-            strong = np.abs(A_ref[-1]) ** 2 > 1e-9
-            assert rel_err(np.abs(r["A_end"][b][strong]) ** 2, np.abs(A_ref[-1][strong]) ** 2) < 1e-10, form
+            # the 1e-12 W lines sit 12 decades below the pumps; FP64 arithmetic of the table sum and of the
+            # correlation form gives every line its own relative accuracy (the oracle: 8e-14 per line against
+            # a long-double march, tests/test_nwave_lines_cpu.py), so each line is compared on its own scale
+            assert_lines(r["A_trace"][b], A_ref, 1e-11, f"N = 64 {form} point {b}")
+            assert_lines(r["A_end"][b], A_ref[-1], 1e-11, f"N = 64 {form} point {b} A_end")
     assert plan.flops_per_step("comb") < plan.flops_per_step("entries") / 10
     # per-point gamma: a batch equals the single runs, bit for bit
     g = np.array([5e-3, 11.5e-3, 2e-2])
