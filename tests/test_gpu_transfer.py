@@ -14,6 +14,7 @@ import pytest
 ROOT = Path(__file__).resolve().parent.parent
 sys.path.insert(0, str(ROOT / "tools"))
 import transfer_model as TM  # noqa: E402
+from test_transfer_ld_cpu import assert_blocks, assert_waves  # noqa: E402
 
 pytestmark = pytest.mark.gpu
 P_IN = [0.3, 0.2, 1e-4, 2e-5]
@@ -84,13 +85,15 @@ def test_batch_jac_matches_cpu_model(gpu, case):
     elif case == "z0":
         gam, alp, z0, z_max = 0.015, 1e-3, 7.5, 37.5
     r = gpu._device.yaman4_transfer(db, gam, alp, A0, 0xFF, z0=z0, z_max=z_max, n_steps=n_steps)
+    worst = 0.0
     for b in range(db.size):
         g = gam if np.isscalar(gam) else gam[b]
         a = alp if np.isscalar(alp) else alp[b]
         A_end, J = TM.integrate(A0[b], g, a, db[b], z_max, n_steps, z0=z0)
-        assert _rel(r["jac"][b], J) <= 1e-12, (case, b)
-        assert _rel(r["A_end"][b], A_end) <= 1e-12
+        worst = max(worst, assert_blocks(r["jac"][b], J, 1e-13, f"{case} point {b}")[0])
+        assert_waves(r["A_end"][b], A_end, 1e-13, f"{case} point {b}")
     assert np.all(r["status"] == -1)
+    print(f"\n{case}: kernel vs the FP64 model, largest per-block error {worst:.1e}")
 
 
 def test_sweep_jac_matches_cpu_model_km(gpu, golden):
@@ -100,10 +103,12 @@ def test_sweep_jac_matches_cpu_model_km(gpu, golden):
     A0 = gpu.simulation.make_initial_amplitudes(P_IN, PHASE_IN)
     n_steps = r["n_steps"]
     # the integration uses dbeta / 1000 per metre; the reported dbeta is per km
+    worst = 0.0
     for i1 in range(2):
         for i3 in range(6):
             _, J = TM.integrate(A0, 11.5e-3, 1e-4, r["dbeta"][i1, i3] / 1000.0, L, n_steps)
-            assert _rel(r["jac"][i1, i3], J) <= 1e-12
+            worst = max(worst, assert_blocks(r["jac"][i1, i3], J, 1e-13, f"point ({i1}, {i3})")[0])
+    print(f"\nkm sweep: kernel vs the FP64 model, largest per-block error {worst:.1e}")
 
 
 # ------------------------------------------------------------------ J against finite differences of the batch integrator
